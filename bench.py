@@ -53,6 +53,8 @@ N_FIELDS, K5 = 39, 8
 B5_FWD = N_FIELDS * (8 + 4 + 4 + 8) + N_FIELDS * (N_FIELDS - 1) * 8 * K5 + 16
 B5_GRAD = B5_FWD + 8 + N_FIELDS * (N_FIELDS - 1) * 8 * K5 + N_FIELDS * 8
 B5_ADA = N_FIELDS * N_FIELDS * K5 * 40      # reference semantics: all fields x row features x k (SURVEY 8d)
+# --dump-outputs: grad P columns of this many features (N_ORDERS * K * 8 B each: 32 MB in all)
+DUMP_FEATURES, DUMP_SEED = 1 << 16, 2024
 
 
 def gen_criteo_rows(n, seed, d=D_FEATURES, dist="criteo"):
@@ -354,6 +356,12 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def workload_config(args, world, rows_per_step):
     return {"workload": "C4: synthetic Criteo-shaped CSR (39 nnz/row, 1M hashed features), HOFM degree 3 "
                         "rank 32 explicit lower orders, logistic loss, predict+grad "
@@ -491,6 +499,8 @@ class Bench:
         launches = _lib.launch_count() - l0
         self.barrier()
         clocks = sampler.stop()
+        if args.dump_outputs and self.rank == 0:
+            dump_outputs(args.dump_outputs, self.c4_outputs(h, loss_sum))
         ms_per_step = self.maxr(ms.value) / args.steps
         value = n * world / (ms_per_step / 1e3)
 
@@ -554,6 +564,16 @@ class Bench:
         if self.on("c3"):
             self.run_c3(line, ds, n, loss_kind)
         ds.free()
+
+    def c4_outputs(self, h, loss_sum):
+        """what the last timed step hands its caller: the loss sum and the gradient (all-reduced when N > 1).
+        grad P is 512 MB, so only the columns of a fixed, seeded sample of features are kept."""
+        gP, gw, gb = np.zeros((N_ORDERS, K, D_FEATURES)), np.zeros(D_FEATURES), C.c_double()
+        self._lib.check(self.lib.nimfm_fm_get_grads(self.ctx, h, self._lib.ptr(gP), self._lib.ptr(gw), C.byref(gb)))
+        feats = np.sort(np.random.default_rng(DUMP_SEED).choice(D_FEATURES, DUMP_FEATURES, replace=False))
+        return {"loss_sum": np.array([loss_sum]), "grad_intercept": np.array([gb.value]), "grad_w": gw,
+                "grad_P_sampled": np.ascontiguousarray(gP[:, :, feats]),
+                "grad_P_sampled_features": feats.astype(np.float64)}
 
     def run_e2e(self, line, h, data, indices, indptr, y, n, loss_kind):
         """end to end through the C ABI with HOST buffers, H2D inside the timed region: caller-pinned arrays,
@@ -878,7 +898,15 @@ def main():
     ap.add_argument("--skip", default="", help="comma list of sections to skip: parity,det,e2e,c4_adagrad,c3,c5,cd,seq,uniform")
     ap.add_argument("--dist", default="criteo", choices=["criteo", "uniform", "zipfall"],
                     help="index distribution; anything but 'criteo' is an experiment, not the reported workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed headline step returned (loss sum, gradient; grad P at a fixed "
+                         "sample of features) to DIR/<name>.npy as float64, for comparing two builds on the same "
+                         "seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.warmup < 3:

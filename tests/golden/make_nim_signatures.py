@@ -1,14 +1,14 @@
 """Extract the exported `fit` / `decisionFunction` signatures of the reference procs the Nim host layer (nim/*.nim)
-replaces, into tests/golden/nim_signatures.json.  Run here (needs /root/reference); the JSON is committed so the CPU test
-does not need the reference tree.
+replaces, into tests/golden/nim_signatures.json.  Needs a checkout of the reference (nimfm); the JSON is committed so
+the CPU test does not need the reference tree.
 
-    python tests/golden/make_nim_signatures.py
+    python tests/golden/make_nim_signatures.py <nimfm checkout>/src/nimfm
 """
 import json
 import os
 import re
+import sys
 
-REF = "/root/reference/src/nimfm"
 FILES = ["optimizer/cd.nim", "optimizer/minibatch_psgd.nim", "optimizer/adagrad.nim", "optimizer/adagrad_multi.nim",
          "optimizer/adagrad_ffm.nim", "optimizer/adagrad_ffm_multi.nim", "optimizer/sgd.nim", "optimizer/sgd_multi.nim",
          "optimizer/sgd_ffm.nim", "optimizer/sgd_ffm_multi.nim", "model/factorization_machine.nim",
@@ -40,10 +40,10 @@ def signatures(text):
     return out
 
 
-def main():
+def main(ref):
     table = {}
     for f in FILES:
-        table[f] = signatures(open(os.path.join(REF, f)).read())
+        table[f] = signatures(open(os.path.join(ref, f)).read())
     here = os.path.dirname(os.path.abspath(__file__))
     json.dump(table, open(os.path.join(here, "nim_signatures.json"), "w"), indent=1)
     for f, sigs in table.items():
@@ -52,4 +52,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -10,7 +10,7 @@ import pytest
 import nimfm_b200 as nf
 from nimfm_b200 import _lib
 from oracle.oracle import CSR
-from helpers import make_fm_params, max_rel
+from helpers import make_fm_params, max_rel, sums_agree
 from test_gpu_fm import dev_loss_grad, make_fm, ragged_csr, csr_ds
 
 pytestmark = pytest.mark.gpu
@@ -89,7 +89,11 @@ def test_deterministic_vs_red_route_and_mbpsgd(oracle, monkeypatch):
     ls_r, gP_r, gw_r, gb_r = dev_loss_grad(fm, csr_ds(csr), y, nf.Logistic())
     monkeypatch.setenv("NIMFM_DETERMINISTIC", "1")
     ls_d, gP_d, gw_d, gb_d = dev_loss_grad(fm, csr_ds(csr), y, nf.Logistic())
-    assert max_rel(gP_d, gP_r) <= 1e-11 and max_rel(gw_d, gw_r) <= 1e-11 and abs(ls_d - ls_r) <= 1e-12 * abs(ls_r)
+    # the RED route adds in arrival order, so its gP elements whose terms nearly cancel move from run to run by up to
+    # ~1e-11 of themselves (9.5e-12 over 40 runs on a B200 at 1000 W, as far from the oracle as from this route)
+    # while every element stays within ~1e-15 of the largest one: see helpers.sums_agree
+    assert sums_agree(gP_d, gP_r, norm_tol=1e-14, elem_tol=5e-11)
+    assert max_rel(gw_d, gw_r) <= 1e-11 and abs(ls_d - ls_r) <= 1e-12 * abs(ls_r)
 
     def fit():
         f = make_fm(degree, k, "explicit", True, True, P, w, 0.0, task=nf.classification)
