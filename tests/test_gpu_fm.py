@@ -46,7 +46,7 @@ def ragged_csr(n, d, seed, max_nnz):
 
 
 # ---------------------------------------------------------------- K1
-@pytest.mark.parametrize("degree", [2, 3, 4, 5])
+@pytest.mark.parametrize("degree", [2, 3, 4, 5, 6])
 @pytest.mark.parametrize("fit_lower", ["explicit", "none", "augment"])
 @pytest.mark.parametrize("k", [4, 10, 30])
 def test_decision_function_matches_oracle(oracle, degree, fit_lower, k):

@@ -20,7 +20,7 @@ LOSSES = {"squared": nf.Squared, "logistic": nf.Logistic, "squared_hinge": nf.Sq
 
 def random_case(seed):
     rng = np.random.default_rng(seed)
-    degree = int(rng.choice([2, 2, 3, 3, 4, 5]))
+    degree = int(rng.choice([2, 2, 3, 3, 4, 5, 6]))
     k = int(rng.choice([1, 3, 5, 8, 8, 16, 16, 32, 32, 40]))
     fit_lower = str(rng.choice(["explicit", "none", "augment"]))
     fit_linear, fit_intercept = bool(rng.integers(0, 2)), bool(rng.integers(0, 2))
