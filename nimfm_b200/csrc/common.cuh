@@ -198,6 +198,8 @@ struct nimfm_ffm {
   double *grad = nullptr;      // [gP | gw | gb, lossSum]
   double *gsP = nullptr, *gnP = nullptr, *gsw = nullptr, *gnw = nullptr, *dG = nullptr, *adaScal = nullptr;
   double *sgdCnt = nullptr;    // minibatch SGD (sgd_mb.cu)
+  mutable unsigned char *unitScratch = nullptr;   // ffm_units_kernel's records of long rows (ffm.cu), grown on demand
+  mutable size_t unitScratchBytes = 0;
   bool adaReady = false;
   double *scalingsP = nullptr, *scalingsW = nullptr, *sgdScal = nullptr;
   bool sgdReady = false;

@@ -43,6 +43,7 @@ struct FfmArgs {
   double eta0, tIt, alpha0, alpha, beta;
   int first;
   int CH;   // staging capacity in nonzeros (>= longest row)
+  unsigned char *unitScratch;   // ffm_units_kernel: per-block records of rows past FFM_UNITS_SMEM_CAP (nimfm_ffm)
 };
 
 struct __align__(16) FfmMeta {
@@ -54,6 +55,7 @@ struct __align__(16) FfmMeta {
 #include "ffm_pairs.cuh"
 #include "ffm_tma.cuh"
 #include "ffm_cols.cuh"
+#include "ffm_units.cuh"
 
 static size_t ffm_smem_bytes(int CH, int SB8, int nFields) {
   size_t b = (((size_t)CH * SB8 * 8 + 15) & ~(size_t)15) + (size_t)CH * sizeof(FfmMeta) + (size_t)CH * 4 +
@@ -312,15 +314,77 @@ static int ffm_has_field_dups(nimfm_ctx *ctx, const nimfm_dataset *X, bool *dups
 }
 
 static int ffm_plan(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset *X, int64_t nRows, FfmKernel kern,
-                    FfmPlan *pl);
+                    FfmPlan *pl, bool *declined);
+
+template <int KT>
+static FfmKernel ffm_units_mode(int mode) {
+  return mode == FFM_PREDICT ? ffm_units_kernel<FFM_PREDICT, KT>
+         : mode == FFM_GRAD  ? ffm_units_kernel<FFM_GRAD, KT>
+                             : ffm_units_kernel<FFM_ADAGRAD, KT>;
+}
+// the lane-group width that idles the fewest lanes over ceil(k / KT) chunks; ties go to the wider group (fewer chunks)
+static int ffm_units_kt(int k) {
+  int best = 32;
+  for (int kt = 16; kt >= 4; kt >>= 1)
+    if ((int64_t)(k + kt - 1) / kt * kt < (int64_t)(k + best - 1) / best * best) best = kt;
+  return best;
+}
+static FfmKernel ffm_units_pick(int k, int mode) {
+  switch (ffm_units_kt(k)) {
+    case 4: return ffm_units_mode<4>(mode);
+    case 8: return ffm_units_mode<8>(mode);
+    case 16: return ffm_units_mode<16>(mode);
+    default: return ffm_units_mode<32>(mode);
+  }
+}
+
+// global scratch of the unit kernel's long rows (ffm_units_row_bytes(longest row) per block) is held to this many
+// bytes by shrinking the grid
+#define FFM_UNITS_SCRATCH_MAX ((size_t)256 << 20)
+
+// the (nonzero, field) kernel (ffm_units.cuh): any k, any row length
+static int ffm_plan_units(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset *X, int64_t nRows, int mode,
+                          FfmPlan *pl) {
+  const int CH = (int)std::max<int64_t>(X->maxSegNnz, 1);
+  FfmKernel kern = ffm_units_pick(m->k, mode);
+  const size_t smem = ffm_units_row_bytes(std::min(CH, FFM_UNITS_SMEM_CAP));
+  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int occ = 0;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, FFM_UNITS_THREADS, smem));
+  if (occ < 1) return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "FFM unit kernel does not fit on an SM");
+  int64_t grid = std::min<int64_t>(nRows, (int64_t)occ * ctx->numSMs);
+  if (grid < 1) grid = 1;
+  if (CH > FFM_UNITS_SMEM_CAP) {
+    const size_t rowBytes = ffm_units_row_bytes(CH);
+    grid = std::max<int64_t>(1, std::min<int64_t>(grid, (int64_t)(FFM_UNITS_SCRATCH_MAX / rowBytes)));
+    const size_t need = (size_t)grid * rowBytes;
+    if (m->unitScratchBytes < need) {
+      CK(cudaStreamSynchronize(ctx->stream));   // an earlier launch may still read the old area
+      CK(cudaFree(m->unitScratch));
+      m->unitScratch = nullptr;
+      m->unitScratchBytes = 0;
+      CK(cudaMalloc(&m->unitScratch, need));
+      m->unitScratchBytes = need;
+    }
+  }
+  pl->CH = CH;
+  pl->grid = (int)grid;
+  pl->smem = smem;
+  pl->kern = kern;
+  pl->block = FFM_UNITS_THREADS;
+  pl->partialRows = grid;
+  return NIMFM_OK;
+}
 
 // Every mode chooses a pair kernel when one exists for k (NIMFM_FFM_KERNEL=block forces the staged
 // block-per-row kernel ffm_rows_kernel); FFM_ADAGRAD additionally needs a dataset without repeated
-// fields in a row.
+// fields in a row.  The staged kernel takes the rest; where its row does not fit shared memory, the
+// (nonzero, field) kernel ffm_units_kernel does (NIMFM_FFM_KERNEL=units forces it for every shape).
 static int ffm_plan_mode(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset *X, int64_t nRows, int mode,
                          FfmPlan *pl, bool targetsAligned16 = true) {
   const char *env = getenv("NIMFM_FFM_KERNEL");
   const bool forceBlock = env && !strcmp(env, "block");
+  if (env && !strcmp(env, "units")) return ffm_plan_units(ctx, m, X, nRows, mode, pl);
   const int CH = (int)std::max<int64_t>(X->maxSegNnz, 1);
   const bool table = CH <= FFM_PAIRS_TABLE_MAXZ;
   // the pair kernel addresses P through 32-bit (j*nFields + f): needs d*nFields < 2^31
@@ -431,27 +495,35 @@ static int ffm_plan_mode(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset
   FfmKernel bk = mode == FFM_PREDICT ? ffm_rows_kernel<FFM_PREDICT>
                  : mode == FFM_GRAD  ? ffm_rows_kernel<FFM_GRAD>
                                      : ffm_rows_kernel<FFM_ADAGRAD>;
-  int rc = ffm_plan(ctx, m, X, nRows, bk, pl);
+  bool declined = false;
+  int rc = ffm_plan(ctx, m, X, nRows, bk, pl, forceBlock ? nullptr : &declined);
   if (rc) return rc;
+  if (declined) return ffm_plan_units(ctx, m, X, nRows, mode, pl);
   pl->kern = bk;
   pl->block = FFM_THREADS;
   pl->partialRows = pl->grid;
   return NIMFM_OK;
 }
 
+// declined != nullptr: a shape the staged kernel cannot run sets *declined instead of failing
 static int ffm_plan(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset *X, int64_t nRows, FfmKernel kern,
-                    FfmPlan *pl) {
+                    FfmPlan *pl, bool *declined) {
   const int SB8 = (int)(m->nFields * m->k);
   const int CH = (int)std::max<int64_t>(X->maxSegNnz, 1);
   const size_t smem = ffm_smem_bytes(CH, SB8, (int)m->nFields);
-  if (smem > (size_t)ctx->smemOptin)
+  if (smem > (size_t)ctx->smemOptin) {
+    if (declined) { *declined = true; return NIMFM_OK; }
     return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
                       "FFM row of %d nonzeros x %d fields x rank %d needs %zu B of shared memory (> %d)", CH,
                       (int)m->nFields, m->k, smem, ctx->smemOptin);
+  }
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int occ = 0;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, FFM_THREADS, smem));
-  if (occ < 1) return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "FFM kernel does not fit on an SM");
+  if (occ < 1) {
+    if (declined) { *declined = true; return NIMFM_OK; }
+    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "FFM kernel does not fit on an SM");
+  }
   int64_t grid = std::min<int64_t>(nRows, (int64_t)occ * ctx->numSMs);
   if (grid < 1) grid = 1;
   pl->CH = CH;
@@ -477,6 +549,7 @@ static void ffm_fill_args(FfmArgs &a, const nimfm_ffm *m, const nimfm_dataset *X
   a.P = m->P; a.w = m->w; a.b = m->b;
   a.fitLinear = m->fitLinear; a.fitIntercept = m->fitIntercept;
   a.mb = 1.0;
+  a.unitScratch = m->unitScratch;
 }
 
 extern "C" {
@@ -514,6 +587,7 @@ int32_t nimfm_ffm_free(nimfm_ctx *ctx, nimfm_ffm *m) {
   for (double *p : {m->P, m->PT, m->w, m->b, m->gsP, m->gnP, m->gsw, m->gnw, m->adaScal, m->scalingsP,
                     m->scalingsW, m->sgdScal})
     cudaFree(p);
+  cudaFree(m->unitScratch);
   delete m;
   return NIMFM_OK;
 }
