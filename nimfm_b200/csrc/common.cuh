@@ -206,6 +206,16 @@ struct nimfm_ffm {
   std::vector<double> hostTmp;
 };
 
+// the lane-group width KT in {4, 8, 16, 32} of a runtime-k kernel that maps lane <-> component (ffm_units_kernel,
+// fm_cols_grad_generic_kernel): the one that idles the fewest lanes over ceil(k / KT) component chunks; ties go to
+// the wider group (fewer chunks)
+inline int lane_group_kt(int k) {
+  int best = 32;
+  for (int kt = 16; kt >= 4; kt >>= 1)
+    if ((int64_t)(k + kt - 1) / kt * kt < (int64_t)(k + best - 1) / best * best) best = kt;
+  return best;
+}
+
 // ------------------------------------------------------------------ error plumbing
 int nimfm_fail(nimfm_ctx *ctx, int code, const char *fmt, ...);
 

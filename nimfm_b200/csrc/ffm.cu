@@ -322,15 +322,8 @@ static FfmKernel ffm_units_mode(int mode) {
          : mode == FFM_GRAD  ? ffm_units_kernel<FFM_GRAD, KT>
                              : ffm_units_kernel<FFM_ADAGRAD, KT>;
 }
-// the lane-group width that idles the fewest lanes over ceil(k / KT) chunks; ties go to the wider group (fewer chunks)
-static int ffm_units_kt(int k) {
-  int best = 32;
-  for (int kt = 16; kt >= 4; kt >>= 1)
-    if ((int64_t)(k + kt - 1) / kt * kt < (int64_t)(k + best - 1) / best * best) best = kt;
-  return best;
-}
 static FfmKernel ffm_units_pick(int k, int mode) {
-  switch (ffm_units_kt(k)) {
+  switch (lane_group_kt(k)) {
     case 4: return ffm_units_mode<4>(mode);
     case 8: return ffm_units_mode<8>(mode);
     case 16: return ffm_units_mode<16>(mode);

@@ -70,9 +70,10 @@ RowKernel nimfm_row_stream_kernel_grad(int degree, bool explicitLower, int k);
 RowKernel nimfm_row_stream_kernel_adagrad(int degree, bool explicitLower, int k);
 RowKernel nimfm_row_fast_kernel_grad(int degree, bool explicitLower, int k);
 RowKernel nimfm_row_stream_kernel_stash(int degree, bool explicitLower, int k);
-int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, int G, int CH,
-                           int grid, int block, size_t smem, int64_t nWarps, int loss, double thr, int64_t rowBegin,
-                           int64_t nRows, double mb, double *yOutDev, const RowArgs &base);
+RowKernel nimfm_row_kernel_stash(int degree, bool explicitLower);
+int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, bool streamStash,
+                           int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+                           int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base);
 
 static bool is_explicit(const nimfm_fm *fm) { return fm->degree > 2 && fm->nOrders == fm->degree - 1; }
 
@@ -91,7 +92,8 @@ static int plan_rows(nimfm_ctx *ctx, const nimfm_fm *fm, const nimfm_dataset *X,
   if (z < 1) z = 1;
   const size_t capPerGroup = 40 * 1024;
   const bool expl = is_explicit(fm);
-  // variant: NIMFM_ROW_KERNEL = stream (default) | fast | generic   (A/B switch for profiling)
+  // variant: NIMFM_ROW_KERNEL = stream (default) | fast | generic   (A/B switch for profiling; generic also forces
+  // the generic stash forward, and with it the generic column kernel, of the deterministic route)
   const char *env = getenv("NIMFM_ROW_KERNEL");
   const bool wantGeneric = env && !strcmp(env, "generic");
   const bool wantFast = env && !strcmp(env, "fast");
@@ -105,10 +107,8 @@ static int plan_rows(nimfm_ctx *ctx, const nimfm_fm *fm, const nimfm_dataset *X,
                                   : nimfm_row_stream_kernel_adagrad(fm->degree, expl, k);
       stream = fast != nullptr;
     }
-    if (mode == MODE_STASH && !fast)
-      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic gradient supports degree 2 / 3 with nComponents in "
-                        "{8,16,32} and rows of at most 512 nonzeros");
-    if (!fast && mode != MODE_ADAGRAD) {
+    // (the staged fast kernel has no stash form: a shape without a streaming stash instance takes the generic one)
+    if (!fast && (mode == MODE_PREDICT || mode == MODE_GRAD)) {
       fast = mode == MODE_PREDICT ? nimfm_row_fast_kernel_predict(fm->degree, expl, k)
                                   : nimfm_row_fast_kernel_grad(fm->degree, expl, k);
       if (fast && (size_t)z * ((size_t)SB8 * 8 + 16) > capPerGroup) fast = nullptr;   // a row does not fit
@@ -124,6 +124,7 @@ static int plan_rows(nimfm_ctx *ctx, const nimfm_fm *fm, const nimfm_dataset *X,
   } else {
     kern = mode == MODE_PREDICT ? nimfm_row_kernel_predict(fm->degree, expl, k)
            : mode == MODE_GRAD  ? nimfm_row_kernel_grad(fm->degree, expl, k)
+           : mode == MODE_STASH ? nimfm_row_kernel_stash(fm->degree, expl)
                                 : nimfm_row_kernel_adagrad(fm->degree, expl, k);
     const size_t perNnz = (size_t)SB8 * 8 + 13;
     CH = std::min<int64_t>(z, (int64_t)(capPerGroup / perNnz));
@@ -436,8 +437,8 @@ static int launch_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X
     if ((rc = plan_rows(ctx, fm, X, nRows, MODE_STASH, &pl))) return rc;
     RowArgs base;
     fill_row_args(base, fm, X);
-    return nimfm_fm_det_loss_grad(ctx, fm, X, pl.kern, pl.G, pl.CH, pl.grid, pl.block, pl.smem, pl.nWarps, loss, thr,
-                                  rowBegin, nRows, mb, yOutDev, base);
+    return nimfm_fm_det_loss_grad(ctx, fm, X, pl.kern, pl.stream, pl.G, pl.CH, pl.grid, pl.block, pl.smem, pl.nWarps,
+                                  loss, thr, rowBegin, nRows, mb, yOutDev, base);
   }
   rc = plan_rows(ctx, fm, X, nRows, MODE_GRAD, &pl);
   if (rc) return rc;

@@ -13,8 +13,15 @@
 // Every gradient element is therefore a sum in ascending row order over fixed segments: bit-identical from run
 // to run and independent of the grid.  Traffic per nonzero: 12 B of CSC + the row's stash record (M_o-1 values per
 // component: 128 B for C3, 768 B for C4) instead of a re-gather of P and a RED; no read-for-ownership of cold
-// gradient lines.  Supported where the streaming row kernel is (degree 2 / 3, k in {8,16,32}) for a contiguous
-// row range without wrap-around.
+// gradient lines.
+// Two forms of each pass, which read and write the same stash record (stride 1 + k * sum_o (M_o - 1), padded to an
+// even number of doubles) and therefore combine either way:
+//   tuned    the streaming row kernel (fm_rows_stream.cuh) and fm_cols_grad_kernel<D, E, KT>: degree 2 / 3,
+//            k in {8,16,32}, rows of at most 512 nonzeros incl. dummy features;
+//   generic  the runtime-k row kernel (fm_rows.cuh, chunked long rows and component chunks) and
+//            fm_cols_grad_generic_kernel<D, E>: degree 2 .. 6, every k, rows of any length.
+// The tuned pair runs where the streaming forward runs; every other shape, and NIMFM_ROW_KERNEL=generic, takes the
+// generic pair.  Both need a contiguous row range without wrap-around (no row list).
 #include <stdlib.h>
 
 #include <algorithm>
@@ -43,6 +50,7 @@ struct ColArgs {
   double *gP, *gw;
   double *partial;          // [nSlots][SB8 + 1]
   int fitLinear;
+  int k, KT;                // fm_cols_grad_generic_kernel only: nComponents and the lane-group width
 };
 
 // first position in [lo, hi) whose row id is >= r
@@ -153,6 +161,111 @@ __global__ void __launch_bounds__(256) fm_cols_grad_kernel(const ColArgs a) {
   }
 }
 
+// fm_cols_grad_kernel with nComponents at run time (every degree, every k): a group of KT lanes (KT in {4,8,16,32},
+// lane_group_kt) maps lane <-> component s = sc*KT + lane of component chunk sc, and a task walks its entries once per
+// chunk; lanes past k idle.  Per entry the arithmetic is fm_cols_grad_kernel's expression sequence in the same
+// ascending row order, so where both kernels run they produce the same bits.
+template <int DEGREE, bool EXPLICIT>
+__global__ void __launch_bounds__(256, 2) fm_cols_grad_generic_kernel(const ColArgs a) {
+  constexpr int NO = RowCfg<DEGREE, EXPLICIT>::NO;
+  constexpr int NV = NO * (2 * DEGREE - NO - 1) / 2;   // stash values per component: sum over o of M_o - 1
+  constexpr int U = NV <= 6 ? 4 : 2;                   // entries per batch (register budget of av below)
+  const int k = a.k, KT = a.KT, SB8 = NO * k;
+  const int gl = (threadIdx.x & 31) & (KT - 1);
+  const int64_t group = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / KT;
+  const int64_t nGroups = (int64_t)gridDim.x * blockDim.x / KT;
+  const int NC = (k + KT - 1) / KT;
+  for (int64_t t = group; t < a.nTasks; t += nGroups) {
+    const int64_t j = a.taskCol[t];
+    const bool dummy = j >= a.d;
+    int64_t eb = a.taskBeg[t], ee = eb + a.taskLen[t];
+    if (!dummy) {   // clip the segment to the row range (rows ascend inside a column)
+      if ((int64_t)a.crow[eb] < a.rowBegin) eb = lower_bound_row(a.crow, eb, ee, a.rowBegin);
+      if (eb < ee && (int64_t)a.crow[ee - 1] >= a.rowEnd) ee = lower_bound_row(a.crow, eb, ee, a.rowEnd);
+    } else {
+      eb = eb < a.rowBegin ? a.rowBegin : eb;
+      ee = ee > a.rowEnd ? a.rowEnd : ee;
+    }
+    const int slot = a.taskSlot[t];
+    for (int sc = 0; sc < NC; ++sc) {
+      const int s = sc * KT + gl;
+      if (s >= k) break;
+      double p[NO], acc[NO], accW = 0.0;
+#pragma unroll
+      for (int o = 0; o < NO; ++o) {
+        p[o] = a.P[j * SB8 + o * k + s];
+        acc[o] = 0.0;
+      }
+      // the same software pipeline as fm_cols_grad_kernel: batch b+1's row ids / values load under batch b's records
+      int64_t rowN[U];
+      double xN[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const int64_t e = eb + u;
+        const bool ok = e < ee;
+        rowN[u] = ok ? (dummy ? e : (int64_t)a.crow[e]) : a.rowBegin;
+        xN[u] = ok ? (dummy ? 1.0 : a.cdata[e]) : 0.0;
+      }
+      for (int64_t e0 = eb; e0 < ee; e0 += U) {
+        double x[U], coef[U], av[U][NO][DEGREE];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+          const bool ok = e0 + u < ee;
+          x[u] = xN[u];
+          const double *rec = a.stash + (size_t)(rowN[u] - a.rowBegin) * a.stashStride;
+          coef[u] = ok ? rec[0] : 0.0;
+          int off = 1 + s;
+#pragma unroll
+          for (int o = 0; o < NO; ++o) {
+            const int M = DEGREE - o;
+#pragma unroll
+            for (int tt = 1; tt < DEGREE; ++tt)
+              if (tt < M) {
+                av[u][o][tt] = ok ? rec[off] : 0.0;
+                off += k;
+              }
+          }
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) {   // next batch's entries
+          const int64_t e = e0 + U + u;
+          const bool ok = e < ee;
+          rowN[u] = ok ? (dummy ? e : (int64_t)a.crow[e]) : a.rowBegin;
+          xN[u] = ok ? (dummy ? 1.0 : a.cdata[e]) : 0.0;
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) {   // entries in ascending row order: the sum has one order
+#pragma unroll
+          for (int o = 0; o < NO; ++o) {
+            const int M = DEGREE - o;
+            double g;
+            if (M == 2) {
+              g = x[u] * (av[u][o][1] - p[o] * x[u]);
+            } else {
+              g = x[u];
+#pragma unroll
+              for (int tt = 1; tt < DEGREE; ++tt)
+                if (tt < M) g = x[u] * (av[u][o][tt] - p[o] * g);
+            }
+            acc[o] += coef[u] * g;
+          }
+          accW += coef[u] * x[u];
+        }
+      }
+      if (slot < 0) {
+#pragma unroll
+        for (int o = 0; o < NO; ++o) a.gP[j * SB8 + o * k + s] += acc[o];
+        if (s == 0 && !dummy && a.fitLinear) a.gw[j] += accW;
+      } else {
+        double *ps = a.partial + (size_t)slot * (SB8 + 1);
+#pragma unroll
+        for (int o = 0; o < NO; ++o) ps[o * k + s] = acc[o];
+        if (s == 0) ps[SB8] = accW;
+      }
+    }
+  }
+}
+
 // columns cut into several segments: their partial sums are added in segment order
 __global__ void fm_cols_combine_kernel(const int32_t *multiCol, const int32_t *multiFirst, const int32_t *multiCount,
                                        int64_t nMulti, const double *partial, int SB8, int64_t d, double *gP, double *gw,
@@ -190,12 +303,35 @@ ColKernel pick_cols(int k) {
   }
 }
 
+ColKernel pick_cols_generic(int degree, bool explicitLower) {
+  switch (degree) {
+    case 2: return fm_cols_grad_generic_kernel<2, false>;
+    case 3: return explicitLower ? fm_cols_grad_generic_kernel<3, true> : fm_cols_grad_generic_kernel<3, false>;
+    case 4: return explicitLower ? fm_cols_grad_generic_kernel<4, true> : fm_cols_grad_generic_kernel<4, false>;
+    case 5: return explicitLower ? fm_cols_grad_generic_kernel<5, true> : fm_cols_grad_generic_kernel<5, false>;
+    case 6: return explicitLower ? fm_cols_grad_generic_kernel<6, true> : fm_cols_grad_generic_kernel<6, false>;
+    default: return nullptr;
+  }
+}
+
 }  // namespace
 
 RowKernel nimfm_row_stream_kernel_stash(int degree, bool explicitLower, int k) {
   switch (degree) {
     case 2: return pick_stash<2, false>(k);
     case 3: return explicitLower ? pick_stash<3, true>(k) : pick_stash<3, false>(k);
+    default: return nullptr;
+  }
+}
+
+// the stash forward of the generic runtime-k row kernel: every degree, every k, rows of any length
+RowKernel nimfm_row_kernel_stash(int degree, bool explicitLower) {
+  switch (degree) {
+    case 2: return fm_rows_kernel<2, false, MODE_STASH, 0>;
+    case 3: return explicitLower ? fm_rows_kernel<3, true, MODE_STASH, 0> : fm_rows_kernel<3, false, MODE_STASH, 0>;
+    case 4: return explicitLower ? fm_rows_kernel<4, true, MODE_STASH, 0> : fm_rows_kernel<4, false, MODE_STASH, 0>;
+    case 5: return explicitLower ? fm_rows_kernel<5, true, MODE_STASH, 0> : fm_rows_kernel<5, false, MODE_STASH, 0>;
+    case 6: return explicitLower ? fm_rows_kernel<6, true, MODE_STASH, 0> : fm_rows_kernel<6, false, MODE_STASH, 0>;
     default: return nullptr;
   }
 }
@@ -279,16 +415,25 @@ int nimfm_det_twin_get(nimfm_ctx *ctx, const nimfm_dataset *X, int nAug, nimfm_d
 
 // Deterministic predict+grad over rows [rowBegin, rowBegin + nRows) of X into the model's gradient buffers
 // (accumulating, like the RED route).  red4 (loss, sum coef, sum dL^2, -) is left at ctx->scalars + 8.
-int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, int G, int CH,
-                           int grid, int block, size_t smem, int64_t nWarps, int loss, double thr, int64_t rowBegin,
-                           int64_t nRows, double mb, double *yOutDev, const RowArgs &base) {
+// streamStash: stashKern is the streaming instance; the tuned column kernel then reads its stash, and every other
+// shape (or NIMFM_ROW_KERNEL=generic, which plans the generic stash forward) takes the runtime-k column kernel.
+int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, bool streamStash,
+                           int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+                           int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base) {
   if (rowBegin < 0 || rowBegin + nRows > X->n)
     return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic gradient needs a contiguous row range without wrap-around");
   const bool expl = fm->degree > 2 && fm->nOrders == fm->degree - 1;
-  ColKernel ck = fm->degree == 2 ? pick_cols<2, false>(fm->k)
-                 : fm->degree == 3 ? (expl ? pick_cols<3, true>(fm->k) : pick_cols<3, false>(fm->k)) : nullptr;
+  ColKernel ck = nullptr;
+  int colKT = fm->k;
+  if (streamStash)
+    ck = fm->degree == 2 ? pick_cols<2, false>(fm->k)
+         : fm->degree == 3 ? (expl ? pick_cols<3, true>(fm->k) : pick_cols<3, false>(fm->k)) : nullptr;
+  if (!ck) {
+    ck = pick_cols_generic(fm->degree, expl);
+    colKT = lane_group_kt(fm->k);
+  }
   if (!ck || !stashKern)
-    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic gradient supports degree 2 / 3 with nComponents in {8,16,32}");
+    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "no deterministic gradient kernel for degree %d", fm->degree);
   int rc;
   nimfm_det_twin *tw = nullptr;
   if ((rc = nimfm_det_twin_get(ctx, X, fm->nAug, &tw))) return rc;
@@ -303,7 +448,14 @@ int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X,
     if (ctx->stash) CK(cudaFree(ctx->stash));
     ctx->stash = nullptr;
     ctx->stashCap = 0;
-    CK(cudaMalloc(&ctx->stash, need * 8));
+    if (cudaMalloc(&ctx->stash, need * 8) != cudaSuccess) {
+      (void)cudaGetLastError();   // an allocation failure is not sticky: later calls must not see it
+      ctx->stash = nullptr;
+      return nimfm_fail(ctx, NIMFM_ERR_CUDA,
+                        "the deterministic gradient could not allocate its stash: %zu bytes = 8 x (nRows %lld x stride %d "
+                        "+ column partial sums); stride = 1 + nComponents x sum_o (degree - o - 1), rounded up to even",
+                        need * 8, (long long)nRows, stride);
+    }
     ctx->stashCap = need;
   }
   if ((rc = nimfm_ensure_partials(ctx, (size_t)nWarps * 4))) return rc;
@@ -342,8 +494,10 @@ int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X,
   c.gw = fm->grad + fm->nP();
   c.partial = ctx->stash + (size_t)std::max<int64_t>(nRows, 1) * stride;
   c.fitLinear = fm->fitLinear;
+  c.k = fm->k;
+  c.KT = colKT;
   if (tw->nTasks > 0) {
-    const int64_t groupsPerBlock = 256 / fm->k;
+    const int64_t groupsPerBlock = 256 / colKT;
     const int cgrid = (int)std::max<int64_t>(1, std::min<int64_t>((tw->nTasks + groupsPerBlock - 1) / groupsPerBlock,
                                                                   (int64_t)ctx->numSMs * 8));
     ck<<<cgrid, 256, 0, ctx->stream>>>(c);

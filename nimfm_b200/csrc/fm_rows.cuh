@@ -12,7 +12,9 @@
 //      the group is reduced with warp shuffles, loss / dloss are evaluated (loss.nim);
 //   4. backward (MODE_GRAD / MODE_ADAGRAD): the derivative recurrence (sgd.nim:176-188) re-reads the
 //      staged slice (no second gather) and scatters coef*dA with FP64 RED atomics
-//      (minibatch_psgd.nim:77-88 / adagrad.nim:113-134).
+//      (minibatch_psgd.nim:77-88 / adagrad.nim:113-134);
+//   4'. MODE_STASH (the deterministic gradient, fm_cols.cu): no backward pass; each component chunk's
+//      A[o][1 .. M_o-1] and the row's coef go to the row's stash record, which the column kernels read.
 // Hot features: columns present in a large fraction of the rows (dense numeric columns, dummy features
 // of fitLower=augment) would serialise ~nRows RED operations on the same few L2 addresses.  The dataset
 // carries a byte table hotSlot[j] (built from a row sample at upload); gradients of hot features are
@@ -99,7 +101,7 @@ __global__ void __launch_bounds__(256, 1) fm_rows_kernel(const RowArgs a) {
   const int gidInWarp = lane / G;
   const int SB8 = NO * k;  // doubles per feature slice
   constexpr int NACC = (MODE == MODE_ADAGRAD) ? 2 : 1;
-  const int nHotTot = (MODE == MODE_PREDICT) ? 0 : a.nHot + a.nAug;
+  const int nHotTot = (MODE == MODE_PREDICT || MODE == MODE_STASH) ? 0 : a.nHot + a.nAug;
   const int ASTR = SB8 + 1;  // accumulator stride per slot: SB8 P-gradients + 1 w-gradient
   const size_t perGroup = row_group_smem(CH, SB8, nHotTot, NACC);
   unsigned char *base = smem_raw + (size_t)(warpInBlock * gpw + gidInWarp) * perGroup;
@@ -161,7 +163,7 @@ __global__ void __launch_bounds__(256, 1) fm_rows_kernel(const RowArgs a) {
         }
         sIdx[u] = j;
         sVal[u] = x;
-        if (MODE != MODE_PREDICT)
+        if (MODE != MODE_PREDICT && MODE != MODE_STASH)
           sSlot[u] = pos >= zReal ? (unsigned char)(a.nHot + (pos - zReal))
                                   : (a.hotSlot ? a.hotSlot[j] : (unsigned char)NIMFM_COLD);
         if (withLinear && pos < zReal) lin += a.w[j] * x;
@@ -251,6 +253,25 @@ __global__ void __launch_bounds__(256, 1) fm_rows_kernel(const RowArgs a) {
     double part = 0.0;
     for (int sc = 0; sc < NS; ++sc) {
       part += fwd_all(sc, A, sc == 0, lin);
+      if (MODE == MODE_STASH) {
+        // the row's stash record (fm_cols.cu) takes A[o][1 .. M_o-1] of this component chunk, laid out like the
+        // streaming kernel's: [coef | A[o][t][s] for o, t = 1 .. M_o-1, s < k]
+        const int s = sc * G + gl;
+        if (active && s < k) {
+          double *rec = a.stash + (size_t)q * a.stashStride + 1 + s;
+          int off = 0;
+#pragma unroll
+          for (int o = 0; o < NO; ++o) {
+            const int M = DEGREE - o;
+#pragma unroll
+            for (int tt = 1; tt < DEGREE; ++tt)
+              if (tt < M) {
+                rec[off] = A[o][tt];
+                off += k;
+              }
+          }
+        }
+      }
     }
     // (for nChunks == 1 the staged slice stays resident for the backward pass)
     const double yhat = bias + group_sum(lin + part, G);
@@ -261,16 +282,17 @@ __global__ void __launch_bounds__(256, 1) fm_rows_kernel(const RowArgs a) {
       if (MODE != MODE_PREDICT) {
         const double yi = a.y[r];
         dL = dev_dloss(a.loss, a.thr, yi, yhat);
-        coef = (MODE == MODE_GRAD) ? dL / a.mb : dL;
+        coef = (MODE == MODE_GRAD || MODE == MODE_STASH) ? dL / a.mb : dL;
         if (gl == 0) {
           accLoss += dev_loss(a.loss, a.thr, yi, yhat);
           accB1 += coef;
           accB2 += dL * dL;
+          if (MODE == MODE_STASH) a.stash[(size_t)q * a.stashStride] = coef;
         }
       }
     }
 
-    if (MODE != MODE_PREDICT) {
+    if (MODE != MODE_PREDICT && MODE != MODE_STASH) {
       for (int sc = NS - 1; sc >= 0; --sc) {
         const int s = sc * G + gl;
         if (sc != NS - 1) {
@@ -337,7 +359,7 @@ __global__ void __launch_bounds__(256, 1) fm_rows_kernel(const RowArgs a) {
     __syncwarp();
   }
 
-  if (MODE != MODE_PREDICT && nHotTot > 0) {
+  if (MODE != MODE_PREDICT && MODE != MODE_STASH && nHotTot > 0) {
     // flush the hot-feature accumulators: every lane writes the elements it owns
     __syncwarp();
     for (int slot = 0; slot < nHotTot; ++slot) {
