@@ -661,7 +661,14 @@ int32_t nimfm_ffm_decision_function(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_da
 static bool ffm_cols_default(int64_t nRows) { (void)nRows; return false; }
 
 // The atomic-free route (ffm_cols.cuh).  *taken = 0: the shape is outside what it supports (the caller runs the
-// RED route) unless `must` is set (NIMFM_DETERMINISTIC=1), in which case that is an error.
+// RED route) unless `must` is set (NIMFM_DETERMINISTIC=1), in which case that is an error.  Under `must` every
+// contiguous row range of a dataset without repeated fields runs: the tuned column kernel where its shape limits
+// hold, the generic one elsewhere.  Without `must` (NIMFM_FFM_GRAD=cols) the route runs where the tuned kernel does.
+// NIMFM_FFM_COLS=generic puts the generic kernel in the tuned kernel's place.
+// A stated upper bound on the generic column kernel's resident 128-thread blocks per SM, not a tuning choice: it
+// equals the register-limited occupancy of the 112 / 126-register instances and lies above that of the 200 /
+// 225-register ones (2), so it changes no launch; the tests size their data past three waves of this bound.
+#define FFM_COLS_GENERIC_BLOCKS_PER_SM 4
 static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int loss, double thr,
                                 int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb, bool must,
                                 int *taken) {
@@ -671,16 +678,38 @@ static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_datase
   ColKern ck = m->k == 4 ? ffm_cols_grad_kernel<4, E> : m->k == 8 ? ffm_cols_grad_kernel<8, E>
                : m->k == 16 ? ffm_cols_grad_kernel<16, E> : (ColKern) nullptr;
   const int CH = (int)std::max<int64_t>(X->maxSegNnz, 1);
+  const bool contiguous = !rowIdxDev && rowBegin >= 0 && rowBegin + nRows <= X->n;
+  const bool tunedShape = ck && CH <= 64 && m->nFields <= 64 && m->d * m->nFields < (int64_t)2147483647;
+  if (!contiguous || !(tunedShape || must)) {
+    if (must)
+      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
+                        "the deterministic FFM gradient needs a contiguous row range (no row list, no wrap-around)");
+    return NIMFM_OK;
+  }
   bool dups = true;
   int rc;
-  const bool shapeOk = ck && !rowIdxDev && rowBegin >= 0 && rowBegin + nRows <= X->n && CH <= 64 && m->nFields <= 64 &&
-                       m->d * m->nFields < (int64_t)2147483647;
-  if (shapeOk && (rc = ffm_has_field_dups(ctx, X, &dups))) return rc;
-  if (!shapeOk || dups) {
+  if ((rc = ffm_has_field_dups(ctx, X, &dups))) return rc;
+  if (dups) {
     if (must)
-      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic FFM gradient needs a contiguous row range, rows of at "
-                        "most 64 nonzeros with one nonzero per field, nFields <= 64 and nComponents in {4,8,16}");
+      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic FFM gradient needs rows with one nonzero per "
+                        "field (a row of this dataset repeats a field)");
     return NIMFM_OK;
+  }
+  const char *envC = getenv("NIMFM_FFM_COLS");
+  const bool generic = !tunedShape || (envC && !strcmp(envC, "generic"));
+  size_t warpSmem = ffm_cols_warp_smem(E);
+  int64_t taskMul = 1;   // warp tasks per column segment
+  if (generic) {
+    const int kt = ffm_cols_generic_kt(m->k);
+    int gE;
+    switch (kt) {   // entries per batch: the most without spills (ptxas), 24-64 partner components per lane in flight
+      case 4: ck = ffm_cols_grad_generic_kernel<4, 6>; gE = 6; break;
+      case 8: ck = ffm_cols_grad_generic_kernel<8, 4>; gE = 4; break;
+      case 16: ck = ffm_cols_grad_generic_kernel<16, 4>; gE = 4; break;
+      default: ck = ffm_cols_grad_generic_kernel<32, 2>; gE = 2; break;
+    }
+    warpSmem = ffm_cols_generic_warp_smem(gE);
+    taskMul = (m->nFields + 31) / 32 * ((m->k + kt - 1) / kt);   // (segment, block of 32 fields, component chunk)
   }
   nimfm_det_twin *tw = nullptr;
   if ((rc = nimfm_det_twin_get(ctx, X, 0, &tw))) return rc;
@@ -691,7 +720,14 @@ static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_datase
     if (ctx->stash) CK(cudaFree(ctx->stash));
     ctx->stash = nullptr;
     ctx->stashCap = 0;
-    CK(cudaMalloc(&ctx->stash, need * 8));
+    if (cudaMalloc(&ctx->stash, need * 8) != cudaSuccess) {
+      (void)cudaGetLastError();   // an allocation failure is not sticky: later calls must not see it
+      ctx->stash = nullptr;
+      return nimfm_fail(ctx, NIMFM_ERR_CUDA,
+                        "the deterministic FFM gradient could not allocate its stash: %zu bytes = 8 x (nRows %lld + "
+                        "%lld column partial sums x (nFields x nComponents %d + 1))",
+                        need * 8, (long long)nRows, (long long)tw->nSlots, SB8);
+    }
     ctx->stashCap = need;
   }
   // pass 1: the forward pair kernel leaves yhat per row, then coef = dloss / mb in place + the loss partials
@@ -724,13 +760,15 @@ static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_datase
   c.PT = m->PT; c.gP = m->grad; c.gw = m->grad + m->nP();
   c.partial = ctx->stash + std::max<int64_t>(nRows, 1);
   c.fitLinear = m->fitLinear;
+  c.k = m->k;
   if (tw->nTasks > 0) {
     const int block = 128;   // 143 registers at k = 8: three 4-warp blocks per SM
-    const size_t smem = (size_t)(block / 32) * ffm_cols_warp_smem(E);
+    const size_t smem = (size_t)(block / 32) * warpSmem;
     CK(cudaFuncSetAttribute(ck, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ck, block, smem));
-    const int64_t wantBlocks = (tw->nTasks + block / 32 - 1) / (block / 32);
+    if (generic) occ = std::min(occ, FFM_COLS_GENERIC_BLOCKS_PER_SM);
+    const int64_t wantBlocks = (tw->nTasks * taskMul + block / 32 - 1) / (block / 32);
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(wantBlocks, (int64_t)std::max(occ, 1) * ctx->numSMs));
     ck<<<grid, block, smem, ctx->stream>>>(c);
     LAUNCHED(ctx);

@@ -12,7 +12,9 @@
 // RED route (ffm_pairs.cuh, 11 856 lane-REDs per 39-field row, each a read-modify-write of a cold line in DRAM)
 // this trades 95 KB/row of REDs for a second 95 KB/row of gathers, and every sum has one order: deterministic.
 // Needs what the pair route's AdaGrad mode needs -- no row with two nonzeros of one field (checked once per dataset
-// on the device) -- plus rows of at most 64 nonzeros and a contiguous row range.
+// on the device) -- and a contiguous row range.  Two column kernels: the tuned ffm_cols_grad_kernel<KT, E> (k in
+// {4, 8, 16}, nFields <= 64, rows of at most 64 nonzeros, d * nFields < 2^31) and ffm_cols_grad_generic_kernel<KT, E>
+// (every k and nFields, rows of any length, 64-bit offsets), which give the same bits where both run.
 #pragma once
 
 struct FfmColArgs {
@@ -31,6 +33,7 @@ struct FfmColArgs {
   const double *PT;          // the parameters in FIELD-major layout PT[f][j][s] (see ffm_field_major_kernel)
   double *gP, *gw, *partial;
   int fitLinear;
+  int k;                     // ffm_cols_grad_generic_kernel only: nComponents (fills the struct's tail padding)
 };
 
 static __device__ __forceinline__ int64_t lower_bound_row_i32(const int32_t *rows, int64_t lo, int64_t hi, int64_t r) {
@@ -232,3 +235,142 @@ __global__ void __launch_bounds__(256) ffm_cols_grad_kernel(const FfmColArgs a) 
     }
   }
 }
+
+// ffm_cols_grad_kernel with k and nFields at run time.  A task is (column segment, block of 32 fields, component
+// chunk of KT); one warp runs one task, lane <-> field fb*32 + lane, KT accumulators per lane.  Per batch of E entries
+// the warp reads each entry's row with coalesced loads (lane <-> position, steps of 32), takes the row's own field f_j
+// from the position whose feature is j (the lowest such position), and files the positions whose field lies in the
+// block as (x, j_u) in a table of 32 field slots: E x 32 x 12 B of shared memory per warp, whatever nFields, k or the
+// row length.  The row is read once per (field block, chunk) where the tuned kernel reads it once.  Partner vectors
+// come from PT[f_j][j_u][s0 .. s0+KT): 16-byte loads when k is even, scalar loads when it is odd; components past k
+// are masked, never read.  Per entry the arithmetic is the tuned kernel's (cx = coef*x_j, sc = cx*x_u, acc += sc*v)
+// in the same ascending row order, so where both run they produce the same bits.
+template <int KT, int E>
+__global__ void __launch_bounds__(128) ffm_cols_grad_generic_kernel(const FfmColArgs a) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  struct WarpScratch {
+    double x[E][32];
+    int32_t ju[E][32];   // the feature of the row's nonzero of field fb*32 + slot, -1: none
+  };
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  WarpScratch &ws = reinterpret_cast<WarpScratch *>(smem_raw)[wib];
+  const int nF = a.nFields, k = a.k;
+  const int64_t SB8 = (int64_t)nF * k;
+  const int NC = (k + KT - 1) / KT;
+  const int64_t per = (int64_t)((nF + 31) >> 5) * NC;
+  const int64_t nAll = a.nTasks * per;
+  const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + wib;
+  const int64_t nWarps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  for (int64_t q = warp; q < nAll; q += nWarps) {
+    const int64_t t = q / per;
+    const int rem = (int)(q - t * per);
+    const int fb = rem / NC, s0 = (rem - fb * NC) * KT;
+    const int f = fb * 32 + lane;
+    const int64_t j = a.taskCol[t];
+    int64_t eb = a.taskBeg[t], ee = eb + a.taskLen[t];
+    if ((int64_t)a.crow[eb] < a.rowBegin) eb = lower_bound_row_i32(a.crow, eb, ee, a.rowBegin);
+    if (eb < ee && (int64_t)a.crow[ee - 1] >= a.rowEnd) ee = lower_bound_row_i32(a.crow, eb, ee, a.rowEnd);
+    double acc[KT], accW = 0.0;
+#pragma unroll
+    for (int c = 0; c < KT; ++c) acc[c] = 0.0;
+    for (int64_t e0 = eb; e0 < ee; e0 += E) {
+      const int nb = (int)(ee - e0 < E ? ee - e0 : E);
+      int64_t rbL = 0;
+      int zL = 0;
+      double cxL = 0.0;
+      if (lane < nb) {
+        const int64_t e = e0 + lane, row = a.crow[e];
+        rbL = a.indptr[row];
+        zL = (int)(a.indptr[row + 1] - rbL);
+        cxL = a.coef[row - a.rowBegin] * a.cdata[e];
+      }
+      __syncwarp();   // the previous batch's readers are done with the scratch
+#pragma unroll
+      for (int i = 0; i < E; ++i) ws.ju[i][lane] = -1;
+      __syncwarp();
+      double cx[E];
+      int fj[E];
+#pragma unroll
+      for (int i = 0; i < E; ++i) {
+        const int64_t rb = __shfl_sync(0xffffffffu, rbL, i);
+        const int z = __shfl_sync(0xffffffffu, zL, i);
+        cx[i] = __shfl_sync(0xffffffffu, cxL, i);
+        fj[i] = -1;
+        for (int u0 = 0; u0 < z; u0 += 32) {   // z is 0 past nb
+          const int u = u0 + lane;
+          int32_t idx = -1;
+          int fld = 0;
+          if (u < z) {
+            idx = a.indices[rb + u];
+            fld = a.fields[rb + u];
+            const unsigned slot = (unsigned)(fld - fb * 32);
+            if (slot < 32u) {
+              ws.x[i][slot] = a.data[rb + u];
+              ws.ju[i][slot] = idx;
+            }
+          }
+          const unsigned hit = __ballot_sync(0xffffffffu, idx == (int32_t)j);
+          if (hit && fj[i] < 0) fj[i] = __shfl_sync(0xffffffffu, fld, __ffs(hit) - 1);
+        }
+      }
+      __syncwarp();
+      double v[E][KT], sc[E];
+#pragma unroll
+      for (int i = 0; i < E; ++i) {
+        sc[i] = 0.0;
+#pragma unroll
+        for (int c = 0; c < KT; ++c) v[i][c] = 0.0;
+        if (i < nb && f < nF && fj[i] >= 0) {
+          const int32_t ju = ws.ju[i][lane];
+          if (ju >= 0 && ju != (int32_t)j) {   // the reference pairs distinct features only
+            const double *src = a.PT + ((int64_t)fj[i] * a.d + ju) * k + s0;   // P[j_u][f_j][s0 ..]
+            if ((k & 1) == 0) {   // s0 and k even: 16-byte aligned pairs, both inside k or both past it
+#pragma unroll
+              for (int c = 0; c < KT / 2; ++c)
+                if (s0 + 2 * c < k) {
+                  const double2 p = __ldg(reinterpret_cast<const double2 *>(src) + c);
+                  v[i][2 * c] = p.x;
+                  v[i][2 * c + 1] = p.y;
+                }
+            } else {
+#pragma unroll
+              for (int c = 0; c < KT; ++c)
+                if (s0 + c < k) v[i][c] = __ldg(src + c);
+            }
+            sc[i] = cx[i] * ws.x[i][lane];
+          }
+        }
+      }
+#pragma unroll
+      for (int i = 0; i < E; ++i)   // entries in ascending row order
+#pragma unroll
+        for (int c = 0; c < KT; ++c) acc[c] += sc[i] * v[i][c];
+      if (lane == 0)
+#pragma unroll
+        for (int i = 0; i < E; ++i)
+          if (i < nb) accW += cx[i];
+    }
+    const int slot = a.taskSlot[t];
+    double *dst = slot < 0 ? a.gP + j * SB8 : a.partial + (size_t)slot * (SB8 + 1);
+    if (f < nF) {
+#pragma unroll
+      for (int c = 0; c < KT; ++c) {
+        if (s0 + c >= k) break;
+        if (slot < 0) dst[(int64_t)f * k + s0 + c] += acc[c];
+        else dst[(int64_t)f * k + s0 + c] = acc[c];
+      }
+    }
+    if (lane == 0 && fb == 0 && s0 == 0) {   // one task per segment owns the linear term
+      if (slot < 0) { if (a.fitLinear) a.gw[j] += accW; }
+      else dst[SB8] = accW;
+    }
+  }
+}
+
+// the component chunk of ffm_cols_grad_generic_kernel: lanes map to fields, so there are no idle lanes to weigh; the
+// narrowest width that holds k in one chunk wastes the fewest accumulator registers, and k > 32 takes chunks of 32
+// (the widest instance that does not spill)
+static inline int ffm_cols_generic_kt(int k) { return k <= 4 ? 4 : k <= 8 ? 8 : k <= 16 ? 16 : 32; }
+
+// bytes of shared scratch one warp of ffm_cols_grad_generic_kernel<KT, E> needs (must match its WarpScratch)
+static inline size_t ffm_cols_generic_warp_smem(int E) { return (size_t)E * 32 * (8 + 4); }
