@@ -30,7 +30,8 @@ struct nimfm_ctx {
   size_t partialsCap = 0;
   double *stash = nullptr;     // deterministic gradient (fm_cols.cu): per-row stash records + segment partials
   size_t stashCap = 0;
-  double *scalars = nullptr;   // small device scalar block (64 doubles)
+  struct nimfm_mb_index *mbIndex = nullptr;   // deterministic AdaGrad: the column index of the current minibatch
+  double *scalars = nullptr;  // small device scalar block (64 doubles)
   double *hostScalars = nullptr;  // pinned mirror
   int64_t *idxScratch = nullptr;  // device copy of host-provided row ids
   size_t idxCap = 0;
@@ -111,6 +112,12 @@ struct nimfm_ctx {
 void nimfm_trace_begin(nimfm_ctx *ctx, const char *tag);
 void nimfm_trace_end(nimfm_ctx *ctx);
 void nimfm_trace_report(nimfm_ctx *ctx, const char *what);
+struct TraceReport {   // reports (and releases) the spans recorded since the last report on every exit path
+  nimfm_ctx *ctx;
+  const char *what;
+  bool on;
+  ~TraceReport() { if (on) nimfm_trace_report(ctx, what); }
+};
 
 struct nimfm_dataset;
 // fm_cols.cu: the CSC twin of a CSR dataset (stable transpose: rows ascending inside a column) and its columns cut
@@ -145,6 +152,47 @@ struct nimfm_dataset {
   // CD only: runs of consecutive columns with pairwise-disjoint row support (built at cd_begin)
   std::vector<int64_t> cdBatchStart;
 };
+
+// dataset_ops.cu: buffers of the stable sort behind nimfm_dataset_transpose, owned by the caller
+struct TransposeScratch {
+  int32_t *segOf, *keysOut;
+  uint32_t *permIn, *permOut;
+  void *tmp;          // CUB scratch; nullptr: nimfm_transpose_sort only sets tmpBytes
+  size_t tmpBytes;
+};
+int nimfm_transpose_sort(nimfm_ctx *ctx, int64_t nsIn, int64_t nsOut, int64_t nnz, const int64_t *inPtr,
+                         const int32_t *inIdx, const double *inData, TransposeScratch *s, double *outData,
+                         int32_t *outIdx, int64_t *outPtr);
+
+// dataset_ops.cu: the column index of ONE minibatch (rows rowIdx[0 .. B) or rowBegin .. rowBegin + B - 1), built on
+// the device for the deterministic AdaGrad epochs.  view: the B rows gathered into a CSR (CSR-field) dataset that keeps
+// the parent's d, nFields, maxSegNnz, hot table and field-repeat flag; csc: its stable column-major twin, whose
+// indices are positions 0 .. B-1 in the view (a row listed twice gives two positions); tw: that twin's 512-entry
+// segments in the dataset twin's layout (dummy columns d + a span all B positions).  Held by the context, grown on
+// demand, rebuilt per minibatch; view, csc and tw only point into the buffers below.
+struct nimfm_mb_index {
+  nimfm_dataset view, csc;
+  nimfm_det_twin tw;
+  double *bias = nullptr;   // [1]: the intercept the minibatch's forward pass sees (AdaGrad refreshes it from g_sum)
+  int64_t *rows = nullptr, *rowLen = nullptr, *ptr = nullptr, *cPtr = nullptr, *colCnt = nullptr, *tot = nullptr;
+  int64_t *hostTot = nullptr;   // pinned: entries, tasks, multi-segment columns, partial slots
+  double *data = nullptr, *y = nullptr, *cData = nullptr;
+  double *yhat = nullptr;       // [B] scratch for the forward pass's decision values
+  int32_t *idx = nullptr, *fld = nullptr, *cIdx = nullptr, *segOf = nullptr, *keysOut = nullptr;
+  uint32_t *permIn = nullptr, *permOut = nullptr;
+  unsigned char *tmp = nullptr;
+  long long *segOff = nullptr;   // per-column segment counts and their exclusive scan
+  int32_t *taskCol = nullptr, *taskLen = nullptr, *taskSlot = nullptr, *multiCol = nullptr, *multiFirst = nullptr,
+          *multiCount = nullptr;
+  int64_t *taskBeg = nullptr;
+  size_t capRows = 0, capRowLen = 0, capPtr = 0, capY = 0, capCol = 0, capColPtr = 0, capSeg = 0, capTot = 0,
+         capBias = 0, capYhat = 0, capTmp = 0, capData = 0, capIdx = 0, capCData = 0, capCIdx = 0, capSegOf = 0, capKeys = 0,
+         capPermIn = 0, capPermOut = 0, capFld = 0, capTaskCol = 0, capTaskBeg = 0, capTaskLen = 0, capTaskSlot = 0,
+         capMultiCol = 0, capMultiFirst = 0, capMultiCount = 0;
+};
+int nimfm_mb_index_build(nimfm_ctx *ctx, const nimfm_dataset *X, int nAug, int64_t rowBegin, int64_t nRows,
+                         const int32_t *rowIdx, nimfm_mb_index **out);
+void nimfm_mb_index_free(nimfm_mb_index *m);
 
 struct nimfm_fm {
   int degree = 2, k = 1, nOrders = 1, nAug = 0;

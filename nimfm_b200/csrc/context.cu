@@ -147,6 +147,7 @@ int32_t nimfm_ctx_destroy(nimfm_ctx *ctx) {
   if (ctx->comm && g_nccl.commDestroy) g_nccl.commDestroy(ctx->comm);
   cudaFree(ctx->partials);
   cudaFree(ctx->stash);
+  nimfm_mb_index_free(ctx->mbIndex);
   cudaFree(ctx->scalars);
   cudaFree(ctx->idxScratch);
   cudaFree(ctx->idx32Scratch);

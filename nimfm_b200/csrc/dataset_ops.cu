@@ -209,6 +209,254 @@ int alloc_arrays(nimfm_ctx *ctx, nimfm_dataset *o, int64_t nSeg, int64_t nnz, bo
 
 }  // namespace
 
+// The stable sort at the core of nimfm_dataset_transpose: the nnz entries of nsIn input segments (inPtr, inIdx = the
+// other axis, inData) sorted by inIdx with a stable radix sort, so entries of one output segment keep input order ->
+// outData, outIdx (the input segment of each entry) and outPtr[0 .. nsOut].  All buffers are the caller's.  With
+// s->tmp == nullptr it only sets s->tmpBytes, the CUB scratch the call needs, and launches nothing.
+int nimfm_transpose_sort(nimfm_ctx *ctx, int64_t nsIn, int64_t nsOut, int64_t nnz, const int64_t *inPtr,
+                         const int32_t *inIdx, const double *inData, TransposeScratch *s, double *outData,
+                         int32_t *outIdx, int64_t *outPtr) {
+  int endBit = 1;
+  while (endBit < 31 && ((int64_t)1 << endBit) < nsOut) endBit++;
+  if (!s->tmp) {
+    s->tmpBytes = 0;
+    if (nnz > 0)
+      CK(cub::DeviceRadixSort::SortPairs(nullptr, s->tmpBytes, inIdx, s->keysOut, s->permIn, s->permOut, (int)nnz, 0,
+                                         endBit, ctx->stream));
+    return NIMFM_OK;
+  }
+  if (nnz > 0) {
+    expand_seg_ids_kernel<<<grid_for(ctx, nsIn * 32), 256, 0, ctx->stream>>>(inPtr, nsIn, s->segOf);
+    iota_kernel<<<grid_for(ctx, nnz), 256, 0, ctx->stream>>>(s->permIn, nnz);
+    ctx->launches += 2;
+    size_t tmpBytes = s->tmpBytes;
+    CK(cub::DeviceRadixSort::SortPairs(s->tmp, tmpBytes, inIdx, s->keysOut, s->permIn, s->permOut, (int)nnz, 0, endBit,
+                                       ctx->stream));
+    permute_gather_kernel<<<grid_for(ctx, nnz), 256, 0, ctx->stream>>>(s->permOut, nnz, inData, s->segOf, outData,
+                                                                      outIdx);
+    LAUNCHED(ctx);
+  }
+  lower_bound_ptr_kernel<<<grid_for(ctx, nsOut + 1), 256, 0, ctx->stream>>>(s->keysOut, nnz, nsOut, outPtr);
+  LAUNCHED(ctx);
+  return NIMFM_OK;
+}
+
+// ------------------------------------------------------------------ the column index of one minibatch
+// nimfm_mb_index_build (common.cuh).  Everything below runs on the stream; the host reads back four counts once.
+namespace {
+
+constexpr int MB_SEG = 512;   // entries per column segment: the SEG of the dataset twin (fm_cols.cu)
+
+struct SegCount {   // per column: segments (tasks), 1 if the column has several, partial slots
+  long long tasks, multi, slots;
+};
+struct SegCountSum {
+  __host__ __device__ SegCount operator()(const SegCount &a, const SegCount &b) const {
+    return {a.tasks + b.tasks, a.multi + b.multi, a.slots + b.slots};
+  }
+};
+
+// one warp per minibatch position q: its source row, its length, and the per-column entry counts (hot columns of the
+// dataset are counted in shared memory first, as in adagrad_count_kernel, so they do not serialise on one counter)
+__global__ void mb_rows_kernel(const int64_t *indptr, const int32_t *indices, int64_t rowBegin, int64_t nRows,
+                               const int32_t *rowIdx, int64_t *rows, int64_t *len, int64_t *colCnt,
+                               const uint8_t *hotSlot, const int32_t *hotList, int nHot) {
+  __shared__ unsigned long long hotCnt[16];
+  if (threadIdx.x < 16) hotCnt[threadIdx.x] = 0;
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
+  const int64_t nWarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t q = warp; q < nRows; q += nWarps) {
+    const int64_t r = rowIdx ? (int64_t)rowIdx[q] : rowBegin + q;
+    if (lane == 0) {
+      rows[q] = r;
+      len[q] = indptr[r + 1] - indptr[r];
+    }
+    for (int64_t e = indptr[r] + lane; e < indptr[r + 1]; e += 32) {
+      const int32_t j = indices[e];
+      const int slot = (hotSlot && nHot > 0) ? hotSlot[j] : 255;
+      if (slot != 255) atomicAdd(&hotCnt[slot], 1ull);
+      else atomicAdd(reinterpret_cast<unsigned long long *>(colCnt + j), 1ull);
+    }
+  }
+  if (warp == 0 && lane == 0) len[nRows] = 0;
+  __syncthreads();
+  if ((int)threadIdx.x < nHot && hotCnt[threadIdx.x] > 0)
+    atomicAdd(reinterpret_cast<unsigned long long *>(colCnt + hotList[threadIdx.x]), hotCnt[threadIdx.x]);
+}
+
+// per column j < d + nAug (dummy columns d + a hold every position): its segment counts; entry d + nAug is zero so
+// that the exclusive scan ends with the totals
+__global__ void mb_seg_count_kernel(const int64_t *colCnt, int64_t d, int nAug, int64_t nRows, SegCount *out) {
+  const int64_t dd = d + nAug;
+  for (int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j <= dd; j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t L = j < d ? colCnt[j] : (j < dd ? nRows : 0);
+    const long long nseg = (L + MB_SEG - 1) / MB_SEG;
+    out[j] = {nseg, nseg > 1 ? 1 : 0, nseg > 1 ? nseg : 0};
+  }
+}
+
+__global__ void mb_totals_kernel(const int64_t *viewPtr, int64_t nRows, const SegCount *off, int64_t dd, int64_t *tot) {
+  tot[0] = viewPtr[nRows];
+  tot[1] = off[dd].tasks;
+  tot[2] = off[dd].multi;
+  tot[3] = off[dd].slots;
+}
+
+// the segment table in the dataset twin's layout (build_twin, fm_cols.cu), one thread per column
+__global__ void mb_seg_table_kernel(const int64_t *colPtr, int64_t d, int nAug, int64_t nRows, const SegCount *off,
+                                    int32_t *taskCol, int64_t *taskBeg, int32_t *taskLen, int32_t *taskSlot,
+                                    int32_t *multiCol, int32_t *multiFirst, int32_t *multiCount) {
+  const int64_t dd = d + nAug;
+  for (int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j < dd; j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t b = j < d ? colPtr[j] : 0, e = j < d ? colPtr[j + 1] : nRows;
+    const SegCount o = off[j];
+    const int64_t nseg = (e - b + MB_SEG - 1) / MB_SEG;
+    if (nseg > 1) {
+      multiCol[o.multi] = (int32_t)j;
+      multiFirst[o.multi] = (int32_t)o.slots;
+      multiCount[o.multi] = (int32_t)nseg;
+    }
+    for (int64_t s = 0; s < nseg; s++) {
+      const int64_t t = o.tasks + s;
+      taskCol[t] = (int32_t)j;
+      taskBeg[t] = b + s * MB_SEG;
+      const int64_t left = e - (b + s * MB_SEG);
+      taskLen[t] = (int32_t)(left < MB_SEG ? left : MB_SEG);
+      taskSlot[t] = nseg > 1 ? (int32_t)(o.slots + s) : -1;
+    }
+  }
+}
+
+// grow *p to hold n elements of T (contents are not kept)
+template <class T>
+int grow(nimfm_ctx *ctx, T **p, size_t &cap, size_t n) {
+  if (n <= cap && *p) return NIMFM_OK;
+  n = std::max<size_t>(n + n / 4, 16);
+  CK(cudaFree(*p));
+  *p = nullptr;
+  cap = 0;
+  if (cudaMalloc(p, n * sizeof(T)) != cudaSuccess) {
+    (void)cudaGetLastError();   // not sticky: the caller reports it
+    *p = nullptr;
+    return nimfm_fail(ctx, NIMFM_ERR_CUDA, "the minibatch column index could not allocate %zu bytes", n * sizeof(T));
+  }
+  cap = n;
+  return NIMFM_OK;
+}
+
+}  // namespace
+
+void nimfm_mb_index_free(nimfm_mb_index *m) {
+  if (!m) return;
+  void *bufs[] = {m->rows, m->rowLen, m->ptr, m->data, m->idx, m->fld, m->y, m->cPtr, m->cData, m->cIdx, m->segOf,
+                  m->keysOut, m->permIn, m->permOut, m->tmp, m->colCnt, m->segOff, m->taskCol, m->taskBeg, m->taskLen,
+                  m->taskSlot, m->multiCol, m->multiFirst, m->multiCount, m->tot, m->bias, m->yhat};
+  for (void *p : bufs) cudaFree(p);
+  cudaFreeHost(m->hostTot);
+  delete m;
+}
+
+int nimfm_mb_index_build(nimfm_ctx *ctx, const nimfm_dataset *X, int nAug, int64_t rowBegin, int64_t nRows,
+                         const int32_t *rowIdx, nimfm_mb_index **out) {
+  REQUIRE(X->kind == NIMFM_DS_CSR || X->kind == NIMFM_DS_CSR_FIELD, "the minibatch column index needs a CSR dataset");
+  REQUIRE(nRows >= 0 && (rowIdx || (rowBegin >= 0 && rowBegin + nRows <= X->n)), "bad minibatch rows");
+  if (!ctx->mbIndex) ctx->mbIndex = new nimfm_mb_index();
+  nimfm_mb_index *m = ctx->mbIndex;
+  const int64_t d = X->d, dd = d + nAug, B = nRows;
+  int rc;
+  // 1. rows, lengths and column counts of the minibatch; its indptr and the segment counts by two scans
+  if ((rc = grow(ctx, &m->rows, m->capRows, (size_t)B + 1)) || (rc = grow(ctx, &m->rowLen, m->capRowLen, (size_t)B + 1)) ||
+      (rc = grow(ctx, &m->ptr, m->capPtr, (size_t)B + 1)) || (rc = grow(ctx, &m->y, m->capY, (size_t)B + 1)) ||
+      (rc = grow(ctx, &m->colCnt, m->capCol, (size_t)d + 1)) || (rc = grow(ctx, &m->cPtr, m->capColPtr, (size_t)d + 1)) ||
+      (rc = grow(ctx, &m->segOff, m->capSeg, 6 * ((size_t)dd + 1))) || (rc = grow(ctx, &m->tot, m->capTot, 4)) ||
+      (rc = grow(ctx, &m->bias, m->capBias, 1)) || (rc = grow(ctx, &m->yhat, m->capYhat, (size_t)B + 1)))
+    return rc;
+  if (!m->hostTot) CK(cudaMallocHost(&m->hostTot, 4 * sizeof(int64_t)));
+  SegCount *cnt = reinterpret_cast<SegCount *>(m->segOff), *off = cnt + dd + 1;
+  CK(cudaMemsetAsync(m->colCnt, 0, (size_t)d * 8, ctx->stream));
+  mb_rows_kernel<<<grid_for(ctx, B * 32), 256, 0, ctx->stream>>>(X->indptr, X->indices, rowBegin, B, rowIdx, m->rows,
+                                                                m->rowLen, m->colCnt, X->hotSlot, X->hotList, X->nHot);
+  LAUNCHED(ctx);
+  mb_seg_count_kernel<<<grid_for(ctx, dd + 1), 256, 0, ctx->stream>>>(m->colCnt, d, nAug, B, cnt);
+  LAUNCHED(ctx);
+  size_t scanRows = 0, scanSeg = 0;
+  CK(cub::DeviceScan::ExclusiveSum(nullptr, scanRows, m->rowLen, m->ptr, B + 1, ctx->stream));
+  CK(cub::DeviceScan::ExclusiveScan(nullptr, scanSeg, cnt, off, SegCountSum(), SegCount{0, 0, 0}, dd + 1, ctx->stream));
+  if ((rc = grow(ctx, &m->tmp, m->capTmp, std::max(scanRows, scanSeg)))) return rc;
+  size_t tb = m->capTmp;
+  CK(cub::DeviceScan::ExclusiveSum(m->tmp, tb, m->rowLen, m->ptr, B + 1, ctx->stream));
+  tb = m->capTmp;
+  CK(cub::DeviceScan::ExclusiveScan(m->tmp, tb, cnt, off, SegCountSum(), SegCount{0, 0, 0}, dd + 1, ctx->stream));
+  mb_totals_kernel<<<1, 1, 0, ctx->stream>>>(m->ptr, B, off, dd, m->tot);
+  LAUNCHED(ctx);
+  // the one device-to-host copy of the minibatch: the entry count and the segment-table sizes
+  CK(cudaMemcpyAsync(m->hostTot, m->tot, 4 * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  const int64_t nnz = m->hostTot[0], nTasks = m->hostTot[1], nMulti = m->hostTot[2], nSlots = m->hostTot[3];
+  if (nnz > (int64_t)2147483647)
+    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
+                      "a minibatch of %lld rows holds %lld nonzeros; the minibatch column index sorts with 32-bit "
+                      "values and takes at most 2147483647 (use a smaller miniBatchSize)",
+                      (long long)B, (long long)nnz);
+  if (nSlots > (int64_t)2147483647)
+    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "too many column segments in one minibatch (%lld)", (long long)nSlots);
+  // 2. the gathered rows (the view) and their stable column-major twin
+  const size_t e = (size_t)nnz + 1;
+  if ((rc = grow(ctx, &m->data, m->capData, e)) || (rc = grow(ctx, &m->idx, m->capIdx, e)) ||
+      (rc = grow(ctx, &m->cData, m->capCData, e)) || (rc = grow(ctx, &m->cIdx, m->capCIdx, e)) ||
+      (rc = grow(ctx, &m->segOf, m->capSegOf, e)) || (rc = grow(ctx, &m->keysOut, m->capKeys, e)) ||
+      (rc = grow(ctx, &m->permIn, m->capPermIn, e)) || (rc = grow(ctx, &m->permOut, m->capPermOut, e)) ||
+      (X->fields && (rc = grow(ctx, &m->fld, m->capFld, e))) ||
+      (rc = grow(ctx, &m->taskCol, m->capTaskCol, (size_t)nTasks + 1)) ||
+      (rc = grow(ctx, &m->taskBeg, m->capTaskBeg, (size_t)nTasks + 1)) ||
+      (rc = grow(ctx, &m->taskLen, m->capTaskLen, (size_t)nTasks + 1)) ||
+      (rc = grow(ctx, &m->taskSlot, m->capTaskSlot, (size_t)nTasks + 1)) ||
+      (rc = grow(ctx, &m->multiCol, m->capMultiCol, (size_t)nMulti + 1)) ||
+      (rc = grow(ctx, &m->multiFirst, m->capMultiFirst, (size_t)nMulti + 1)) ||
+      (rc = grow(ctx, &m->multiCount, m->capMultiCount, (size_t)nMulti + 1)))
+    return rc;
+  if (B > 0) {
+    gather_rows_kernel<<<grid_for(ctx, B * 32), 256, 0, ctx->stream>>>(
+        X->indptr, m->ptr, m->rows, B, X->data, X->indices, X->fields, m->data, m->idx, m->fld, X->y, m->y);
+    LAUNCHED(ctx);
+  }
+  TransposeScratch s{m->segOf, m->keysOut, m->permIn, m->permOut, nullptr, 0};
+  if ((rc = nimfm_transpose_sort(ctx, B, d, nnz, m->ptr, m->idx, m->data, &s, m->cData, m->cIdx, m->cPtr)))
+    return rc;
+  if ((rc = grow(ctx, &m->tmp, m->capTmp, s.tmpBytes))) return rc;
+  s.tmp = m->tmp;
+  s.tmpBytes = m->capTmp;
+  if ((rc = nimfm_transpose_sort(ctx, B, d, nnz, m->ptr, m->idx, m->data, &s, m->cData, m->cIdx, m->cPtr)))
+    return rc;
+  // 3. the segment table
+  if (dd > 0) {
+    mb_seg_table_kernel<<<grid_for(ctx, dd), 256, 0, ctx->stream>>>(m->cPtr, d, nAug, B, off, m->taskCol, m->taskBeg,
+                                                                    m->taskLen, m->taskSlot, m->multiCol, m->multiFirst,
+                                                                    m->multiCount);
+    LAUNCHED(ctx);
+  }
+  CK(cudaGetLastError());
+  // the view keeps the parent's shape and planning facts (maxSegNnz picks the same row kernels), hot table and
+  // field-repeat flag; the view, the twin and the table only point into the buffers above
+  nimfm_dataset &v = m->view;
+  v.kind = X->kind; v.n = B; v.d = d; v.nnz = nnz; v.nFields = X->nFields; v.maxSegNnz = X->maxSegNnz;
+  v.data = m->data; v.indices = m->idx; v.indptr = m->ptr; v.fields = X->fields ? m->fld : nullptr;
+  v.y = X->y ? m->y : nullptr;
+  v.hotSlot = X->hotSlot; v.hotList = X->hotList; v.nHot = X->nHot; v.fieldDup = X->fieldDup;
+  nimfm_dataset &c = m->csc;
+  c.kind = NIMFM_DS_CSC; c.n = B; c.d = d; c.nnz = nnz;
+  c.data = m->cData; c.indices = m->cIdx; c.indptr = m->cPtr;
+  nimfm_det_twin &t = m->tw;
+  t.csc = &m->csc;
+  t.taskCol = m->taskCol; t.taskBeg = m->taskBeg; t.taskLen = m->taskLen; t.taskSlot = m->taskSlot;
+  t.multiCol = m->multiCol; t.multiFirst = m->multiFirst; t.multiCount = m->multiCount;
+  t.nTasks = nTasks; t.nMulti = nMulti; t.nSlots = nSlots; t.nAug = nAug;
+  *out = m;
+  return NIMFM_OK;
+}
+
 extern "C" {
 
 // X[indicesRow] for CSRDataset / CSRFieldDataset (dataset.nim:319-367 -> tensor/sparse.nim:263-285);
@@ -402,24 +650,15 @@ int32_t nimfm_dataset_transpose(nimfm_ctx *ctx, const nimfm_dataset *in, nimfm_d
   CK(cudaMalloc(&keysOut.p, n4));
   CK(cudaMalloc(&permIn.p, n4));
   CK(cudaMalloc(&permOut.p, n4));
-  if (nnz > 0) {
-    expand_seg_ids_kernel<<<grid_for(ctx, nsIn * 32), 256, 0, ctx->stream>>>(in->indptr, nsIn, segOf.as<int32_t>());
-    iota_kernel<<<grid_for(ctx, nnz), 256, 0, ctx->stream>>>(permIn.as<uint32_t>(), nnz);
-    ctx->launches += 2;
-    int endBit = 1;
-    while (endBit < 31 && ((int64_t)1 << endBit) < nsOut) endBit++;
-    size_t tmpBytes = 0;
-    CK(cub::DeviceRadixSort::SortPairs(nullptr, tmpBytes, in->indices, keysOut.as<int32_t>(), permIn.as<uint32_t>(),
-                                       permOut.as<uint32_t>(), (int)nnz, 0, endBit, ctx->stream));
-    CK(cudaMalloc(&tmp.p, tmpBytes ? tmpBytes : 16));
-    CK(cub::DeviceRadixSort::SortPairs(tmp.p, tmpBytes, in->indices, keysOut.as<int32_t>(), permIn.as<uint32_t>(),
-                                       permOut.as<uint32_t>(), (int)nnz, 0, endBit, ctx->stream));
-    permute_gather_kernel<<<grid_for(ctx, nnz), 256, 0, ctx->stream>>>(permOut.as<uint32_t>(), nnz, in->data,
-                                                                      segOf.as<int32_t>(), o->data, o->indices);
-    LAUNCHED(ctx);
-  }
-  lower_bound_ptr_kernel<<<grid_for(ctx, nsOut + 1), 256, 0, ctx->stream>>>(keysOut.as<int32_t>(), nnz, nsOut, o->indptr);
-  LAUNCHED(ctx);
+  TransposeScratch s{segOf.as<int32_t>(), keysOut.as<int32_t>(), permIn.as<uint32_t>(), permOut.as<uint32_t>(), nullptr, 0};
+  if ((rc = nimfm_transpose_sort(ctx, nsIn, nsOut, nnz, in->indptr, in->indices, in->data, &s, o->data, o->indices,
+                                 o->indptr)))
+    return rc;
+  CK(cudaMalloc(&tmp.p, s.tmpBytes ? s.tmpBytes : 16));
+  s.tmp = tmp.p;
+  if ((rc = nimfm_transpose_sort(ctx, nsIn, nsOut, nnz, in->indptr, in->indices, in->data, &s, o->data, o->indices,
+                                 o->indptr)))
+    return rc;
   if (in->y) {
     CK(cudaMalloc(&o->y, (size_t)std::max<int64_t>(o->n, 1) * 8));
     CK(cudaMemcpyAsync(o->y, in->y, (size_t)o->n * 8, cudaMemcpyDeviceToDevice, ctx->stream));

@@ -414,6 +414,45 @@ static __global__ void adagrad_scalar_kernel(double *b, double *adaScal, const d
   scal[0] += part[0];
   scal[1] += viol;
 }
+
+// coef_i = dloss(y_i, yhat_i) / mb in place of yhat (a forward kernel's output), and the loss / sum coef / sum dL^2
+// partials per block: their order depends on nRows and the grid only, not on the forward kernel (the column routes)
+static __global__ void dloss_coef_kernel(double *yhatCoef, const double *y, int64_t rowBegin, int64_t nRows, int loss,
+                                         double thr, double mb, double *partials) {
+  __shared__ double red[8];
+  double l = 0.0, c = 0.0, d2 = 0.0;
+  for (int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; q < nRows; q += (int64_t)gridDim.x * blockDim.x) {
+    const double yi = y[rowBegin + q], yh = yhatCoef[q];
+    const double dL = dev_dloss(loss, thr, yi, yh);
+    l += dev_loss(loss, thr, yi, yh);
+    c += dL / mb;
+    d2 += dL * dL;
+    yhatCoef[q] = dL / mb;
+  }
+  l = block_sum(l, red);
+  __syncthreads();
+  c = block_sum(c, red);
+  __syncthreads();
+  d2 = block_sum(d2, red);
+  if (threadIdx.x == 0) {
+    partials[blockIdx.x * 4 + 0] = l;
+    partials[blockIdx.x * 4 + 1] = c;
+    partials[blockIdx.x * 4 + 2] = d2;
+    partials[blockIdx.x * 4 + 3] = 0.0;
+  }
+}
+
+// the intercept every row of an AdaGrad minibatch sees (adagrad.nim:101-105), written to *out for a forward pass that
+// reads its intercept from memory: the same expression as the AdaGrad row kernels' prologue (fm_rows.cuh, ffm.cu)
+static __global__ void adagrad_bias_kernel(double *out, const double *b, const double *adaScal, int fitIntercept,
+                                           int first, double eta0, double tIt, double alpha0) {
+  double bias = b[0];
+  if (!first && fitIntercept) {
+    const double den = sqrt(adaScal[1]) + eta0 * tIt * alpha0;
+    bias = -eta0 * adaScal[0] / den;
+  }
+  *out = bias;
+}
 // AdaGrad.finalize (adagrad.nim:65-84)
 static __global__ void adagrad_finalize_kernel(double *P, const double *gsP, const double *gnP, int64_t nP, double *w,
                                         const double *gsw, const double *gnw, int64_t d, int fitLinear,

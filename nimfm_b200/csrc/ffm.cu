@@ -669,52 +669,60 @@ static bool ffm_cols_default(int64_t nRows) { (void)nRows; return false; }
 // equals the register-limited occupancy of the 112 / 126-register instances and lies above that of the 200 /
 // 225-register ones (2), so it changes no launch; the tests size their data past three waves of this bound.
 #define FFM_COLS_GENERIC_BLOCKS_PER_SM 4
-static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int loss, double thr,
-                                int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb, bool must,
-                                int *taken) {
-  *taken = 0;
+// where the column route's outputs go (ffm_det_pass)
+struct FfmDetTargets {
+  double *gP, *gw;       // gradient sums (the model's gradient, g_sum or its delta block)
+  double *gnP, *gnw;     // AdaGrad: sums of squared gradients; nullptr: plain gradient
+  double *red4;          // (loss, sum coef, sum dL^2, -)
+  const double *b;       // the intercept the forward pass sees
+};
+
+// AdaGrad's generic column-kernel width: ffm_cols_generic_kt, but k > 16 takes chunks of 16 -- the square accumulators
+// do not fit beside 32 components per lane without spills (ptxas)
+static inline int ffm_cols_ada_kt(int k) { return k <= 4 ? 4 : k <= 8 ? 8 : 16; }
+
+// the two passes of the column route over rows [rowBegin, rowBegin + nRows) of X with X's column twin tw (row ids
+// X's): the forward kernel and dloss_coef_kernel, then the tuned column kernel (tunedKernel) or the generic one
+static int ffm_det_pass(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, const nimfm_det_twin *tw, int loss,
+                        double thr, int64_t rowBegin, int64_t nRows, double mb, bool tunedKernel,
+                        const FfmDetTargets &o) {
   typedef void (*ColKern)(const FfmColArgs);
   constexpr int E = 4;   // column entries in flight per warp
-  ColKern ck = m->k == 4 ? ffm_cols_grad_kernel<4, E> : m->k == 8 ? ffm_cols_grad_kernel<8, E>
-               : m->k == 16 ? ffm_cols_grad_kernel<16, E> : (ColKern) nullptr;
-  const int CH = (int)std::max<int64_t>(X->maxSegNnz, 1);
-  const bool contiguous = !rowIdxDev && rowBegin >= 0 && rowBegin + nRows <= X->n;
-  const bool tunedShape = ck && CH <= 64 && m->nFields <= 64 && m->d * m->nFields < (int64_t)2147483647;
-  if (!contiguous || !(tunedShape || must)) {
-    if (must)
-      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
-                        "the deterministic FFM gradient needs a contiguous row range (no row list, no wrap-around)");
-    return NIMFM_OK;
-  }
-  bool dups = true;
-  int rc;
-  if ((rc = ffm_has_field_dups(ctx, X, &dups))) return rc;
-  if (dups) {
-    if (must)
-      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic FFM gradient needs rows with one nonzero per "
-                        "field (a row of this dataset repeats a field)");
-    return NIMFM_OK;
-  }
-  const char *envC = getenv("NIMFM_FFM_COLS");
-  const bool generic = !tunedShape || (envC && !strcmp(envC, "generic"));
+  const bool ada = o.gnP != nullptr;
+  ColKern ck = nullptr;
   size_t warpSmem = ffm_cols_warp_smem(E);
   int64_t taskMul = 1;   // warp tasks per column segment
-  if (generic) {
-    const int kt = ffm_cols_generic_kt(m->k);
+  if (tunedKernel && !ada) {
+    ck = m->k == 4 ? ffm_cols_grad_kernel<4, E> : m->k == 8 ? ffm_cols_grad_kernel<8, E> : ffm_cols_grad_kernel<16, E>;
+  } else if (tunedKernel) {
+    // AdaGrad: at k = 16 two entries in flight leave room for the square accumulators (ptxas)
+    ck = m->k == 4 ? ffm_cols_grad_kernel<4, E, true> : m->k == 8 ? ffm_cols_grad_kernel<8, E, true>
+                                                                  : ffm_cols_grad_kernel<16, 2, true>;
+    warpSmem = ffm_cols_warp_smem(m->k == 16 ? 2 : E);
+  } else {
+    const int kt = ada ? ffm_cols_ada_kt(m->k) : ffm_cols_generic_kt(m->k);
     int gE;
-    switch (kt) {   // entries per batch: the most without spills (ptxas), 24-64 partner components per lane in flight
-      case 4: ck = ffm_cols_grad_generic_kernel<4, 6>; gE = 6; break;
-      case 8: ck = ffm_cols_grad_generic_kernel<8, 4>; gE = 4; break;
-      case 16: ck = ffm_cols_grad_generic_kernel<16, 4>; gE = 4; break;
-      default: ck = ffm_cols_grad_generic_kernel<32, 2>; gE = 2; break;
+    if (!ada) {
+      switch (kt) {   // entries per batch: the most without spills (ptxas), 24-64 partner components per lane in flight
+        case 4: ck = ffm_cols_grad_generic_kernel<4, 6>; gE = 6; break;
+        case 8: ck = ffm_cols_grad_generic_kernel<8, 4>; gE = 4; break;
+        case 16: ck = ffm_cols_grad_generic_kernel<16, 4>; gE = 4; break;
+        default: ck = ffm_cols_grad_generic_kernel<32, 2>; gE = 2; break;
+      }
+    } else {
+      switch (kt) {   // the same entries per batch as the gradient's instances: still no spills (ptxas)
+        case 4: ck = ffm_cols_grad_generic_kernel<4, 6, true>; gE = 6; break;
+        case 8: ck = ffm_cols_grad_generic_kernel<8, 4, true>; gE = 4; break;
+        default: ck = ffm_cols_grad_generic_kernel<16, 4, true>; gE = 4; break;
+      }
     }
     warpSmem = ffm_cols_generic_warp_smem(gE);
     taskMul = (m->nFields + 31) / 32 * ((m->k + kt - 1) / kt);   // (segment, block of 32 fields, component chunk)
   }
-  nimfm_det_twin *tw = nullptr;
-  if ((rc = nimfm_det_twin_get(ctx, X, 0, &tw))) return rc;
+  int rc;
   const int SB8 = (int)(m->nFields * m->k);
-  const size_t need = (size_t)std::max<int64_t>(nRows, 1) + (size_t)tw->nSlots * (SB8 + 1) + 16;
+  const size_t slotLen = (size_t)(ada ? 2 : 1) * (SB8 + 1);
+  const size_t need = (size_t)std::max<int64_t>(nRows, 1) + (size_t)tw->nSlots * slotLen + 16;
   if (ctx->stashCap < need) {
     CK(cudaStreamSynchronize(ctx->stream));
     if (ctx->stash) CK(cudaFree(ctx->stash));
@@ -735,29 +743,31 @@ static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_datase
   if ((rc = ffm_plan_mode(ctx, m, X, nRows, FFM_PREDICT, &pl))) return rc;
   FfmArgs a;
   ffm_fill_args(a, m, X);
+  a.b = o.b;
   a.rowBegin = rowBegin; a.nRows = nRows; a.yOut = ctx->stash; a.CH = pl.CH;
   pl.kern<<<pl.grid, pl.block, pl.smem, ctx->stream>>>(a);
   LAUNCHED(ctx);
   const int cgrid = (int)std::max<int64_t>(1, std::min<int64_t>((nRows + 255) / 256, (int64_t)ctx->numSMs * 4));
   if ((rc = nimfm_ensure_partials(ctx, (size_t)cgrid * 4))) return rc;
-  ffm_coef_kernel<<<cgrid, 256, 0, ctx->stream>>>(ctx->stash, X->y, rowBegin, nRows, loss, thr, mb, ctx->partials);
+  dloss_coef_kernel<<<cgrid, 256, 0, ctx->stream>>>(ctx->stash, X->y, rowBegin, nRows, loss, thr, mb, ctx->partials);
   LAUNCHED(ctx);
-  reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, cgrid, ctx->scalars + 8, 0);
+  reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, cgrid, o.red4, 0);
   LAUNCHED(ctx);
   // pass 2: the column kernel
   FfmColArgs c;
+  memset(&c, 0, sizeof(c));
   c.cdata = tw->csc->data; c.crow = tw->csc->indices;
   c.taskCol = tw->taskCol; c.taskLen = tw->taskLen; c.taskSlot = tw->taskSlot; c.taskBeg = tw->taskBeg;
   c.nTasks = tw->nTasks;
   c.data = X->data; c.indices = X->indices; c.fields = X->fields; c.indptr = X->indptr;
   c.coef = ctx->stash;
   c.rowBegin = rowBegin; c.rowEnd = rowBegin + nRows;
-  c.nFields = (int)m->nFields; c.CH = CH;
+  c.nFields = (int)m->nFields; c.CH = (int)std::max<int64_t>(X->maxSegNnz, 1);
   c.d = m->d;
   if (!m->PT) CK(cudaMalloc(&m->PT, (size_t)m->nP() * 8));
   ffm_field_major_kernel<<<ew_grid(ctx, m->nP()), 256, 0, ctx->stream>>>(m->P, m->PT, m->d, (int)m->nFields, m->k);
   LAUNCHED(ctx);
-  c.PT = m->PT; c.gP = m->grad; c.gw = m->grad + m->nP();
+  c.PT = m->PT; c.gP = o.gP; c.gw = o.gw; c.gnP = o.gnP; c.gnw = o.gnw;
   c.partial = ctx->stash + std::max<int64_t>(nRows, 1);
   c.fitLinear = m->fitLinear;
   c.k = m->k;
@@ -767,18 +777,65 @@ static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_datase
     CK(cudaFuncSetAttribute(ck, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ck, block, smem));
-    if (generic) occ = std::min(occ, FFM_COLS_GENERIC_BLOCKS_PER_SM);
+    if (!tunedKernel) occ = std::min(occ, FFM_COLS_GENERIC_BLOCKS_PER_SM);
     const int64_t wantBlocks = (tw->nTasks * taskMul + block / 32 - 1) / (block / 32);
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(wantBlocks, (int64_t)std::max(occ, 1) * ctx->numSMs));
     ck<<<grid, block, smem, ctx->stream>>>(c);
     LAUNCHED(ctx);
   }
   if (tw->nMulti > 0) {
-    ffm_cols_combine_kernel<<<(unsigned)tw->nMulti, 128, 0, ctx->stream>>>(tw->multiCol, tw->multiFirst, tw->multiCount,
-                                                                          tw->nMulti, c.partial, SB8, c.gP, c.gw, m->fitLinear);
+    if (ada)
+      ffm_cols_combine_ada_kernel<<<(unsigned)tw->nMulti, 128, 0, ctx->stream>>>(
+          tw->multiCol, tw->multiFirst, tw->multiCount, tw->nMulti, c.partial, SB8, c.gP, c.gw, c.gnP, c.gnw,
+          m->fitLinear);
+    else
+      ffm_cols_combine_kernel<<<(unsigned)tw->nMulti, 128, 0, ctx->stream>>>(tw->multiCol, tw->multiFirst,
+                                                                             tw->multiCount, tw->nMulti, c.partial, SB8,
+                                                                             c.gP, c.gw, m->fitLinear);
     LAUNCHED(ctx);
   }
   CK(cudaGetLastError());
+  return NIMFM_OK;
+}
+
+// the tuned column kernel's shape limits (ffm_cols.cuh), and whether it runs: NIMFM_FFM_COLS=generic puts the generic
+// kernel in its place
+static bool ffm_cols_tuned_shape(const nimfm_ffm *m, const nimfm_dataset *X) {
+  const int CH = (int)std::max<int64_t>(X->maxSegNnz, 1);
+  return (m->k == 4 || m->k == 8 || m->k == 16) && CH <= 64 && m->nFields <= 64 &&
+         m->d * m->nFields < (int64_t)2147483647;
+}
+static bool ffm_cols_want_generic() {
+  const char *envC = getenv("NIMFM_FFM_COLS");
+  return envC && !strcmp(envC, "generic");
+}
+
+static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int loss, double thr,
+                                int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb, bool must,
+                                int *taken) {
+  *taken = 0;
+  const bool contiguous = !rowIdxDev && rowBegin >= 0 && rowBegin + nRows <= X->n;
+  const bool tunedShape = ffm_cols_tuned_shape(m, X);
+  if (!contiguous || !(tunedShape || must)) {
+    if (must)
+      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
+                        "the deterministic FFM gradient needs a contiguous row range (no row list, no wrap-around)");
+    return NIMFM_OK;
+  }
+  bool dups = true;
+  int rc;
+  if ((rc = ffm_has_field_dups(ctx, X, &dups))) return rc;
+  if (dups) {
+    if (must)
+      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic FFM gradient needs rows with one nonzero per "
+                        "field (a row of this dataset repeats a field)");
+    return NIMFM_OK;
+  }
+  nimfm_det_twin *tw = nullptr;
+  if ((rc = nimfm_det_twin_get(ctx, X, 0, &tw))) return rc;
+  const FfmDetTargets o{m->grad, m->grad + m->nP(), nullptr, nullptr, ctx->scalars + 8, m->b};
+  if ((rc = ffm_det_pass(ctx, m, X, tw, loss, thr, rowBegin, nRows, mb, tunedShape && !ffm_cols_want_generic(), o)))
+    return rc;
   *taken = 1;
   return NIMFM_OK;
 }
@@ -944,6 +1001,20 @@ int32_t nimfm_ffm_adagrad_epoch(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_datase
   if ((rc = nimfm_mb_schedule(ctx, nRows, mb, *it, &sch))) return rc;
   PeerScope peers(ctx, {m->dG});
   if (peers.rc) return peers.rc;
+  // NIMFM_DETERMINISTIC=1 with miniBatchSize > 1: the gradient sums and their squares come from the column route
+  // (ffm_cols.cuh) over the minibatch's own column index (nimfm_mb_index_build), added in sample order without
+  // atomics.  A one-row minibatch of a row with one nonzero per field adds each element once: the RED route is
+  // already reproducible there and keeps it.
+  const char *envDet = getenv("NIMFM_DETERMINISTIC");
+  const bool det = envDet && envDet[0] == '1' && mb > 1;
+  TraceReport traceReport{ctx, "deterministic adagrad epoch", det};
+  if (det) {
+    bool dups = true;
+    if ((rc = ffm_has_field_dups(ctx, X, &dups))) return rc;
+    if (dups)
+      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic FFM AdaGrad needs rows with one nonzero per "
+                        "field (a row of this dataset repeats a field)");
+  }
   for (int64_t t = 0; t < sch.T; t++) {
     const int64_t start = std::min(t * mb, nRows);
     const int64_t cnt = sch.local(t);   // 0 once this rank's (shorter) shard is used up: it still joins the collectives
@@ -971,25 +1042,44 @@ int32_t nimfm_ffm_adagrad_epoch(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_datase
     }
     // one rank: accumulate straight into g_sum / g_norm (see nimfm_fm_adagrad_epoch)
     const bool direct = ctx->nranks == 1;
-    FfmPlan pl;
-    const bool aligned = ((reinterpret_cast<uintptr_t>(direct ? m->gsP : dGsP) | reinterpret_cast<uintptr_t>(direct ? m->gnP : dGnP)) & 15) == 0;
-    if ((rc = ffm_plan_mode(ctx, m, X, cnt, FFM_ADAGRAD, &pl, aligned))) return rc;
-    if ((rc = nimfm_ensure_partials(ctx, (size_t)pl.partialRows * 4))) return rc;
-    FfmArgs a;
-    ffm_fill_args(a, m, X);
-    a.rowBegin = start; a.nRows = cnt; a.rowIdx = rows;
-    a.gP = direct ? m->gsP : dGsP; a.gw = direct ? m->gsw : dGsw;
-    a.dGnP = direct ? m->gnP : dGnP; a.dGnw = direct ? m->gnw : dGnw;
-    a.partials = ctx->partials;
-    a.loss = cfg->loss; a.thr = cfg->huberThreshold;
-    a.gsP = m->gsP; a.gnP = m->gnP; a.gsw = m->gsw; a.gnw = m->gnw; a.adaScal = m->adaScal;
-    a.eta0 = cfg->eta0; a.tIt = tIt; a.alpha0 = cfg->alpha0; a.alpha = cfg->alpha; a.beta = cfg->beta;
-    a.first = first;
-    a.CH = pl.CH;
-    pl.kern<<<pl.grid, pl.block, pl.smem, ctx->stream>>>(a);
-    LAUNCHED(ctx);
-    reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, pl.partialRows, part, 0);
-    LAUNCHED(ctx);
+    if (det) {
+      nimfm_trace_begin(ctx, "det index");
+      nimfm_mb_index *ix = nullptr;
+      rc = nimfm_mb_index_build(ctx, X, 0, start, cnt, rows, &ix);
+      nimfm_trace_end(ctx);
+      if (rc) return rc;
+      nimfm_trace_begin(ctx, "det passes");
+      // the intercept every row of the minibatch sees (the AdaGrad kernels' prologue)
+      adagrad_bias_kernel<<<1, 1, 0, ctx->stream>>>(ix->bias, m->b, m->adaScal, m->fitIntercept, first, cfg->eta0, tIt,
+                                                    cfg->alpha0);
+      LAUNCHED(ctx);
+      const FfmDetTargets o{direct ? m->gsP : dGsP, direct ? m->gsw : dGsw, direct ? m->gnP : dGnP,
+                            direct ? m->gnw : dGnw, part, ix->bias};
+      rc = ffm_det_pass(ctx, m, &ix->view, &ix->tw, cfg->loss, cfg->huberThreshold, 0, cnt, 1.0,
+                        ffm_cols_tuned_shape(m, X) && !ffm_cols_want_generic(), o);
+      nimfm_trace_end(ctx);
+      if (rc) return rc;
+    } else {
+      FfmPlan pl;
+      const bool aligned = ((reinterpret_cast<uintptr_t>(direct ? m->gsP : dGsP) | reinterpret_cast<uintptr_t>(direct ? m->gnP : dGnP)) & 15) == 0;
+      if ((rc = ffm_plan_mode(ctx, m, X, cnt, FFM_ADAGRAD, &pl, aligned))) return rc;
+      if ((rc = nimfm_ensure_partials(ctx, (size_t)pl.partialRows * 4))) return rc;
+      FfmArgs a;
+      ffm_fill_args(a, m, X);
+      a.rowBegin = start; a.nRows = cnt; a.rowIdx = rows;
+      a.gP = direct ? m->gsP : dGsP; a.gw = direct ? m->gsw : dGsw;
+      a.dGnP = direct ? m->gnP : dGnP; a.dGnw = direct ? m->gnw : dGnw;
+      a.partials = ctx->partials;
+      a.loss = cfg->loss; a.thr = cfg->huberThreshold;
+      a.gsP = m->gsP; a.gnP = m->gnP; a.gsw = m->gsw; a.gnw = m->gnw; a.adaScal = m->adaScal;
+      a.eta0 = cfg->eta0; a.tIt = tIt; a.alpha0 = cfg->alpha0; a.alpha = cfg->alpha; a.beta = cfg->beta;
+      a.first = first;
+      a.CH = pl.CH;
+      pl.kern<<<pl.grid, pl.block, pl.smem, ctx->stream>>>(a);
+      LAUNCHED(ctx);
+      reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, pl.partialRows, part, 0);
+      LAUNCHED(ctx);
+    }
     if ((rc = nimfm_allreduce_sum(ctx, m->dG, nDelta))) return rc;
     adagrad_scalar_kernel<<<1, 1, 0, ctx->stream>>>(m->b, m->adaScal, part, violPart, ctx->scalars, m->fitIntercept,
                                                     cfg->eta0, tIt, cfg->alpha0, first);

@@ -26,7 +26,7 @@ struct FfmColArgs {
   const double *data;        // the CSR itself
   const int32_t *indices, *fields;
   const int64_t *indptr;
-  const double *coef;        // [rowEnd - rowBegin] coef_i = dloss_i / mb (written by ffm_coef_kernel)
+  const double *coef;        // [rowEnd - rowBegin] coef_i = dloss_i / mb (written by dloss_coef_kernel)
   int64_t rowBegin, rowEnd;
   int nFields, CH;
   int64_t d;
@@ -34,6 +34,7 @@ struct FfmColArgs {
   double *gP, *gw, *partial;
   int fitLinear;
   int k;                     // ffm_cols_grad_generic_kernel only: nComponents (fills the struct's tail padding)
+  double *gnP, *gnw;         // AdaGrad forms: where the squared gradients go (g_norm or its delta block)
 };
 
 static __device__ __forceinline__ int64_t lower_bound_row_i32(const int32_t *rows, int64_t lo, int64_t hi, int64_t r) {
@@ -61,29 +62,22 @@ static __global__ void ffm_cols_combine_kernel(const int32_t *multiCol, const in
   }
 }
 
-// coef_i = dloss(y_i, yhat_i) / mb in place of yhat (the forward kernel's output), loss / sum coef / sum dL^2 partials
-static __global__ void ffm_coef_kernel(double *yhatCoef, const double *y, int64_t rowBegin, int64_t nRows, int loss,
-                                       double thr, double mb, double *partials) {
-  __shared__ double red[8];
-  double l = 0.0, c = 0.0, d2 = 0.0;
-  for (int64_t q = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; q < nRows; q += (int64_t)gridDim.x * blockDim.x) {
-    const double yi = y[rowBegin + q], yh = yhatCoef[q];
-    const double dL = dev_dloss(loss, thr, yi, yh);
-    l += dev_loss(loss, thr, yi, yh);
-    c += dL / mb;
-    d2 += dL * dL;
-    yhatCoef[q] = dL / mb;
-  }
-  l = block_sum(l, red);
-  __syncthreads();
-  c = block_sum(c, red);
-  __syncthreads();
-  d2 = block_sum(d2, red);
-  if (threadIdx.x == 0) {
-    partials[blockIdx.x * 4 + 0] = l;
-    partials[blockIdx.x * 4 + 1] = c;
-    partials[blockIdx.x * 4 + 2] = d2;
-    partials[blockIdx.x * 4 + 3] = 0.0;
+// the AdaGrad form: a slot holds the sums, then the sums of squares, [SB8 | w | SB8 | w]; the second half goes to gnP / gnw
+static __global__ void ffm_cols_combine_ada_kernel(const int32_t *multiCol, const int32_t *multiFirst, const int32_t *multiCount,
+                                                   int64_t nMulti, const double *partial, int SB8, double *gP, double *gw,
+                                                   double *gnP, double *gnw, int fitLinear) {
+  const int64_t c = blockIdx.x;
+  if (c >= nMulti) return;
+  const int64_t j = multiCol[c];
+  const int S = 2 * (SB8 + 1);
+  for (int e = threadIdx.x; e < S; e += blockDim.x) {
+    double s = 0.0;
+    const double *ps = partial + (size_t)multiFirst[c] * S + e;
+    for (int q = 0; q < multiCount[c]; ++q) s += ps[(size_t)q * S];
+    const int h = e <= SB8 ? e : e - (SB8 + 1);
+    double *dP = e <= SB8 ? gP : gnP, *dW = e <= SB8 ? gw : gnw;
+    if (h < SB8) dP[j * SB8 + h] += s;
+    else if (fitLinear) dW[j] += s;
   }
 }
 
@@ -115,7 +109,10 @@ static inline size_t ffm_cols_warp_smem(int E) {
 // loads in flight per lane -- and accumulates.  No block-wide barrier anywhere: warps run independent segments.
 // (The first form -- a block per segment, thread <-> (field, component), three __syncthreads per batch -- ran the
 // C5 shape at 21 M rows/s against 60 M for the forward kernel gathering the same bytes: barrier- and latency-bound.)
-template <int KT, int E>
+// ADA (AdaGrad, adagrad.nim:113-124): every product g = sc * v is rounded on its own and g * g is summed into gnP, and
+// cx * cx into gnw.  With one nonzero per field, g is the sample's whole gradient element, so its square is the
+// reference's.
+template <int KT, int E, bool ADA = false>
 __global__ void __launch_bounds__(256) ffm_cols_grad_kernel(const FfmColArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int MAXZ = 64;
@@ -137,9 +134,9 @@ __global__ void __launch_bounds__(256) ffm_cols_grad_kernel(const FfmColArgs a) 
     int64_t eb = a.taskBeg[t], ee = eb + a.taskLen[t];
     if ((int64_t)a.crow[eb] < a.rowBegin) eb = lower_bound_row_i32(a.crow, eb, ee, a.rowBegin);
     if (eb < ee && (int64_t)a.crow[ee - 1] >= a.rowEnd) ee = lower_bound_row_i32(a.crow, eb, ee, a.rowEnd);
-    double acc0[KT], acc1[KT], accW = 0.0;
+    double acc0[KT], acc1[KT], accW = 0.0, accN0[KT], accN1[KT], accWN = 0.0;
 #pragma unroll
-    for (int c = 0; c < KT; ++c) acc0[c] = acc1[c] = 0.0;
+    for (int c = 0; c < KT; ++c) acc0[c] = acc1[c] = accN0[c] = accN1[c] = 0.0;
     for (int64_t e0 = eb; e0 < ee; e0 += E) {
       const int nb = (int)(ee - e0 < E ? ee - e0 : E);
       int64_t rbL = 0;
@@ -206,17 +203,32 @@ __global__ void __launch_bounds__(256) ffm_cols_grad_kernel(const FfmColArgs a) 
         for (int i = 0; i < E; ++i)   // entries in ascending row order
 #pragma unroll
           for (int c = 0; c < KT; ++c) {
-            if (pass == 0) acc0[c] += sc[i] * v[i][c];
-            else acc1[c] += sc[i] * v[i][c];
+            if (ADA) {
+              const double g = __dmul_rn(sc[i], v[i][c]);
+              if (pass == 0) {
+                acc0[c] += g;
+                accN0[c] += __dmul_rn(g, g);
+              } else {
+                acc1[c] += g;
+                accN1[c] += __dmul_rn(g, g);
+              }
+            } else {
+              if (pass == 0) acc0[c] += sc[i] * v[i][c];
+              else acc1[c] += sc[i] * v[i][c];
+            }
           }
       }
       if (lane == 0)
 #pragma unroll
         for (int i = 0; i < E; ++i)
-          if (i < nb) accW += cx[i];
+          if (i < nb) {
+            accW += cx[i];
+            if (ADA) accWN += __dmul_rn(cx[i], cx[i]);
+          }
     }
     const int slot = a.taskSlot[t];
-    double *dst = slot < 0 ? a.gP + (int64_t)jb * KT : a.partial + (size_t)slot * (SB8 + 1);
+    double *dst = slot < 0 ? a.gP + (int64_t)jb * KT : a.partial + (size_t)slot * (ADA ? 2 : 1) * (SB8 + 1);
+    double *dstN = ADA ? (slot < 0 ? a.gnP + (int64_t)jb * KT : dst + SB8 + 1) : nullptr;
 #pragma unroll
     for (int pass = 0; pass < 2; ++pass) {
       const int f = lane + 32 * pass;
@@ -226,12 +238,24 @@ __global__ void __launch_bounds__(256) ffm_cols_grad_kernel(const FfmColArgs a) 
           const double val = pass == 0 ? acc0[c] : acc1[c];
           if (slot < 0) dst[f * KT + c] += val;
           else dst[f * KT + c] = val;
+          if (ADA) {
+            const double valN = pass == 0 ? accN0[c] : accN1[c];
+            if (slot < 0) dstN[f * KT + c] += valN;
+            else dstN[f * KT + c] = valN;
+          }
         }
       }
     }
     if (lane == 0) {
-      if (slot < 0) { if (a.fitLinear) a.gw[j] += accW; }
-      else dst[SB8] = accW;
+      if (slot < 0) {
+        if (a.fitLinear) {
+          a.gw[j] += accW;
+          if (ADA) a.gnw[j] += accWN;
+        }
+      } else {
+        dst[SB8] = accW;
+        if (ADA) dstN[SB8] = accWN;
+      }
     }
   }
 }
@@ -244,8 +268,8 @@ __global__ void __launch_bounds__(256) ffm_cols_grad_kernel(const FfmColArgs a) 
 // row length.  The row is read once per (field block, chunk) where the tuned kernel reads it once.  Partner vectors
 // come from PT[f_j][j_u][s0 .. s0+KT): 16-byte loads when k is even, scalar loads when it is odd; components past k
 // are masked, never read.  Per entry the arithmetic is the tuned kernel's (cx = coef*x_j, sc = cx*x_u, acc += sc*v)
-// in the same ascending row order, so where both run they produce the same bits.
-template <int KT, int E>
+// in the same ascending row order, so where both run they produce the same bits.  ADA: as in ffm_cols_grad_kernel.
+template <int KT, int E, bool ADA = false>
 __global__ void __launch_bounds__(128) ffm_cols_grad_generic_kernel(const FfmColArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   struct WarpScratch {
@@ -270,9 +294,9 @@ __global__ void __launch_bounds__(128) ffm_cols_grad_generic_kernel(const FfmCol
     int64_t eb = a.taskBeg[t], ee = eb + a.taskLen[t];
     if ((int64_t)a.crow[eb] < a.rowBegin) eb = lower_bound_row_i32(a.crow, eb, ee, a.rowBegin);
     if (eb < ee && (int64_t)a.crow[ee - 1] >= a.rowEnd) ee = lower_bound_row_i32(a.crow, eb, ee, a.rowEnd);
-    double acc[KT], accW = 0.0;
+    double acc[KT], accW = 0.0, accN[KT], accWN = 0.0;
 #pragma unroll
-    for (int c = 0; c < KT; ++c) acc[c] = 0.0;
+    for (int c = 0; c < KT; ++c) acc[c] = accN[c] = 0.0;
     for (int64_t e0 = eb; e0 < ee; e0 += E) {
       const int nb = (int)(ee - e0 < E ? ee - e0 : E);
       int64_t rbL = 0;
@@ -344,25 +368,48 @@ __global__ void __launch_bounds__(128) ffm_cols_grad_generic_kernel(const FfmCol
 #pragma unroll
       for (int i = 0; i < E; ++i)   // entries in ascending row order
 #pragma unroll
-        for (int c = 0; c < KT; ++c) acc[c] += sc[i] * v[i][c];
+        for (int c = 0; c < KT; ++c) {
+          if (ADA) {
+            const double g = __dmul_rn(sc[i], v[i][c]);
+            acc[c] += g;
+            accN[c] += __dmul_rn(g, g);
+          } else {
+            acc[c] += sc[i] * v[i][c];
+          }
+        }
       if (lane == 0)
 #pragma unroll
         for (int i = 0; i < E; ++i)
-          if (i < nb) accW += cx[i];
+          if (i < nb) {
+            accW += cx[i];
+            if (ADA) accWN += __dmul_rn(cx[i], cx[i]);
+          }
     }
     const int slot = a.taskSlot[t];
-    double *dst = slot < 0 ? a.gP + j * SB8 : a.partial + (size_t)slot * (SB8 + 1);
+    double *dst = slot < 0 ? a.gP + j * SB8 : a.partial + (size_t)slot * (ADA ? 2 : 1) * (SB8 + 1);
+    double *dstN = ADA ? (slot < 0 ? a.gnP + j * SB8 : dst + SB8 + 1) : nullptr;
     if (f < nF) {
 #pragma unroll
       for (int c = 0; c < KT; ++c) {
         if (s0 + c >= k) break;
         if (slot < 0) dst[(int64_t)f * k + s0 + c] += acc[c];
         else dst[(int64_t)f * k + s0 + c] = acc[c];
+        if (ADA) {
+          if (slot < 0) dstN[(int64_t)f * k + s0 + c] += accN[c];
+          else dstN[(int64_t)f * k + s0 + c] = accN[c];
+        }
       }
     }
     if (lane == 0 && fb == 0 && s0 == 0) {   // one task per segment owns the linear term
-      if (slot < 0) { if (a.fitLinear) a.gw[j] += accW; }
-      else dst[SB8] = accW;
+      if (slot < 0) {
+        if (a.fitLinear) {
+          a.gw[j] += accW;
+          if (ADA) a.gnw[j] += accWN;
+        }
+      } else {
+        dst[SB8] = accW;
+        if (ADA) dstN[SB8] = accWN;
+      }
     }
   }
 }

@@ -74,6 +74,10 @@ RowKernel nimfm_row_kernel_stash(int degree, bool explicitLower);
 int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, bool streamStash,
                            int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
                            int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base);
+int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, RowKernel stashKern, bool streamStash,
+                      int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+                      int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base,
+                      const FmDetTargets &o);
 
 static bool is_explicit(const nimfm_fm *fm) { return fm->degree > 2 && fm->nOrders == fm->degree - 1; }
 
@@ -1036,6 +1040,13 @@ int32_t nimfm_fm_adagrad_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset
   if ((rc = nimfm_mb_schedule(ctx, nRows, mb, *it, &sch))) return rc;
   PeerScope peers(ctx, {fm->dG});
   if (peers.rc) return peers.rc;
+  // NIMFM_DETERMINISTIC=1 with miniBatchSize > 1: the gradient sums and their squares come from the column route
+  // (fm_cols.cu) over the minibatch's own column index (nimfm_mb_index_build), added in sample order without atomics.
+  // A one-row minibatch adds each element once (a CSR row holds a feature once): the RED route is already
+  // reproducible there and keeps it.
+  const char *envDet = getenv("NIMFM_DETERMINISTIC");
+  const bool det = envDet && envDet[0] == '1' && mb > 1;
+  TraceReport traceReport{ctx, "deterministic adagrad epoch", det};
   for (int64_t t = 0; t < sch.T; t++) {
     const int64_t start = std::min(t * mb, nRows);
     const int64_t cnt = sch.local(t);   // 0 once this rank's (shorter) shard is used up: it still joins the collectives
@@ -1062,34 +1073,63 @@ int32_t nimfm_fm_adagrad_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset
       reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, rgrid, violPart, 0);
       LAUNCHED(ctx);
     }
-    RowPlan pl;
-    if ((rc = plan_rows(ctx, fm, X, cnt, MODE_ADAGRAD, &pl))) return rc;
-    RowKernel kern = pl.kern;
-    if ((rc = nimfm_ensure_partials(ctx, (size_t)pl.nWarps * 4))) return rc;
-    RowArgs a;
-    fill_row_args(a, fm, X);
-    a.rowBegin = start;
-    a.nRows = cnt;
-    a.rowIdx = rows;
     // one rank: the gradients and their squares go straight into g_sum / g_norm (nothing reads them before
     // the next minibatch's refresh), so the delta block and the apply pass are only needed for the all-reduce
     const bool direct = ctx->nranks == 1;
-    a.gP = direct ? fm->gsP : dGsP;
-    a.gw = direct ? fm->gsw : dGsw;
-    a.dGnP = direct ? fm->gnP : dGnP;
-    a.dGnw = direct ? fm->gnw : dGnw;
-    a.partials = ctx->partials;
-    a.loss = cfg->loss;
-    a.thr = cfg->huberThreshold;
-    a.gsP = fm->gsP; a.gnP = fm->gnP; a.gsw = fm->gsw; a.gnw = fm->gnw; a.adaScal = fm->adaScal;
-    a.eta0 = cfg->eta0; a.tIt = tIt; a.alpha0 = cfg->alpha0; a.alpha = cfg->alpha; a.beta = cfg->beta;
-    a.first = first;
-    a.G = pl.G;
-    a.CH = pl.CH;
-    kern<<<pl.grid, pl.block, pl.smem, ctx->stream>>>(a);
-    LAUNCHED(ctx);
-    reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, pl.nWarps, part, 0);
-    LAUNCHED(ctx);
+    if (det) {
+      nimfm_trace_begin(ctx, "det index");
+      nimfm_mb_index *ix = nullptr;
+      rc = nimfm_mb_index_build(ctx, X, fm->nAug, start, cnt, rows, &ix);
+      nimfm_trace_end(ctx);
+      if (rc) return rc;
+      nimfm_trace_begin(ctx, "det passes");
+      // the intercept every row of the minibatch sees (the row kernels' AdaGrad prologue, fm_rows.cuh)
+      adagrad_bias_kernel<<<1, 1, 0, ctx->stream>>>(ix->bias, fm->b, fm->adaScal, fm->fitIntercept, first, cfg->eta0,
+                                                    tIt, cfg->alpha0);
+      LAUNCHED(ctx);
+      RowPlan pl;
+      if ((rc = plan_rows(ctx, fm, &ix->view, cnt, MODE_STASH, &pl))) return rc;
+      RowArgs base;
+      fill_row_args(base, fm, &ix->view);
+      base.b = ix->bias;
+      FmDetTargets o;
+      o.gP = direct ? fm->gsP : dGsP;
+      o.gw = direct ? fm->gsw : dGsw;
+      o.gnP = direct ? fm->gnP : dGnP;
+      o.gnw = direct ? fm->gnw : dGnw;
+      o.red4 = part;
+      o.yhat = ix->yhat;
+      rc = nimfm_fm_det_pass(ctx, fm, &ix->tw, pl.kern, pl.stream, pl.G, pl.CH, pl.grid, pl.block, pl.smem, pl.nWarps,
+                             cfg->loss, cfg->huberThreshold, 0, cnt, 1.0, nullptr, base, o);
+      nimfm_trace_end(ctx);
+      if (rc) return rc;
+    } else {
+      RowPlan pl;
+      if ((rc = plan_rows(ctx, fm, X, cnt, MODE_ADAGRAD, &pl))) return rc;
+      RowKernel kern = pl.kern;
+      if ((rc = nimfm_ensure_partials(ctx, (size_t)pl.nWarps * 4))) return rc;
+      RowArgs a;
+      fill_row_args(a, fm, X);
+      a.rowBegin = start;
+      a.nRows = cnt;
+      a.rowIdx = rows;
+      a.gP = direct ? fm->gsP : dGsP;
+      a.gw = direct ? fm->gsw : dGsw;
+      a.dGnP = direct ? fm->gnP : dGnP;
+      a.dGnw = direct ? fm->gnw : dGnw;
+      a.partials = ctx->partials;
+      a.loss = cfg->loss;
+      a.thr = cfg->huberThreshold;
+      a.gsP = fm->gsP; a.gnP = fm->gnP; a.gsw = fm->gsw; a.gnw = fm->gnw; a.adaScal = fm->adaScal;
+      a.eta0 = cfg->eta0; a.tIt = tIt; a.alpha0 = cfg->alpha0; a.alpha = cfg->alpha; a.beta = cfg->beta;
+      a.first = first;
+      a.G = pl.G;
+      a.CH = pl.CH;
+      kern<<<pl.grid, pl.block, pl.smem, ctx->stream>>>(a);
+      LAUNCHED(ctx);
+      reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, pl.nWarps, part, 0);
+      LAUNCHED(ctx);
+    }
     // synchronous data parallelism: all-reduce the deltas [dGs | dGn | dGsw | dGnw | loss, dL, dL^2, -]
     if ((rc = nimfm_allreduce_sum(ctx, fm->dG, nDelta))) return rc;
     adagrad_scalar_kernel<<<1, 1, 0, ctx->stream>>>(fm->b, fm->adaScal, part, violPart, ctx->scalars, fm->fitIntercept,

@@ -48,9 +48,10 @@ struct ColArgs {
   const double *stash;
   int stashStride;
   double *gP, *gw;
-  double *partial;          // [nSlots][SB8 + 1]
+  double *partial;          // [nSlots][SB8 + 1]; AdaGrad forms: [nSlots][2 (SB8 + 1)], sums then squares
   int fitLinear;
   int k, KT;                // fm_cols_grad_generic_kernel only: nComponents and the lane-group width
+  double *gnP, *gnw;        // AdaGrad forms: where the squared gradients go (g_norm or its delta block)
 };
 
 // first position in [lo, hi) whose row id is >= r
@@ -63,8 +64,12 @@ __device__ __forceinline__ int64_t lower_bound_row(const int32_t *rows, int64_t 
   return lo;
 }
 
-template <int DEGREE, bool EXPLICIT, int KT>
-__global__ void __launch_bounds__(256) fm_cols_grad_kernel(const ColArgs a) {
+// ADA (AdaGrad, adagrad.nim:113-124): every entry's gradient g = coef * dA is rounded on its own, as the RED route adds
+// it, and the kernel also sums g * g into gnP / gnw.  A CSR row holds a feature once, so an entry is the sample's whole
+// gradient element and its square is the reference's.  The ADA instances ask for two resident blocks per SM: left to
+// its default, ptxas holds <3, false, KT, true> to 64 registers and spills; the gradient instances keep no minimum.
+template <int DEGREE, bool EXPLICIT, int KT, bool ADA = false>
+__global__ void __launch_bounds__(256, ADA ? 2 : 0) fm_cols_grad_kernel(const ColArgs a) {
   constexpr int NO = RowCfg<DEGREE, EXPLICIT>::NO;
   constexpr int G = KT, GPW = 32 / G, SB8 = NO * KT, U = 4;
   const int lane = threadIdx.x & 31, gl = lane & (G - 1), gid = lane / G;
@@ -83,11 +88,12 @@ __global__ void __launch_bounds__(256) fm_cols_grad_kernel(const ColArgs a) {
       eb = eb < a.rowBegin ? a.rowBegin : eb;
       ee = ee > a.rowEnd ? a.rowEnd : ee;
     }
-    double p[NO], acc[NO], accW = 0.0;
+    double p[NO], acc[NO], accW = 0.0, accN[NO], accWN = 0.0;
 #pragma unroll
     for (int o = 0; o < NO; ++o) {
       p[o] = a.P[j * SB8 + o * KT + gl];
       acc[o] = 0.0;
+      accN[o] = 0.0;
     }
     // software pipeline: the row ids / values of batch b+1 are fetched while batch b's stash records are in flight,
     // so a batch costs ONE dependent memory latency (stash gather) instead of two (ncu on the unpipelined form:
@@ -142,21 +148,45 @@ __global__ void __launch_bounds__(256) fm_cols_grad_kernel(const ColArgs a) {
             for (int tt = 1; tt < DEGREE; ++tt)
               if (tt < M) g = x[u] * (av[u][o][tt] - p[o] * g);
           }
-          acc[o] += coef[u] * g;
+          if (ADA) {
+            const double gr = __dmul_rn(coef[u], g);
+            acc[o] += gr;
+            accN[o] += __dmul_rn(gr, gr);
+          } else {
+            acc[o] += coef[u] * g;
+          }
         }
-        accW += coef[u] * x[u];
+        if (ADA) {
+          const double gx = __dmul_rn(coef[u], x[u]);
+          accW += gx;
+          accWN += __dmul_rn(gx, gx);
+        } else {
+          accW += coef[u] * x[u];
+        }
       }
     }
     const int slot = a.taskSlot[t];
     if (slot < 0) {
 #pragma unroll
-      for (int o = 0; o < NO; ++o) a.gP[j * SB8 + o * KT + gl] += acc[o];
-      if (gl == 0 && !dummy && a.fitLinear) a.gw[j] += accW;
+      for (int o = 0; o < NO; ++o) {
+        a.gP[j * SB8 + o * KT + gl] += acc[o];
+        if (ADA) a.gnP[j * SB8 + o * KT + gl] += accN[o];
+      }
+      if (gl == 0 && !dummy && a.fitLinear) {
+        a.gw[j] += accW;
+        if (ADA) a.gnw[j] += accWN;
+      }
     } else {
-      double *ps = a.partial + (size_t)slot * (SB8 + 1);
+      double *ps = a.partial + (size_t)slot * (ADA ? 2 : 1) * (SB8 + 1);
 #pragma unroll
-      for (int o = 0; o < NO; ++o) ps[o * KT + gl] = acc[o];
-      if (gl == 0) ps[SB8] = accW;
+      for (int o = 0; o < NO; ++o) {
+        ps[o * KT + gl] = acc[o];
+        if (ADA) ps[SB8 + 1 + o * KT + gl] = accN[o];
+      }
+      if (gl == 0) {
+        ps[SB8] = accW;
+        if (ADA) ps[2 * SB8 + 1] = accWN;
+      }
     }
   }
 }
@@ -164,9 +194,10 @@ __global__ void __launch_bounds__(256) fm_cols_grad_kernel(const ColArgs a) {
 // fm_cols_grad_kernel with nComponents at run time (every degree, every k): a group of KT lanes (KT in {4,8,16,32},
 // lane_group_kt) maps lane <-> component s = sc*KT + lane of component chunk sc, and a task walks its entries once per
 // chunk; lanes past k idle.  Per entry the arithmetic is fm_cols_grad_kernel's expression sequence in the same
-// ascending row order, so where both kernels run they produce the same bits.
-template <int DEGREE, bool EXPLICIT>
-__global__ void __launch_bounds__(256, 2) fm_cols_grad_generic_kernel(const ColArgs a) {
+// ascending row order, so where both kernels run they produce the same bits.  ADA: as in fm_cols_grad_kernel; those
+// instances are held to one 256-thread block per SM by their launch bounds, for room for the square accumulators.
+template <int DEGREE, bool EXPLICIT, bool ADA = false>
+__global__ void __launch_bounds__(256, ADA ? 1 : 2) fm_cols_grad_generic_kernel(const ColArgs a) {
   constexpr int NO = RowCfg<DEGREE, EXPLICIT>::NO;
   constexpr int NV = NO * (2 * DEGREE - NO - 1) / 2;   // stash values per component: sum over o of M_o - 1
   constexpr int U = NV <= 6 ? 4 : 2;                   // entries per batch (register budget of av below)
@@ -190,11 +221,12 @@ __global__ void __launch_bounds__(256, 2) fm_cols_grad_generic_kernel(const ColA
     for (int sc = 0; sc < NC; ++sc) {
       const int s = sc * KT + gl;
       if (s >= k) break;
-      double p[NO], acc[NO], accW = 0.0;
+      double p[NO], acc[NO], accW = 0.0, accN[NO], accWN = 0.0;
 #pragma unroll
       for (int o = 0; o < NO; ++o) {
         p[o] = a.P[j * SB8 + o * k + s];
         acc[o] = 0.0;
+        accN[o] = 0.0;
       }
       // the same software pipeline as fm_cols_grad_kernel: batch b+1's row ids / values load under batch b's records
       int64_t rowN[U];
@@ -247,20 +279,44 @@ __global__ void __launch_bounds__(256, 2) fm_cols_grad_generic_kernel(const ColA
               for (int tt = 1; tt < DEGREE; ++tt)
                 if (tt < M) g = x[u] * (av[u][o][tt] - p[o] * g);
             }
-            acc[o] += coef[u] * g;
+            if (ADA) {
+              const double gr = __dmul_rn(coef[u], g);
+              acc[o] += gr;
+              accN[o] += __dmul_rn(gr, gr);
+            } else {
+              acc[o] += coef[u] * g;
+            }
           }
-          accW += coef[u] * x[u];
+          if (ADA) {
+            const double gx = __dmul_rn(coef[u], x[u]);
+            accW += gx;
+            accWN += __dmul_rn(gx, gx);
+          } else {
+            accW += coef[u] * x[u];
+          }
         }
       }
       if (slot < 0) {
 #pragma unroll
-        for (int o = 0; o < NO; ++o) a.gP[j * SB8 + o * k + s] += acc[o];
-        if (s == 0 && !dummy && a.fitLinear) a.gw[j] += accW;
+        for (int o = 0; o < NO; ++o) {
+          a.gP[j * SB8 + o * k + s] += acc[o];
+          if (ADA) a.gnP[j * SB8 + o * k + s] += accN[o];
+        }
+        if (s == 0 && !dummy && a.fitLinear) {
+          a.gw[j] += accW;
+          if (ADA) a.gnw[j] += accWN;
+        }
       } else {
-        double *ps = a.partial + (size_t)slot * (SB8 + 1);
+        double *ps = a.partial + (size_t)slot * (ADA ? 2 : 1) * (SB8 + 1);
 #pragma unroll
-        for (int o = 0; o < NO; ++o) ps[o * k + s] = acc[o];
-        if (s == 0) ps[SB8] = accW;
+        for (int o = 0; o < NO; ++o) {
+          ps[o * k + s] = acc[o];
+          if (ADA) ps[SB8 + 1 + o * k + s] = accN[o];
+        }
+        if (s == 0) {
+          ps[SB8] = accW;
+          if (ADA) ps[2 * SB8 + 1] = accWN;
+        }
       }
     }
   }
@@ -282,6 +338,25 @@ __global__ void fm_cols_combine_kernel(const int32_t *multiCol, const int32_t *m
   }
 }
 
+// the AdaGrad form: a slot holds the sums, then the sums of squares, [SB8 | w | SB8 | w]; the second half goes to gnP / gnw
+__global__ void fm_cols_combine_ada_kernel(const int32_t *multiCol, const int32_t *multiFirst, const int32_t *multiCount,
+                                           int64_t nMulti, const double *partial, int SB8, int64_t d, double *gP, double *gw,
+                                           double *gnP, double *gnw, int fitLinear) {
+  const int64_t c = blockIdx.x;
+  if (c >= nMulti) return;
+  const int64_t j = multiCol[c];
+  const int S = 2 * (SB8 + 1);
+  for (int e = threadIdx.x; e < S; e += blockDim.x) {
+    double s = 0.0;
+    const double *ps = partial + (size_t)multiFirst[c] * S + e;
+    for (int q = 0; q < multiCount[c]; ++q) s += ps[(size_t)q * S];
+    const int h = e <= SB8 ? e : e - (SB8 + 1);
+    double *dP = e <= SB8 ? gP : gnP, *dW = e <= SB8 ? gw : gnw;
+    if (h < SB8) dP[j * SB8 + h] += s;
+    else if (j < d && fitLinear) dW[j] += s;
+  }
+}
+
 template <int DEGREE, bool EXPLICIT>
 RowKernel pick_stash(int k) {
   switch (k) {
@@ -293,23 +368,24 @@ RowKernel pick_stash(int k) {
 }
 
 typedef void (*ColKernel)(const ColArgs);
-template <int DEGREE, bool EXPLICIT>
+template <int DEGREE, bool EXPLICIT, bool ADA>
 ColKernel pick_cols(int k) {
   switch (k) {
-    case 8: return fm_cols_grad_kernel<DEGREE, EXPLICIT, 8>;
-    case 16: return fm_cols_grad_kernel<DEGREE, EXPLICIT, 16>;
-    case 32: return fm_cols_grad_kernel<DEGREE, EXPLICIT, 32>;
+    case 8: return fm_cols_grad_kernel<DEGREE, EXPLICIT, 8, ADA>;
+    case 16: return fm_cols_grad_kernel<DEGREE, EXPLICIT, 16, ADA>;
+    case 32: return fm_cols_grad_kernel<DEGREE, EXPLICIT, 32, ADA>;
     default: return nullptr;
   }
 }
 
+template <bool ADA>
 ColKernel pick_cols_generic(int degree, bool explicitLower) {
   switch (degree) {
-    case 2: return fm_cols_grad_generic_kernel<2, false>;
-    case 3: return explicitLower ? fm_cols_grad_generic_kernel<3, true> : fm_cols_grad_generic_kernel<3, false>;
-    case 4: return explicitLower ? fm_cols_grad_generic_kernel<4, true> : fm_cols_grad_generic_kernel<4, false>;
-    case 5: return explicitLower ? fm_cols_grad_generic_kernel<5, true> : fm_cols_grad_generic_kernel<5, false>;
-    case 6: return explicitLower ? fm_cols_grad_generic_kernel<6, true> : fm_cols_grad_generic_kernel<6, false>;
+    case 2: return fm_cols_grad_generic_kernel<2, false, ADA>;
+    case 3: return explicitLower ? fm_cols_grad_generic_kernel<3, true, ADA> : fm_cols_grad_generic_kernel<3, false, ADA>;
+    case 4: return explicitLower ? fm_cols_grad_generic_kernel<4, true, ADA> : fm_cols_grad_generic_kernel<4, false, ADA>;
+    case 5: return explicitLower ? fm_cols_grad_generic_kernel<5, true, ADA> : fm_cols_grad_generic_kernel<5, false, ADA>;
+    case 6: return explicitLower ? fm_cols_grad_generic_kernel<6, true, ADA> : fm_cols_grad_generic_kernel<6, false, ADA>;
     default: return nullptr;
   }
 }
@@ -413,36 +489,40 @@ int nimfm_det_twin_get(nimfm_ctx *ctx, const nimfm_dataset *X, int nAug, nimfm_d
   return NIMFM_OK;
 }
 
-// Deterministic predict+grad over rows [rowBegin, rowBegin + nRows) of X into the model's gradient buffers
-// (accumulating, like the RED route).  red4 (loss, sum coef, sum dL^2, -) is left at ctx->scalars + 8.
-// streamStash: stashKern is the streaming instance; the tuned column kernel then reads its stash, and every other
-// shape (or NIMFM_ROW_KERNEL=generic, which plans the generic stash forward) takes the runtime-k column kernel.
-int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, bool streamStash,
-                           int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
-                           int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base) {
-  if (rowBegin < 0 || rowBegin + nRows > X->n)
-    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic gradient needs a contiguous row range without wrap-around");
+// The two passes of the deterministic route over rows [rowBegin, rowBegin + nRows) of X, with the column twin `tw` of
+// X (its row ids are X's) and the given targets: the stash forward leaves red4 (loss, sum coef, sum dL^2, -) at
+// o.red4, the column kernel and the combine add the gradient into o.gP / o.gw and, when o.gnP is set (AdaGrad, coef =
+// dL), its squares into o.gnP / o.gnw.  streamStash: stashKern is the streaming instance; the tuned column kernel then
+// reads its stash, and every other shape (or NIMFM_ROW_KERNEL=generic, which plans the generic stash forward) takes
+// the runtime-k column kernel.  base: the row arguments of X and the model (RowArgs.b may point at a refreshed
+// intercept).
+int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, RowKernel stashKern, bool streamStash,
+                      int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+                      int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base,
+                      const FmDetTargets &o) {
   const bool expl = fm->degree > 2 && fm->nOrders == fm->degree - 1;
+  const bool ada = o.gnP != nullptr;
   ColKernel ck = nullptr;
   int colKT = fm->k;
   if (streamStash)
-    ck = fm->degree == 2 ? pick_cols<2, false>(fm->k)
-         : fm->degree == 3 ? (expl ? pick_cols<3, true>(fm->k) : pick_cols<3, false>(fm->k)) : nullptr;
+    ck = ada ? (fm->degree == 2 ? pick_cols<2, false, true>(fm->k)
+                : fm->degree == 3 ? (expl ? pick_cols<3, true, true>(fm->k) : pick_cols<3, false, true>(fm->k)) : nullptr)
+             : (fm->degree == 2 ? pick_cols<2, false, false>(fm->k)
+                : fm->degree == 3 ? (expl ? pick_cols<3, true, false>(fm->k) : pick_cols<3, false, false>(fm->k)) : nullptr);
   if (!ck) {
-    ck = pick_cols_generic(fm->degree, expl);
+    ck = ada ? pick_cols_generic<true>(fm->degree, expl) : pick_cols_generic<false>(fm->degree, expl);
     colKT = lane_group_kt(fm->k);
   }
   if (!ck || !stashKern)
     return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "no deterministic gradient kernel for degree %d", fm->degree);
   int rc;
-  nimfm_det_twin *tw = nullptr;
-  if ((rc = nimfm_det_twin_get(ctx, X, fm->nAug, &tw))) return rc;
   // stash record: coef + (M_o - 1) values per component and order, padded to an even number of doubles
   int vals = 0;
-  for (int o = 0; o < fm->nOrders; o++) vals += (fm->degree - o) - 1;
+  for (int q = 0; q < fm->nOrders; q++) vals += (fm->degree - q) - 1;
   int stride = 1 + vals * fm->k;
   stride += stride & 1;
-  const size_t need = (size_t)std::max<int64_t>(nRows, 1) * stride + (size_t)tw->nSlots * (fm->nOrders * fm->k + 1) + 16;
+  const size_t slotLen = (size_t)(ada ? 2 : 1) * (fm->nOrders * fm->k + 1);
+  const size_t need = (size_t)std::max<int64_t>(nRows, 1) * stride + (size_t)tw->nSlots * slotLen + 16;
   if (ctx->stashCap < need) {
     CK(cudaStreamSynchronize(ctx->stream));
     if (ctx->stash) CK(cudaFree(ctx->stash));
@@ -472,11 +552,21 @@ int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X,
   a.CH = CH;
   a.stash = ctx->stash;
   a.stashStride = stride;
+  if (o.yhat) a.yOut = o.yhat;
   stashKern<<<grid, block, smem, ctx->stream>>>(a);
   LAUNCHED(ctx);
-  reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, nWarps, ctx->scalars + 8, 0);
+  if (o.yhat) {
+    const int cgrid = (int)std::max<int64_t>(1, std::min<int64_t>((nRows + 255) / 256, (int64_t)ctx->numSMs * 4));
+    if ((rc = nimfm_ensure_partials(ctx, (size_t)cgrid * 4))) return rc;
+    dloss_coef_kernel<<<cgrid, 256, 0, ctx->stream>>>(o.yhat, a.y, rowBegin, nRows, loss, thr, mb, ctx->partials);
+    LAUNCHED(ctx);
+    reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, cgrid, o.red4, 0);
+  } else {
+    reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, nWarps, o.red4, 0);
+  }
   LAUNCHED(ctx);
   ColArgs c;
+  memset(&c, 0, sizeof(c));
   c.cdata = tw->csc->data;
   c.crow = tw->csc->indices;
   c.taskCol = tw->taskCol;
@@ -490,8 +580,10 @@ int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X,
   c.P = fm->P;
   c.stash = ctx->stash;
   c.stashStride = stride;
-  c.gP = fm->grad;
-  c.gw = fm->grad + fm->nP();
+  c.gP = o.gP;
+  c.gw = o.gw;
+  c.gnP = o.gnP;
+  c.gnw = o.gnw;
   c.partial = ctx->stash + (size_t)std::max<int64_t>(nRows, 1) * stride;
   c.fitLinear = fm->fitLinear;
   c.k = fm->k;
@@ -504,11 +596,36 @@ int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X,
     LAUNCHED(ctx);
   }
   if (tw->nMulti > 0) {
-    fm_cols_combine_kernel<<<(unsigned)tw->nMulti, 64, 0, ctx->stream>>>(tw->multiCol, tw->multiFirst, tw->multiCount,
-                                                                         tw->nMulti, c.partial, fm->nOrders * fm->k, fm->d,
-                                                                         c.gP, c.gw, fm->fitLinear);
+    const int SB8 = fm->nOrders * fm->k;
+    if (ada)
+      fm_cols_combine_ada_kernel<<<(unsigned)tw->nMulti, 64, 0, ctx->stream>>>(
+          tw->multiCol, tw->multiFirst, tw->multiCount, tw->nMulti, c.partial, SB8, fm->d, c.gP, c.gw, c.gnP, c.gnw,
+          fm->fitLinear);
+    else
+      fm_cols_combine_kernel<<<(unsigned)tw->nMulti, 64, 0, ctx->stream>>>(tw->multiCol, tw->multiFirst, tw->multiCount,
+                                                                           tw->nMulti, c.partial, SB8, fm->d, c.gP,
+                                                                           c.gw, fm->fitLinear);
     LAUNCHED(ctx);
   }
   CK(cudaGetLastError());
   return NIMFM_OK;
+}
+
+// Deterministic predict+grad over rows [rowBegin, rowBegin + nRows) of X into the model's gradient buffers
+// (accumulating, like the RED route), with the dataset's column twin.  red4 (loss, sum coef, sum dL^2, -) is left at
+// ctx->scalars + 8.
+int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, bool streamStash,
+                           int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+                           int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base) {
+  if (rowBegin < 0 || rowBegin + nRows > X->n)
+    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic gradient needs a contiguous row range without wrap-around");
+  int rc;
+  nimfm_det_twin *tw = nullptr;
+  if ((rc = nimfm_det_twin_get(ctx, X, fm->nAug, &tw))) return rc;
+  FmDetTargets o;
+  o.gP = fm->grad;
+  o.gw = fm->grad + fm->nP();
+  o.red4 = ctx->scalars + 8;
+  return nimfm_fm_det_pass(ctx, fm, tw, stashKern, streamStash, G, CH, grid, block, smem, nWarps, loss, thr, rowBegin,
+                           nRows, mb, yOutDev, base, o);
 }

@@ -71,6 +71,15 @@ struct RowArgs {
   int G, CH;
 };
 
+// where the deterministic route's outputs go (nimfm_fm_det_pass)
+struct FmDetTargets {
+  double *gP = nullptr, *gw = nullptr;     // gradient sums (the model's gradient, g_sum or its delta block)
+  double *gnP = nullptr, *gnw = nullptr;   // AdaGrad: sums of squared gradients; nullptr: plain gradient
+  double *red4 = nullptr;                  // (loss, sum coef, sum dL^2, -)
+  double *yhat = nullptr;   // [nRows] scratch: when set, red4 is summed from the rows' yhat by dloss_coef_kernel, in an
+                            // order that does not depend on which forward kernel ran (AdaGrad: red4 moves the intercept)
+};
+
 #define NIMFM_COLD 255
 #define NIMFM_MAX_HOT 16
 
