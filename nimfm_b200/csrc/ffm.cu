@@ -53,7 +53,6 @@ struct __align__(16) FfmMeta {
 };
 
 #include "ffm_pairs.cuh"
-#include "ffm_tma.cuh"
 #include "ffm_cols.cuh"
 #include "ffm_units.cuh"
 
@@ -228,18 +227,18 @@ struct FfmPlan {
 };
 
 // pair-streaming kernel when k is 4/8/16/32, else nullptr
-template <int KT, bool TABLE>
+template <int KT>
 static FfmKernel ffm_pairs_mode(int mode) {
-  return mode == FFM_PREDICT ? ffm_pairs_kernel<FFM_PAIRS_PREDICT, KT, TABLE, FfmArgs>
-         : mode == FFM_GRAD  ? ffm_pairs_kernel<FFM_PAIRS_GRAD, KT, TABLE, FfmArgs>
-                             : ffm_pairs_kernel<FFM_PAIRS_ADAGRAD, KT, TABLE, FfmArgs>;
+  return mode == FFM_PREDICT ? ffm_pairs_kernel<FFM_PAIRS_PREDICT, KT, FfmArgs>
+         : mode == FFM_GRAD  ? ffm_pairs_kernel<FFM_PAIRS_GRAD, KT, FfmArgs>
+                             : ffm_pairs_kernel<FFM_PAIRS_ADAGRAD, KT, FfmArgs>;
 }
-static FfmKernel ffm_pairs_pick(int k, int mode, bool table) {
+static FfmKernel ffm_pairs_pick(int k, int mode) {
   switch (k) {
-    case 4: return table ? ffm_pairs_mode<4, true>(mode) : ffm_pairs_mode<4, false>(mode);
-    case 8: return table ? ffm_pairs_mode<8, true>(mode) : ffm_pairs_mode<8, false>(mode);
-    case 16: return table ? ffm_pairs_mode<16, true>(mode) : ffm_pairs_mode<16, false>(mode);
-    case 32: return table ? ffm_pairs_mode<32, true>(mode) : ffm_pairs_mode<32, false>(mode);
+    case 4: return ffm_pairs_mode<4>(mode);
+    case 8: return ffm_pairs_mode<8>(mode);
+    case 16: return ffm_pairs_mode<16>(mode);
+    case 32: return ffm_pairs_mode<32>(mode);
     default: return nullptr;
   }
 }
@@ -272,22 +271,6 @@ static FfmKernel ffm_pairs_bulk_pick(int k, int mode) {
     case 8: return ffm_pairs_bulk_mode<8>(mode);
     case 16: return ffm_pairs_bulk_mode<16>(mode);
     case 32: return ffm_pairs_bulk_mode<32>(mode);
-    default: return nullptr;
-  }
-}
-
-template <int KT>
-static FfmKernel ffm_tma_mode(int mode) {
-  return mode == FFM_PREDICT ? ffm_rows_tma_kernel<FFM_PAIRS_PREDICT, KT, FfmArgs>
-         : mode == FFM_GRAD  ? ffm_rows_tma_kernel<FFM_PAIRS_GRAD, KT, FfmArgs>
-                             : ffm_rows_tma_kernel<FFM_PAIRS_ADAGRAD, KT, FfmArgs>;
-}
-static FfmKernel ffm_tma_pick(int k, int mode) {
-  switch (k) {
-    case 4: return ffm_tma_mode<4>(mode);
-    case 8: return ffm_tma_mode<8>(mode);
-    case 16: return ffm_tma_mode<16>(mode);
-    case 32: return ffm_tma_mode<32>(mode);
     default: return nullptr;
   }
 }
@@ -382,7 +365,7 @@ static int ffm_plan_mode(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset
   const bool table = CH <= FFM_PAIRS_TABLE_MAXZ;
   // the pair kernel addresses P through 32-bit (j*nFields + f): needs d*nFields < 2^31
   FfmKernel pk = (forceBlock || CH > 1024 || m->d * m->nFields >= (int64_t)2147483647)
-                     ? nullptr : ffm_pairs_pick(m->k, mode, table);
+                     ? nullptr : ffm_pairs_pick(m->k, mode);
   if (pk && mode == FFM_ADAGRAD) {
     // the pair kernel squares per-pair contributions, which equals the per-sample gradient entry
     // (adagrad.nim:119-124) only when no row has two nonzeros of one field
@@ -390,32 +373,6 @@ static int ffm_plan_mode(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset
     int rc = ffm_has_field_dups(ctx, X, &dups);
     if (rc) return rc;
     if (dups) pk = nullptr;
-  }
-  // rows up to FFM_PAIRS_TABLE_MAXZ nonzeros: the block-per-row form of the pair loop (grad 15.1 -> 22.7 M
-  // rows/s on C5); NIMFM_FFM_KERNEL=pairwarp keeps the warp-per-row form for A/B
-  const bool wantPairWarp = env && !strcmp(env, "pairwarp");
-  // NIMFM_FFM_KERNEL=tma: the TMA-staged form (ffm_tma.cuh) when two stages of the longest row fit
-  const bool wantTma = env && !strcmp(env, "tma");
-  if (pk && table && wantTma) {
-    const int SB8 = (int)(m->nFields * m->k);
-    const size_t smem = ffm_tma_smem(CH, SB8);
-    if (smem + 1024 <= (size_t)ctx->smemOptin && (SB8 & 1) == 0) {
-      FfmKernel tk = ffm_tma_pick(m->k, mode);
-      CK(cudaFuncSetAttribute(tk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      int occ = 0;
-      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, tk, FFM_TMA_THREADS, smem));
-      if (occ >= 1) {
-        int64_t grid = std::min<int64_t>(nRows, (int64_t)occ * ctx->numSMs);
-        if (grid < 1) grid = 1;
-        pl->CH = CH;
-        pl->grid = (int)grid;
-        pl->smem = smem;
-        pl->kern = tk;
-        pl->block = FFM_TMA_THREADS;
-        pl->partialRows = grid;
-        return NIMFM_OK;
-      }
-    }
   }
   // Gradient blocks assembled in shared memory and added by TMA bulk reductions (ffm_pairs.cuh); needs a dataset
   // without repeated fields in a row (every segment of a block is written by exactly one partner).  Default for
@@ -425,7 +382,7 @@ static int ffm_plan_mode(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset
   const char *benv = getenv("NIMFM_FFM_BULK");
   const bool wantBulk = benv ? atoi(benv) == 1 : mode == FFM_ADAGRAD;
   // a bulk reduction wants 16-byte aligned global targets: an even block length and aligned buffer bases
-  if (pk && table && !wantPairWarp && !wantTma && mode != FFM_PREDICT && wantBulk && ((m->nFields * m->k) & 1) == 0 &&
+  if (pk && table && mode != FFM_PREDICT && wantBulk && ((m->nFields * m->k) & 1) == 0 &&
       targetsAligned16) {
     bool dups = false;
     int rc = ffm_has_field_dups(ctx, X, &dups);
@@ -450,7 +407,9 @@ static int ffm_plan_mode(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset
       }
     }
   }
-  if (pk && table && !wantPairWarp) {
+  // rows up to FFM_PAIRS_TABLE_MAXZ nonzeros: the block-per-row form of the pair loop (grad 15.1 -> 22.7 M
+  // rows/s on C5); longer rows take the warp-per-row form
+  if (pk && table) {
     FfmKernel bk = ffm_pairs_block_pick(m->k, mode);
     const int block = 256;
     const size_t smem = ffm_pairs_warp_smem(CH, true);
@@ -470,7 +429,7 @@ static int ffm_plan_mode(nimfm_ctx *ctx, const nimfm_ffm *m, const nimfm_dataset
   }
   if (pk) {
     const int block = 256, wpb = block / 32;
-    const size_t smem = (size_t)wpb * ffm_pairs_warp_smem(CH, table);
+    const size_t smem = (size_t)wpb * ffm_pairs_warp_smem(CH, false);
     CK(cudaFuncSetAttribute(pk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int occ = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pk, block, smem));
@@ -657,14 +616,9 @@ int32_t nimfm_ffm_decision_function(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_da
   return NIMFM_OK;
 }
 
-// which route by default: decided by measurement (DESIGN.md); the RED route until the column route is shown to win
-static bool ffm_cols_default(int64_t nRows) { (void)nRows; return false; }
-
-// The atomic-free route (ffm_cols.cuh).  *taken = 0: the shape is outside what it supports (the caller runs the
-// RED route) unless `must` is set (NIMFM_DETERMINISTIC=1), in which case that is an error.  Under `must` every
-// contiguous row range of a dataset without repeated fields runs: the tuned column kernel where its shape limits
-// hold, the generic one elsewhere.  Without `must` (NIMFM_FFM_GRAD=cols) the route runs where the tuned kernel does.
-// NIMFM_FFM_COLS=generic puts the generic kernel in the tuned kernel's place.
+// The atomic-free route (ffm_cols.cuh), taken under NIMFM_DETERMINISTIC=1: every contiguous row range of a dataset
+// without repeated fields runs, with the tuned column kernel where its shape limits hold and the generic one elsewhere;
+// any other request is an error.  NIMFM_FFM_COLS=generic puts the generic kernel in the tuned kernel's place.
 // A stated upper bound on the generic column kernel's resident 128-thread blocks per SM, not a tuning choice: it
 // equals the register-limited occupancy of the 112 / 126-register instances and lies above that of the 200 /
 // 225-register ones (2), so it changes no launch; the tests size their data past three waves of this bound.
@@ -811,51 +765,29 @@ static bool ffm_cols_want_generic() {
 }
 
 static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int loss, double thr,
-                                int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb, bool must,
-                                int *taken) {
-  *taken = 0;
-  const bool contiguous = !rowIdxDev && rowBegin >= 0 && rowBegin + nRows <= X->n;
-  const bool tunedShape = ffm_cols_tuned_shape(m, X);
-  if (!contiguous || !(tunedShape || must)) {
-    if (must)
-      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
-                        "the deterministic FFM gradient needs a contiguous row range (no row list, no wrap-around)");
-    return NIMFM_OK;
-  }
+                                int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb) {
+  if (rowIdxDev || rowBegin < 0 || rowBegin + nRows > X->n)
+    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
+                      "the deterministic FFM gradient needs a contiguous row range (no row list, no wrap-around)");
   bool dups = true;
   int rc;
   if ((rc = ffm_has_field_dups(ctx, X, &dups))) return rc;
-  if (dups) {
-    if (must)
-      return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic FFM gradient needs rows with one nonzero per "
-                        "field (a row of this dataset repeats a field)");
-    return NIMFM_OK;
-  }
+  if (dups)
+    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic FFM gradient needs rows with one nonzero per "
+                      "field (a row of this dataset repeats a field)");
   nimfm_det_twin *tw = nullptr;
   if ((rc = nimfm_det_twin_get(ctx, X, 0, &tw))) return rc;
   const FfmDetTargets o{m->grad, m->grad + m->nP(), nullptr, nullptr, ctx->scalars + 8, m->b};
-  if ((rc = ffm_det_pass(ctx, m, X, tw, loss, thr, rowBegin, nRows, mb, tunedShape && !ffm_cols_want_generic(), o)))
-    return rc;
-  *taken = 1;
-  return NIMFM_OK;
+  return ffm_det_pass(ctx, m, X, tw, loss, thr, rowBegin, nRows, mb,
+                      ffm_cols_tuned_shape(m, X) && !ffm_cols_want_generic(), o);
 }
 
 static int ffm_launch_grad(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int loss, double thr,
                            int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb) {
+  if (const char *env = getenv("NIMFM_DETERMINISTIC"); env && env[0] == '1' && nRows > 0)
+    return ffm_launch_grad_cols(ctx, m, X, loss, thr, rowBegin, nRows, rowIdxDev, mb);
   FfmPlan pl;
-  int rc;
-  {
-    // NIMFM_FFM_GRAD = cols | red | unset (automatic); NIMFM_DETERMINISTIC=1 insists on the atomic-free route
-    const char *envG = getenv("NIMFM_FFM_GRAD"), *envD = getenv("NIMFM_DETERMINISTIC");
-    const bool must = envD && envD[0] == '1';
-    const bool want = must || (envG ? !strcmp(envG, "cols") : ffm_cols_default(nRows));
-    if (want && nRows > 0) {
-      int taken = 0;
-      if ((rc = ffm_launch_grad_cols(ctx, m, X, loss, thr, rowBegin, nRows, rowIdxDev, mb, must, &taken))) return rc;
-      if (taken) return NIMFM_OK;
-    }
-  }
-  rc = ffm_plan_mode(ctx, m, X, nRows, FFM_GRAD, &pl, (reinterpret_cast<uintptr_t>(m->grad) & 15) == 0);
+  int rc = ffm_plan_mode(ctx, m, X, nRows, FFM_GRAD, &pl, (reinterpret_cast<uintptr_t>(m->grad) & 15) == 0);
   if (rc) return rc;
   if ((rc = nimfm_ensure_partials(ctx, (size_t)pl.partialRows * 4))) return rc;
   FfmArgs a;

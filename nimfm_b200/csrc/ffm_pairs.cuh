@@ -39,16 +39,15 @@ __device__ __forceinline__ void ffm_pair_advance(int &u, int &v, int step, int z
   }
 }
 
-// bytes of shared memory one warp needs: the row's records + (TABLE) the pair table of the longest row
+// bytes of shared memory one row needs: its records + (table) the pair table of the longest row
 __host__ __device__ inline size_t ffm_pairs_warp_smem(int CH, bool table) {
   size_t b = (size_t)CH * sizeof(FfmRec) + (table ? (size_t)CH * (CH - 1) / 2 * sizeof(uint16_t) : 0);
   return (b + 15) & ~(size_t)15;
 }
 
-// TABLE: the (u, v) of pair p comes from a per-warp table (u | v << 8) that depends only on the row
-// length z and is rebuilt when z changes (never, for one-feature-per-field data); ncu on the cursor
-// form (r01i): 26 K warp instructions per 39-nonzero row, most of them cursor and address arithmetic.
-template <int MODE, int KT, bool TABLE, class Args>
+// The warp form runs the rows longer than FFM_PAIRS_TABLE_MAXZ (up to 1024 nonzeros), whose pair table would not
+// fit: each slot walks the row-major pair order with a cursor (ffm_pair_advance).
+template <int MODE, int KT, class Args>
 __global__ void __launch_bounds__(256, 2) ffm_pairs_kernel(const Args a) {
   constexpr int SLOTS = 32 / KT;
   constexpr int PB = 8;   // pairs in flight per slot (2*PB gathers per lane)
@@ -58,10 +57,7 @@ __global__ void __launch_bounds__(256, 2) ffm_pairs_kernel(const Args a) {
   const int s = lane & (KT - 1);
   const int slot = lane / KT;
   const int CH = a.CH;
-  unsigned char *wbase = smem_raw + (size_t)warpInBlock * ffm_pairs_warp_smem(CH, TABLE);
-  FfmRec *rec = reinterpret_cast<FfmRec *>(wbase);
-  uint16_t *tab = reinterpret_cast<uint16_t *>(wbase + (size_t)CH * sizeof(FfmRec));
-  int zTab = -1;
+  FfmRec *rec = reinterpret_cast<FfmRec *>(smem_raw + (size_t)warpInBlock * ffm_pairs_warp_smem(CH, false));
   const int warpsPerBlock = blockDim.x >> 5;
   const int64_t warpGlobal = (int64_t)blockIdx.x * warpsPerBlock + warpInBlock;
   const int64_t nWarps = (int64_t)gridDim.x * warpsPerBlock;
@@ -88,22 +84,13 @@ __global__ void __launch_bounds__(256, 2) ffm_pairs_kernel(const Args a) {
       lin += a.w[j] * m.x;
     }
     const int nPairs = z * (z - 1) / 2;
-    if (TABLE && z != zTab) {
-      int u = 0, v = 1;
-      ffm_pair_advance(u, v, lane, z);
-      for (int p = lane; p < nPairs; p += 32) {
-        tab[p] = (uint16_t)(u | (v << 8));
-        ffm_pair_advance(u, v, 32, z);
-      }
-      zTab = z;
-    }
     __syncwarp();
 
     // ---- forward: running dot over this slot's pairs
     double acc = 0.0;
     {
       int u = 0, v = 1;
-      if (!TABLE) ffm_pair_advance(u, v, slot, z);
+      ffm_pair_advance(u, v, slot, z);
       for (int p = slot; p < nPairs; p += SLOTS * PB) {
         double a1[PB], a2[PB], xx[PB];
 #pragma unroll
@@ -111,11 +98,6 @@ __global__ void __launch_bounds__(256, 2) ffm_pairs_kernel(const Args a) {
           const bool ok = p + i * SLOTS < nPairs;
           a1[i] = 0.0; a2[i] = 0.0; xx[i] = 0.0;
           if (ok) {
-            if (TABLE) {
-              const unsigned uv = tab[p + i * SLOTS];
-              u = uv & 0xff;
-              v = uv >> 8;
-            }
             const FfmRec mu = rec[u], mv = rec[v];
             if (mv.jb != mu.jb) {                                               // the reference pairs j1 < j2 only
               a1[i] = __ldg(Pg + (int64_t)(mu.jb + mv.f) * KT);                 // P[j_u][f_v][s]
@@ -123,7 +105,7 @@ __global__ void __launch_bounds__(256, 2) ffm_pairs_kernel(const Args a) {
               xx[i] = mu.x * mv.x;
             }
           }
-          if (!TABLE) ffm_pair_advance(u, v, SLOTS, z);
+          ffm_pair_advance(u, v, SLOTS, z);
         }
 #pragma unroll
         for (int i = 0; i < PB; ++i) acc += xx[i] * (a1[i] * a2[i]);
@@ -146,7 +128,7 @@ __global__ void __launch_bounds__(256, 2) ffm_pairs_kernel(const Args a) {
     double *__restrict__ gNg = (MODE == FFM_PAIRS_ADAGRAD) ? a.dGnP + s : nullptr;
     {
       int u = 0, v = 1;
-      if (!TABLE) ffm_pair_advance(u, v, slot, z);
+      ffm_pair_advance(u, v, slot, z);
       for (int p = slot; p < nPairs; p += SLOTS * PB) {
         double a1[PB], a2[PB], cx[PB];
         int32_t e1[PB], e2[PB];   // (j*nFields + f): element offset / KT
@@ -155,11 +137,6 @@ __global__ void __launch_bounds__(256, 2) ffm_pairs_kernel(const Args a) {
           const bool ok = p + i * SLOTS < nPairs;
           e1[i] = -1; e2[i] = 0; a1[i] = 0.0; a2[i] = 0.0; cx[i] = 0.0;
           if (ok) {
-            if (TABLE) {
-              const unsigned uv = tab[p + i * SLOTS];
-              u = uv & 0xff;
-              v = uv >> 8;
-            }
             const FfmRec mu = rec[u], mv = rec[v];
             if (mv.jb != mu.jb) {
               e1[i] = mu.jb + mv.f;                        // entry (j_u, f_v)
@@ -169,7 +146,7 @@ __global__ void __launch_bounds__(256, 2) ffm_pairs_kernel(const Args a) {
               cx[i] = coef * (mu.x * mv.x);
             }
           }
-          if (!TABLE) ffm_pair_advance(u, v, SLOTS, z);
+          ffm_pair_advance(u, v, SLOTS, z);
         }
 #pragma unroll
         for (int i = 0; i < PB; ++i) {

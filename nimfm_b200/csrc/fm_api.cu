@@ -13,11 +13,6 @@
 #include "adagrad_seq.cuh"
 #include "host_stage.h"
 
-typedef void (*RowKernel)(const RowArgs);
-RowKernel nimfm_row_kernel_predict(int degree, bool explicitLower, int k);
-RowKernel nimfm_row_kernel_grad(int degree, bool explicitLower, int k);
-RowKernel nimfm_row_kernel_adagrad(int degree, bool explicitLower, int k);
-
 // ------------------------------------------------------------------ layout permutations
 // reference model layout  R[o][s][j]   (factorization_machine.nim:33-36)
 // reference solver layout S[o][j][s]   (sgd.nim:92-96)
@@ -56,34 +51,18 @@ __global__ void permute_solver_dev(const double *S, double *D, int nO, int k, in
 }
 
 // ------------------------------------------------------------------ launch planning
-struct RowPlan {
-  RowKernel kern;
-  bool fast, stream;
-  int G, CH, block, grid;
-  size_t smem;
-  int64_t nWarps;
-};
-
-RowKernel nimfm_row_fast_kernel_predict(int degree, bool explicitLower, int k);
-RowKernel nimfm_row_stream_kernel_predict(int degree, bool explicitLower, int k);
-RowKernel nimfm_row_stream_kernel_grad(int degree, bool explicitLower, int k);
-RowKernel nimfm_row_stream_kernel_adagrad(int degree, bool explicitLower, int k);
-RowKernel nimfm_row_fast_kernel_grad(int degree, bool explicitLower, int k);
-RowKernel nimfm_row_stream_kernel_stash(int degree, bool explicitLower, int k);
-RowKernel nimfm_row_kernel_stash(int degree, bool explicitLower);
-int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, bool streamStash,
-                           int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, const RowPlan &pl, int loss, double thr,
                            int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base);
-int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, RowKernel stashKern, bool streamStash,
-                      int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, const RowPlan &pl, int loss, double thr,
                       int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base,
                       const FmDetTargets &o);
 
 static bool is_explicit(const nimfm_fm *fm) { return fm->degree > 2 && fm->nOrders == fm->degree - 1; }
 
-// Chooses the kernel (tuned instance when one exists for the shape and every row fits the staging
-// buffer, else the generic one), the staging capacity CH, the block size that maximises resident
-// warps under the shared-memory budget, and a persistent grid of occupancy x numSMs blocks.
+// Chooses the kernel (the streaming instance when one exists for the shape and no row, dummy features
+// included, holds more than 512 nonzeros, else the generic one), the staging capacity CH, the block size
+// that maximises resident warps under the shared-memory budget, and a persistent grid of occupancy x
+// numSMs blocks.
 static int plan_rows(nimfm_ctx *ctx, const nimfm_fm *fm, const nimfm_dataset *X, int64_t nRows, int mode,
                      RowPlan *pl) {
   const int nAcc = (mode == MODE_PREDICT || mode == MODE_STASH) ? 0 : (mode == MODE_GRAD ? 1 : 2);
@@ -96,40 +75,23 @@ static int plan_rows(nimfm_ctx *ctx, const nimfm_fm *fm, const nimfm_dataset *X,
   if (z < 1) z = 1;
   const size_t capPerGroup = 40 * 1024;
   const bool expl = is_explicit(fm);
-  // variant: NIMFM_ROW_KERNEL = stream (default) | fast | generic   (A/B switch for profiling; generic also forces
-  // the generic stash forward, and with it the generic column kernel, of the deterministic route)
-  const char *env = getenv("NIMFM_ROW_KERNEL");
-  const bool wantGeneric = env && !strcmp(env, "generic");
-  const bool wantFast = env && !strcmp(env, "fast");
-  RowKernel fast = nullptr;
-  bool stream = false;
-  if (!wantGeneric) {
-    if ((!wantFast || mode == MODE_STASH) && z <= 512) {
-      fast = mode == MODE_PREDICT ? nimfm_row_stream_kernel_predict(fm->degree, expl, k)
-             : mode == MODE_GRAD  ? nimfm_row_stream_kernel_grad(fm->degree, expl, k)
-             : mode == MODE_STASH ? nimfm_row_stream_kernel_stash(fm->degree, expl, k)
-                                  : nimfm_row_stream_kernel_adagrad(fm->degree, expl, k);
-      stream = fast != nullptr;
-    }
-    // (the staged fast kernel has no stash form: a shape without a streaming stash instance takes the generic one)
-    if (!fast && (mode == MODE_PREDICT || mode == MODE_GRAD)) {
-      fast = mode == MODE_PREDICT ? nimfm_row_fast_kernel_predict(fm->degree, expl, k)
-                                  : nimfm_row_fast_kernel_grad(fm->degree, expl, k);
-      if (fast && (size_t)z * ((size_t)SB8 * 8 + 16) > capPerGroup) fast = nullptr;   // a row does not fit
-    }
+  RowKernels ks;
+  switch (mode) {
+    case MODE_PREDICT: ks = row_kernels<MODE_PREDICT>(fm->degree, expl, k); break;
+    case MODE_GRAD: ks = row_kernels<MODE_GRAD>(fm->degree, expl, k); break;
+    case MODE_ADAGRAD: ks = row_kernels<MODE_ADAGRAD>(fm->degree, expl, k); break;
+    default: ks = row_kernels<MODE_STASH>(fm->degree, expl, k); break;
   }
-  RowKernel kern = fast;
+  // NIMFM_ROW_KERNEL=generic forces the generic kernel onto the streaming instance's shapes (and with the generic
+  // stash forward, the generic column kernel of the deterministic route)
+  const char *env = getenv("NIMFM_ROW_KERNEL");
+  const bool stream = ks.stream && z <= 512 && !(env && !strcmp(env, "generic"));
+  RowKernel kern = stream ? ks.stream : ks.generic;
   int64_t CH = z;
   size_t perGroup;
   if (stream) {
     perGroup = stream_group_smem((int)CH, SB8, nHotTot, nAcc);
-  } else if (fast) {
-    perGroup = fast_group_smem((int)CH, SB8, nHotTot);
   } else {
-    kern = mode == MODE_PREDICT ? nimfm_row_kernel_predict(fm->degree, expl, k)
-           : mode == MODE_GRAD  ? nimfm_row_kernel_grad(fm->degree, expl, k)
-           : mode == MODE_STASH ? nimfm_row_kernel_stash(fm->degree, expl)
-                                : nimfm_row_kernel_adagrad(fm->degree, expl, k);
     const size_t perNnz = (size_t)SB8 * 8 + 13;
     CH = std::min<int64_t>(z, (int64_t)(capPerGroup / perNnz));
     if (CH < 1)
@@ -156,7 +118,6 @@ static int plan_rows(nimfm_ctx *ctx, const nimfm_fm *fm, const nimfm_dataset *X,
   if (bestBlock == 0 || bestOcc == 0)
     return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "row kernel does not fit on an SM (perGroup=%zu B)", perGroup);
   pl->kern = kern;
-  pl->fast = fast != nullptr;
   pl->stream = stream;
   pl->G = G;
   pl->CH = (int)CH;
@@ -441,8 +402,7 @@ static int launch_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X
     if ((rc = plan_rows(ctx, fm, X, nRows, MODE_STASH, &pl))) return rc;
     RowArgs base;
     fill_row_args(base, fm, X);
-    return nimfm_fm_det_loss_grad(ctx, fm, X, pl.kern, pl.stream, pl.G, pl.CH, pl.grid, pl.block, pl.smem, pl.nWarps,
-                                  loss, thr, rowBegin, nRows, mb, yOutDev, base);
+    return nimfm_fm_det_loss_grad(ctx, fm, X, pl, loss, thr, rowBegin, nRows, mb, yOutDev, base);
   }
   rc = plan_rows(ctx, fm, X, nRows, MODE_GRAD, &pl);
   if (rc) return rc;
@@ -1099,8 +1059,7 @@ int32_t nimfm_fm_adagrad_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset
       o.gnw = direct ? fm->gnw : dGnw;
       o.red4 = part;
       o.yhat = ix->yhat;
-      rc = nimfm_fm_det_pass(ctx, fm, &ix->tw, pl.kern, pl.stream, pl.G, pl.CH, pl.grid, pl.block, pl.smem, pl.nWarps,
-                             cfg->loss, cfg->huberThreshold, 0, cnt, 1.0, nullptr, base, o);
+      rc = nimfm_fm_det_pass(ctx, fm, &ix->tw, pl, cfg->loss, cfg->huberThreshold, 0, cnt, 1.0, nullptr, base, o);
       nimfm_trace_end(ctx);
       if (rc) return rc;
     } else {

@@ -29,7 +29,8 @@
 #include "dense_kernels.cuh"
 #include "fm_rows_stream.cuh"
 
-typedef void (*RowKernel)(const RowArgs);
+// the stash forwards: the streaming instances and the generic runtime-k kernel (every degree, every k, any row length)
+template RowKernels row_kernels<MODE_STASH>(int, bool, int);
 
 namespace {
 
@@ -357,16 +358,6 @@ __global__ void fm_cols_combine_ada_kernel(const int32_t *multiCol, const int32_
   }
 }
 
-template <int DEGREE, bool EXPLICIT>
-RowKernel pick_stash(int k) {
-  switch (k) {
-    case 8: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_STASH, 8>;
-    case 16: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_STASH, 16>;
-    case 32: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_STASH, 32>;
-    default: return nullptr;
-  }
-}
-
 typedef void (*ColKernel)(const ColArgs);
 template <int DEGREE, bool EXPLICIT, bool ADA>
 ColKernel pick_cols(int k) {
@@ -391,26 +382,6 @@ ColKernel pick_cols_generic(int degree, bool explicitLower) {
 }
 
 }  // namespace
-
-RowKernel nimfm_row_stream_kernel_stash(int degree, bool explicitLower, int k) {
-  switch (degree) {
-    case 2: return pick_stash<2, false>(k);
-    case 3: return explicitLower ? pick_stash<3, true>(k) : pick_stash<3, false>(k);
-    default: return nullptr;
-  }
-}
-
-// the stash forward of the generic runtime-k row kernel: every degree, every k, rows of any length
-RowKernel nimfm_row_kernel_stash(int degree, bool explicitLower) {
-  switch (degree) {
-    case 2: return fm_rows_kernel<2, false, MODE_STASH, 0>;
-    case 3: return explicitLower ? fm_rows_kernel<3, true, MODE_STASH, 0> : fm_rows_kernel<3, false, MODE_STASH, 0>;
-    case 4: return explicitLower ? fm_rows_kernel<4, true, MODE_STASH, 0> : fm_rows_kernel<4, false, MODE_STASH, 0>;
-    case 5: return explicitLower ? fm_rows_kernel<5, true, MODE_STASH, 0> : fm_rows_kernel<5, false, MODE_STASH, 0>;
-    case 6: return explicitLower ? fm_rows_kernel<6, true, MODE_STASH, 0> : fm_rows_kernel<6, false, MODE_STASH, 0>;
-    default: return nullptr;
-  }
-}
 
 void nimfm_det_twin_free(nimfm_ctx *ctx, nimfm_det_twin *t) {
   if (!t) return;
@@ -492,19 +463,18 @@ int nimfm_det_twin_get(nimfm_ctx *ctx, const nimfm_dataset *X, int nAug, nimfm_d
 // The two passes of the deterministic route over rows [rowBegin, rowBegin + nRows) of X, with the column twin `tw` of
 // X (its row ids are X's) and the given targets: the stash forward leaves red4 (loss, sum coef, sum dL^2, -) at
 // o.red4, the column kernel and the combine add the gradient into o.gP / o.gw and, when o.gnP is set (AdaGrad, coef =
-// dL), its squares into o.gnP / o.gnw.  streamStash: stashKern is the streaming instance; the tuned column kernel then
-// reads its stash, and every other shape (or NIMFM_ROW_KERNEL=generic, which plans the generic stash forward) takes
-// the runtime-k column kernel.  base: the row arguments of X and the model (RowArgs.b may point at a refreshed
-// intercept).
-int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, RowKernel stashKern, bool streamStash,
-                      int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+// dL), its squares into o.gnP / o.gnw.  pl: the stash forward's plan (plan_rows, MODE_STASH); when it is the streaming
+// instance the tuned column kernel reads its stash, and every other shape (or NIMFM_ROW_KERNEL=generic, which plans the
+// generic stash forward) takes the runtime-k column kernel.  base: the row arguments of X and the model (RowArgs.b may
+// point at a refreshed intercept).
+int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, const RowPlan &pl, int loss, double thr,
                       int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base,
                       const FmDetTargets &o) {
   const bool expl = fm->degree > 2 && fm->nOrders == fm->degree - 1;
   const bool ada = o.gnP != nullptr;
   ColKernel ck = nullptr;
   int colKT = fm->k;
-  if (streamStash)
+  if (pl.stream)
     ck = ada ? (fm->degree == 2 ? pick_cols<2, false, true>(fm->k)
                 : fm->degree == 3 ? (expl ? pick_cols<3, true, true>(fm->k) : pick_cols<3, false, true>(fm->k)) : nullptr)
              : (fm->degree == 2 ? pick_cols<2, false, false>(fm->k)
@@ -513,7 +483,7 @@ int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, Ro
     ck = ada ? pick_cols_generic<true>(fm->degree, expl) : pick_cols_generic<false>(fm->degree, expl);
     colKT = lane_group_kt(fm->k);
   }
-  if (!ck || !stashKern)
+  if (!ck || !pl.kern)
     return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "no deterministic gradient kernel for degree %d", fm->degree);
   int rc;
   // stash record: coef + (M_o - 1) values per component and order, padded to an even number of doubles
@@ -538,7 +508,7 @@ int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, Ro
     }
     ctx->stashCap = need;
   }
-  if ((rc = nimfm_ensure_partials(ctx, (size_t)nWarps * 4))) return rc;
+  if ((rc = nimfm_ensure_partials(ctx, (size_t)pl.nWarps * 4))) return rc;
   RowArgs a = base;
   a.rowBegin = rowBegin;
   a.nRows = nRows;
@@ -548,12 +518,12 @@ int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, Ro
   a.loss = loss;
   a.thr = thr;
   a.mb = mb;
-  a.G = G;
-  a.CH = CH;
+  a.G = pl.G;
+  a.CH = pl.CH;
   a.stash = ctx->stash;
   a.stashStride = stride;
   if (o.yhat) a.yOut = o.yhat;
-  stashKern<<<grid, block, smem, ctx->stream>>>(a);
+  pl.kern<<<pl.grid, pl.block, pl.smem, ctx->stream>>>(a);
   LAUNCHED(ctx);
   if (o.yhat) {
     const int cgrid = (int)std::max<int64_t>(1, std::min<int64_t>((nRows + 255) / 256, (int64_t)ctx->numSMs * 4));
@@ -562,7 +532,7 @@ int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, Ro
     LAUNCHED(ctx);
     reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, cgrid, o.red4, 0);
   } else {
-    reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, nWarps, o.red4, 0);
+    reduce_partials_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, pl.nWarps, o.red4, 0);
   }
   LAUNCHED(ctx);
   ColArgs c;
@@ -614,8 +584,7 @@ int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, Ro
 // Deterministic predict+grad over rows [rowBegin, rowBegin + nRows) of X into the model's gradient buffers
 // (accumulating, like the RED route), with the dataset's column twin.  red4 (loss, sum coef, sum dL^2, -) is left at
 // ctx->scalars + 8.
-int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, RowKernel stashKern, bool streamStash,
-                           int G, int CH, int grid, int block, size_t smem, int64_t nWarps, int loss, double thr,
+int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, const RowPlan &pl, int loss, double thr,
                            int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base) {
   if (rowBegin < 0 || rowBegin + nRows > X->n)
     return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic gradient needs a contiguous row range without wrap-around");
@@ -626,6 +595,5 @@ int nimfm_fm_det_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X,
   o.gP = fm->grad;
   o.gw = fm->grad + fm->nP();
   o.red4 = ctx->scalars + 8;
-  return nimfm_fm_det_pass(ctx, fm, tw, stashKern, streamStash, G, CH, grid, block, smem, nWarps, loss, thr, rowBegin,
-                           nRows, mb, yOutDev, base, o);
+  return nimfm_fm_det_pass(ctx, fm, tw, pl, loss, thr, rowBegin, nRows, mb, yOutDev, base, o);
 }

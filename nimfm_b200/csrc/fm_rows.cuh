@@ -71,6 +71,17 @@ struct RowArgs {
   int G, CH;
 };
 
+typedef void (*RowKernel)(const RowArgs);
+
+// one launch of a row kernel, as plan_rows (fm_api.cu) chooses it
+struct RowPlan {
+  RowKernel kern;
+  bool stream;   // kern is the register-streaming instance (fm_rows_stream.cuh), else the generic kernel
+  int G, CH, block, grid;
+  size_t smem;
+  int64_t nWarps;
+};
+
 // where the deterministic route's outputs go (nimfm_fm_det_pass)
 struct FmDetTargets {
   double *gP = nullptr, *gw = nullptr;     // gradient sums (the model's gradient, g_sum or its delta block)

@@ -2,34 +2,4 @@
 // for degree 2..6 and the register-streaming kernel for degree 2/3 with k in {8,16,32}.
 #include "fm_rows_stream.cuh"
 
-typedef void (*RowKernel)(const RowArgs);
-
-RowKernel nimfm_row_kernel_adagrad(int degree, bool explicitLower, int k) {
-  (void)k;
-  switch (degree) {
-    case 2: return fm_rows_kernel<2, false, MODE_ADAGRAD, 0>;
-    case 3: return explicitLower ? fm_rows_kernel<3, true, MODE_ADAGRAD, 0> : fm_rows_kernel<3, false, MODE_ADAGRAD, 0>;
-    case 4: return explicitLower ? fm_rows_kernel<4, true, MODE_ADAGRAD, 0> : fm_rows_kernel<4, false, MODE_ADAGRAD, 0>;
-    case 5: return explicitLower ? fm_rows_kernel<5, true, MODE_ADAGRAD, 0> : fm_rows_kernel<5, false, MODE_ADAGRAD, 0>;
-    case 6: return explicitLower ? fm_rows_kernel<6, true, MODE_ADAGRAD, 0> : fm_rows_kernel<6, false, MODE_ADAGRAD, 0>;
-    default: return nullptr;
-  }
-}
-
-template <int DEGREE, bool EXPLICIT>
-static RowKernel pick_stream(int k) {
-  switch (k) {
-    case 8: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_ADAGRAD, 8>;
-    case 16: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_ADAGRAD, 16>;
-    case 32: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_ADAGRAD, 32>;
-    default: return nullptr;
-  }
-}
-
-RowKernel nimfm_row_stream_kernel_adagrad(int degree, bool explicitLower, int k) {
-  switch (degree) {
-    case 2: return pick_stream<2, false>(k);
-    case 3: return explicitLower ? pick_stream<3, true>(k) : pick_stream<3, false>(k);
-    default: return nullptr;
-  }
-}
+template RowKernels row_kernels<MODE_ADAGRAD>(int, bool, int);

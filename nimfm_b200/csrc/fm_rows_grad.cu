@@ -1,56 +1,6 @@
 // fm_rows_grad.cu -- instantiations of the MODE_GRAD row kernels (one TU per mode so the families
 // compile in parallel): the generic runtime-k kernel fm_rows_kernel<DEGREE, EXPLICIT, MODE, 0> for
-// degree 2..6, and the tuned fm_rows_fast_kernel / fm_rows_stream_kernel<.., KT> for degree 2/3 with
-// k in {8,16,32}.
+// degree 2..6, and fm_rows_stream_kernel<.., KT> for degree 2/3 with k in {8,16,32}.
 #include "fm_rows_stream.cuh"
 
-typedef void (*RowKernel)(const RowArgs);
-
-RowKernel nimfm_row_kernel_grad(int degree, bool explicitLower, int k) {
-  (void)k;
-  switch (degree) {
-    case 2: return fm_rows_kernel<2, false, MODE_GRAD, 0>;
-    case 3: return explicitLower ? fm_rows_kernel<3, true, MODE_GRAD, 0> : fm_rows_kernel<3, false, MODE_GRAD, 0>;
-    case 4: return explicitLower ? fm_rows_kernel<4, true, MODE_GRAD, 0> : fm_rows_kernel<4, false, MODE_GRAD, 0>;
-    case 5: return explicitLower ? fm_rows_kernel<5, true, MODE_GRAD, 0> : fm_rows_kernel<5, false, MODE_GRAD, 0>;
-    case 6: return explicitLower ? fm_rows_kernel<6, true, MODE_GRAD, 0> : fm_rows_kernel<6, false, MODE_GRAD, 0>;
-    default: return nullptr;
-  }
-}
-
-template <int DEGREE, bool EXPLICIT>
-static RowKernel pick_fast(int k) {
-  switch (k) {
-    case 8: return fm_rows_fast_kernel<DEGREE, EXPLICIT, MODE_GRAD, 8>;
-    case 16: return fm_rows_fast_kernel<DEGREE, EXPLICIT, MODE_GRAD, 16>;
-    case 32: return fm_rows_fast_kernel<DEGREE, EXPLICIT, MODE_GRAD, 32>;
-    default: return nullptr;
-  }
-}
-
-template <int DEGREE, bool EXPLICIT>
-static RowKernel pick_stream(int k) {
-  switch (k) {
-    case 8: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_GRAD, 8>;
-    case 16: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_GRAD, 16>;
-    case 32: return fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE_GRAD, 32>;
-    default: return nullptr;
-  }
-}
-
-// nullptr when no tuned instance exists for this shape
-RowKernel nimfm_row_fast_kernel_grad(int degree, bool explicitLower, int k) {
-  switch (degree) {
-    case 2: return pick_fast<2, false>(k);
-    case 3: return explicitLower ? pick_fast<3, true>(k) : pick_fast<3, false>(k);
-    default: return nullptr;
-  }
-}
-
-RowKernel nimfm_row_stream_kernel_grad(int degree, bool explicitLower, int k) {
-  switch (degree) {
-    case 2: return pick_stream<2, false>(k);
-    case 3: return explicitLower ? pick_stream<3, true>(k) : pick_stream<3, false>(k);
-    default: return nullptr;
-  }
-}
+template RowKernels row_kernels<MODE_GRAD>(int, bool, int);

@@ -10,9 +10,16 @@
 // the forward DP consumes them, and the backward pass re-gathers the same lines (L1/L2 hits: the row
 // was just read) instead of re-reading shared memory.  Shared memory holds only the per-nonzero
 // records {x, j, hot-slot offset} (16 B each) and the hot-column accumulators, so 20+ warps/SM fit.
-// Arithmetic, summation structure and the hot-column handling are identical to fm_rows_fast.cuh.
+// Arithmetic and summation structure are those of the generic kernel (fm_rows.cuh).
 #pragma once
-#include "fm_rows_fast.cuh"
+#include "fm_rows.cuh"
+
+// one nonzero of the row: one LDS.128 per nonzero in the inner loops, no integer address math
+struct __align__(16) NnzMeta {
+  double x;
+  int32_t j;
+  int32_t acc;   // element offset of the hot-slot accumulator row in sAcc, or -1 (cold)
+};
 
 __host__ __device__ inline size_t stream_group_smem(int CH, int SB8, int nHotTot, int nAcc) {
   size_t b = (size_t)CH * sizeof(NnzMeta) + (size_t)nHotTot * (SB8 + 1) * 8 * (nAcc > 0 ? nAcc : 1);
@@ -310,3 +317,41 @@ __global__ void __launch_bounds__(256, (RowCfg<DEGREE, EXPLICIT>::NO == 1 || MOD
     }
   }
 }
+
+// The row kernels of one mode for (degree, explicit lower orders, k): the streaming instance (degree 2 / 3 with k in
+// {8, 16, 32}, else null) and the generic runtime-k kernel (degree 2..6, else null).
+struct RowKernels {
+  RowKernel stream, generic;
+};
+
+template <int DEGREE, bool EXPLICIT, int MODE>
+RowKernels row_kernels_of(int k) {
+  RowKernels r{nullptr, fm_rows_kernel<DEGREE, EXPLICIT, MODE, 0>};
+  if constexpr (DEGREE <= 3) {
+    switch (k) {
+      case 8: r.stream = fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE, 8>; break;
+      case 16: r.stream = fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE, 16>; break;
+      case 32: r.stream = fm_rows_stream_kernel<DEGREE, EXPLICIT, MODE, 32>; break;
+    }
+  }
+  return r;
+}
+
+template <int MODE>
+RowKernels row_kernels(int degree, bool explicitLower, int k) {
+  switch (degree) {
+    case 2: return row_kernels_of<2, false, MODE>(k);
+    case 3: return explicitLower ? row_kernels_of<3, true, MODE>(k) : row_kernels_of<3, false, MODE>(k);
+    case 4: return explicitLower ? row_kernels_of<4, true, MODE>(k) : row_kernels_of<4, false, MODE>(k);
+    case 5: return explicitLower ? row_kernels_of<5, true, MODE>(k) : row_kernels_of<5, false, MODE>(k);
+    case 6: return explicitLower ? row_kernels_of<6, true, MODE>(k) : row_kernels_of<6, false, MODE>(k);
+    default: return {nullptr, nullptr};
+  }
+}
+
+// Each mode is instantiated in its own translation unit, so the kernel families compile in parallel:
+// fm_rows_predict.cu, fm_rows_grad.cu, fm_rows_adagrad.cu and fm_cols.cu (MODE_STASH).
+extern template RowKernels row_kernels<MODE_PREDICT>(int, bool, int);
+extern template RowKernels row_kernels<MODE_GRAD>(int, bool, int);
+extern template RowKernels row_kernels<MODE_ADAGRAD>(int, bool, int);
+extern template RowKernels row_kernels<MODE_STASH>(int, bool, int);

@@ -137,7 +137,7 @@ def sms():
 
 @pytest.fixture
 def deterministic(monkeypatch):
-    for v in ("NIMFM_ROW_KERNEL", "NIMFM_FFM_COLS", "NIMFM_FFM_GRAD", "NIMFM_ADAGRAD_SEQ"):
+    for v in ("NIMFM_ROW_KERNEL", "NIMFM_FFM_COLS", "NIMFM_ADAGRAD_SEQ"):
         monkeypatch.delenv(v, raising=False)
     monkeypatch.setenv("NIMFM_DETERMINISTIC", "1")
 

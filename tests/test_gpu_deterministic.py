@@ -155,12 +155,9 @@ def ffm_dev_grad(csr, y, P, w, b, loss, row_begin=0, n_rows=None, rows=None):
 
 
 @pytest.mark.parametrize("k", [4, 8, 16])
-@pytest.mark.parametrize("route", ["deterministic", "cols"])
+@pytest.mark.parametrize("route", ["deterministic"])
 def test_ffm_column_route_matches_oracle(oracle, monkeypatch, k, route):
-    if route == "deterministic":
-        monkeypatch.setenv("NIMFM_DETERMINISTIC", "1")
-    else:
-        monkeypatch.setenv("NIMFM_FFM_GRAD", "cols")
+    monkeypatch.setenv("NIMFM_DETERMINISTIC", "1")
     n, nF, per = 1300, 7, 9
     csr = one_per_field_csr(n, nF, per, 5 + k)
     d = nF * per

@@ -29,9 +29,9 @@ TUNED_K = (8, 16, 32)
 def det_route(degree, fit_lower, k, z_max, n_aug, env=None):
     """(forward, column kernel) the deterministic route takes.  plan_rows (fm_api.cu) gives the stash forward the
     streaming instance when one exists for (degree, explicit, k) and the longest row incl. dummies fits 512 entries,
-    else the generic runtime-k kernel; NIMFM_ROW_KERNEL=generic forces the generic one ("fast" is ignored: the staged
-    kernel has no stash form).  The tuned column kernel runs exactly where the streaming forward ran."""
-    fwd = "generic" if env == "generic" else expected_route(degree, fit_lower, k, z_max, n_aug, "det", env=env)
+    else the generic runtime-k kernel; NIMFM_ROW_KERNEL=generic forces the generic one.  The tuned column kernel runs
+    exactly where the streaming forward ran."""
+    fwd = expected_route(degree, fit_lower, k, z_max, n_aug, env=env)
     assert fwd in ("stream", "generic")
     return fwd, ("tuned" if fwd == "stream" else "generic")
 
@@ -93,7 +93,6 @@ def test_det_route_table_covers_every_cell(n_sms):
     fitLinear=False, and the multi-wave size."""
     # the rule on its own
     assert det_route(3, "explicit", 32, 39, 0) == ("stream", "tuned")
-    assert det_route(3, "explicit", 32, 39, 0, env="fast") == ("stream", "tuned")
     assert det_route(3, "explicit", 32, 39, 0, env="generic") == ("generic", "generic")
     assert det_route(2, "explicit", 30, 39, 0) == ("generic", "generic")            # the default model's rank
     assert det_route(4, "explicit", 16, 39, 0) == ("generic", "generic")

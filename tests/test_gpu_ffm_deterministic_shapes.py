@@ -174,7 +174,6 @@ def sms():
 @pytest.fixture
 def deterministic(monkeypatch):
     monkeypatch.delenv("NIMFM_FFM_COLS", raising=False)
-    monkeypatch.delenv("NIMFM_FFM_GRAD", raising=False)
     monkeypatch.setenv("NIMFM_DETERMINISTIC", "1")
 
 
