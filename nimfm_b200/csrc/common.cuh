@@ -105,7 +105,7 @@ struct nimfm_ctx {
   uint32_t barrierEpoch = 0;
   // NIMFM_TRACE=1: device time per phase of the multi-rank epochs (CUDA events on the stream, summed per tag and
   // printed to stderr by nimfm_trace_report) -- a measurement aid, off by default
-  struct TraceSpan { const char *tag; cudaEvent_t e0, e1; };
+  struct TraceSpan { const char *tag; cudaEvent_t e0, e1; bool open; };   // spans may nest: end closes the innermost
   std::vector<TraceSpan> trace;
   int traceOn = -1;
 };
@@ -164,12 +164,13 @@ int nimfm_transpose_sort(nimfm_ctx *ctx, int64_t nsIn, int64_t nsOut, int64_t nn
                          const int32_t *inIdx, const double *inData, TransposeScratch *s, double *outData,
                          int32_t *outIdx, int64_t *outPtr);
 
-// dataset_ops.cu: the column index of ONE minibatch (rows rowIdx[0 .. B) or rowBegin .. rowBegin + B - 1), built on
-// the device for the deterministic AdaGrad epochs.  view: the B rows gathered into a CSR (CSR-field) dataset that keeps
-// the parent's d, nFields, maxSegNnz, hot table and field-repeat flag; csc: its stable column-major twin, whose
-// indices are positions 0 .. B-1 in the view (a row listed twice gives two positions); tw: that twin's 512-entry
-// segments in the dataset twin's layout (dummy columns d + a span all B positions).  Held by the context, grown on
-// demand, rebuilt per minibatch; view, csc and tw only point into the buffers below.
+// dataset_ops.cu: the column index of ONE minibatch (rows rowIdx[0 .. B), or (rowBegin + q) mod n for q < B: a
+// cursor that may wrap past the last row, and pass it more than once when B > n), built on the device for the
+// deterministic minibatch solvers (AdaGrad, MBPSGD, minibatch SGD).  view: the B rows gathered into a CSR (CSR-field)
+// dataset that keeps the parent's d, nFields, maxSegNnz, hot table and field-repeat flag; csc: its stable
+// column-major twin, whose indices are positions 0 .. B-1 in the view (a row listed twice gives two positions); tw:
+// that twin's 512-entry segments in the dataset twin's layout (dummy columns d + a span all B positions).  Held by the
+// context, grown on demand, rebuilt per minibatch; view, csc and tw only point into the buffers below.
 struct nimfm_mb_index {
   nimfm_dataset view, csc;
   nimfm_det_twin tw;

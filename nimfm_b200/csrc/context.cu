@@ -345,15 +345,20 @@ int nimfm_mb_schedule(nimfm_ctx *ctx, int64_t nRows, int64_t mb, int64_t it, MbS
 void nimfm_trace_begin(nimfm_ctx *ctx, const char *tag) {
   if (ctx->traceOn < 0) { const char *e = getenv("NIMFM_TRACE"); ctx->traceOn = e && e[0] == '1'; }
   if (!ctx->traceOn) return;
-  nimfm_ctx::TraceSpan sp{tag, nullptr, nullptr};
+  nimfm_ctx::TraceSpan sp{tag, nullptr, nullptr, true};
   cudaEventCreate(&sp.e0);
   cudaEventCreate(&sp.e1);
   cudaEventRecord(sp.e0, ctx->stream);
   ctx->trace.push_back(sp);
 }
 void nimfm_trace_end(nimfm_ctx *ctx) {
-  if (ctx->traceOn != 1 || ctx->trace.empty()) return;
-  cudaEventRecord(ctx->trace.back().e1, ctx->stream);
+  if (ctx->traceOn != 1) return;
+  for (auto sp = ctx->trace.rbegin(); sp != ctx->trace.rend(); ++sp)
+    if (sp->open) {
+      cudaEventRecord(sp->e1, ctx->stream);
+      sp->open = false;
+      return;
+    }
 }
 void nimfm_trace_report(nimfm_ctx *ctx, const char *what) {
   if (ctx->traceOn != 1 || ctx->trace.empty()) return;

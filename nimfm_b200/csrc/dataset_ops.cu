@@ -256,10 +256,11 @@ struct SegCountSum {
   }
 };
 
-// one warp per minibatch position q: its source row, its length, and the per-column entry counts (hot columns of the
-// dataset are counted in shared memory first, as in adagrad_count_kernel, so they do not serialise on one counter)
-__global__ void mb_rows_kernel(const int64_t *indptr, const int32_t *indices, int64_t rowBegin, int64_t nRows,
-                               const int32_t *rowIdx, int64_t *rows, int64_t *len, int64_t *colCnt,
+// one warp per minibatch position q: its source row (rowIdx[q], or (rowBegin + q) mod n: a cursor that wraps past the
+// last row), its length, and the per-column entry counts (hot columns of the dataset are counted in shared memory
+// first, as in adagrad_count_kernel, so they do not serialise on one counter)
+__global__ void mb_rows_kernel(const int64_t *indptr, const int32_t *indices, int64_t n, int64_t rowBegin,
+                               int64_t nRows, const int32_t *rowIdx, int64_t *rows, int64_t *len, int64_t *colCnt,
                                const uint8_t *hotSlot, const int32_t *hotList, int nHot) {
   __shared__ unsigned long long hotCnt[16];
   if (threadIdx.x < 16) hotCnt[threadIdx.x] = 0;
@@ -268,7 +269,7 @@ __global__ void mb_rows_kernel(const int64_t *indptr, const int32_t *indices, in
   const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5;
   const int64_t nWarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t q = warp; q < nRows; q += nWarps) {
-    const int64_t r = rowIdx ? (int64_t)rowIdx[q] : rowBegin + q;
+    const int64_t r = rowIdx ? (int64_t)rowIdx[q] : (rowBegin + q) % n;
     if (lane == 0) {
       rows[q] = r;
       len[q] = indptr[r + 1] - indptr[r];
@@ -361,7 +362,8 @@ void nimfm_mb_index_free(nimfm_mb_index *m) {
 int nimfm_mb_index_build(nimfm_ctx *ctx, const nimfm_dataset *X, int nAug, int64_t rowBegin, int64_t nRows,
                          const int32_t *rowIdx, nimfm_mb_index **out) {
   REQUIRE(X->kind == NIMFM_DS_CSR || X->kind == NIMFM_DS_CSR_FIELD, "the minibatch column index needs a CSR dataset");
-  REQUIRE(nRows >= 0 && (rowIdx || (rowBegin >= 0 && rowBegin + nRows <= X->n)), "bad minibatch rows");
+  REQUIRE(nRows >= 0 && (rowIdx || (rowBegin >= 0 && (rowBegin < X->n || rowBegin + nRows <= X->n))),
+          "bad minibatch rows");
   if (!ctx->mbIndex) ctx->mbIndex = new nimfm_mb_index();
   nimfm_mb_index *m = ctx->mbIndex;
   const int64_t d = X->d, dd = d + nAug, B = nRows;
@@ -376,8 +378,9 @@ int nimfm_mb_index_build(nimfm_ctx *ctx, const nimfm_dataset *X, int nAug, int64
   if (!m->hostTot) CK(cudaMallocHost(&m->hostTot, 4 * sizeof(int64_t)));
   SegCount *cnt = reinterpret_cast<SegCount *>(m->segOff), *off = cnt + dd + 1;
   CK(cudaMemsetAsync(m->colCnt, 0, (size_t)d * 8, ctx->stream));
-  mb_rows_kernel<<<grid_for(ctx, B * 32), 256, 0, ctx->stream>>>(X->indptr, X->indices, rowBegin, B, rowIdx, m->rows,
-                                                                m->rowLen, m->colCnt, X->hotSlot, X->hotList, X->nHot);
+  mb_rows_kernel<<<grid_for(ctx, B * 32), 256, 0, ctx->stream>>>(X->indptr, X->indices, X->n, rowBegin, B, rowIdx,
+                                                                m->rows, m->rowLen, m->colCnt, X->hotSlot, X->hotList,
+                                                                X->nHot);
   LAUNCHED(ctx);
   mb_seg_count_kernel<<<grid_for(ctx, dd + 1), 256, 0, ctx->stream>>>(m->colCnt, d, nAug, B, cnt);
   LAUNCHED(ctx);

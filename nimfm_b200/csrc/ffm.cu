@@ -764,17 +764,24 @@ static bool ffm_cols_want_generic() {
   return envC && !strcmp(envC, "generic");
 }
 
-static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int loss, double thr,
-                                int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb) {
-  if (rowIdxDev || rowBegin < 0 || rowBegin + nRows > X->n)
-    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
-                      "the deterministic FFM gradient needs a contiguous row range (no row list, no wrap-around)");
+// a column entry is a sample's whole gradient element only when its row holds one nonzero per field
+static int ffm_det_require_one_per_field(nimfm_ctx *ctx, const nimfm_dataset *X) {
   bool dups = true;
   int rc;
   if ((rc = ffm_has_field_dups(ctx, X, &dups))) return rc;
   if (dups)
     return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "the deterministic FFM gradient needs rows with one nonzero per "
                       "field (a row of this dataset repeats a field)");
+  return NIMFM_OK;
+}
+
+static int ffm_launch_grad_cols(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int loss, double thr,
+                                int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb) {
+  if (rowIdxDev || rowBegin < 0 || rowBegin + nRows > X->n)
+    return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED,
+                      "the deterministic FFM gradient needs a contiguous row range (no row list, no wrap-around)");
+  int rc;
+  if ((rc = ffm_det_require_one_per_field(ctx, X))) return rc;
   nimfm_det_twin *tw = nullptr;
   if ((rc = nimfm_det_twin_get(ctx, X, 0, &tw))) return rc;
   const FfmDetTargets o{m->grad, m->grad + m->nP(), nullptr, nullptr, ctx->scalars + 8, m->b};
@@ -802,10 +809,28 @@ static int ffm_launch_grad(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X,
   return NIMFM_OK;
 }
 
-// the pair kernel over rows of a resident dataset into m->grad (+ red4 at ctx->scalars+8), for sgd_mb.cu
+// the gradient of one minibatch of the minibatch-SGD epoch (rows rowIdxDev[0 .. nRows), or the cursor
+// (rowBegin + q) mod n) into m->grad, red4 at ctx->scalars + 8, for sgd_mb.cu.  Under NIMFM_DETERMINISTIC=1 a row list
+// or a cursor that wraps past the last row gets the minibatch's own column index (nimfm_mb_index_build) and the column
+// route runs over its view (as in nimfm_fm_launch_grad_rows); every other minibatch takes ffm_launch_grad as before.
 int nimfm_ffm_launch_grad_rows(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int loss, double thr,
                                int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb) {
-  return ffm_launch_grad(ctx, m, X, loss, thr, rowBegin, nRows, rowIdxDev, mb);
+  const char *env = getenv("NIMFM_DETERMINISTIC");
+  if (!(env && env[0] == '1') || (!rowIdxDev && rowBegin + nRows <= X->n))
+    return ffm_launch_grad(ctx, m, X, loss, thr, rowBegin, nRows, rowIdxDev, mb);
+  int rc;
+  if ((rc = ffm_det_require_one_per_field(ctx, X))) return rc;
+  nimfm_trace_begin(ctx, "det index");
+  nimfm_mb_index *ix = nullptr;
+  rc = nimfm_mb_index_build(ctx, X, 0, rowBegin, nRows, rowIdxDev, &ix);
+  nimfm_trace_end(ctx);
+  if (rc) return rc;
+  nimfm_trace_begin(ctx, "det passes");
+  const FfmDetTargets o{m->grad, m->grad + m->nP(), nullptr, nullptr, ctx->scalars + 8, m->b};
+  rc = ffm_det_pass(ctx, m, &ix->view, &ix->tw, loss, thr, 0, nRows, mb,
+                    ffm_cols_tuned_shape(m, X) && !ffm_cols_want_generic(), o);
+  nimfm_trace_end(ctx);
+  return rc;
 }
 
 int32_t nimfm_ffm_loss_grad(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_dataset *X, int32_t loss,

@@ -439,6 +439,39 @@ static int launch_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X
   return NIMFM_OK;
 }
 
+// The gradient of one minibatch of the MBPSGD and minibatch-SGD epochs (rows rowIdxDev[0 .. nRows), or the cursor
+// (rowBegin + q) mod n) into fm->grad, red4 at ctx->scalars + 8.  Under NIMFM_DETERMINISTIC=1 a row list or a cursor
+// that wraps past the last row cannot clip the dataset's column twin to a row range, so such a minibatch gets its own
+// column index (nimfm_mb_index_build) and the stash forward and column kernel run over its view; red4 is summed from
+// the rows' decision values (FmDetTargets::yhat), so the tuned and the generic forms give the same bits.  Every other
+// minibatch takes launch_loss_grad as before.
+static int minibatch_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, int loss, double thr,
+                               int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb) {
+  const char *env = getenv("NIMFM_DETERMINISTIC");
+  if (!(env && env[0] == '1') || (!rowIdxDev && rowBegin + nRows <= X->n))
+    return launch_loss_grad(ctx, fm, X, loss, thr, rowBegin, nRows, rowIdxDev, mb, nullptr);
+  nimfm_trace_begin(ctx, "det index");
+  nimfm_mb_index *ix = nullptr;
+  int rc = nimfm_mb_index_build(ctx, X, fm->nAug, rowBegin, nRows, rowIdxDev, &ix);
+  nimfm_trace_end(ctx);
+  if (rc) return rc;
+  nimfm_trace_begin(ctx, "det passes");
+  RowPlan pl;
+  rc = plan_rows(ctx, fm, &ix->view, nRows, MODE_STASH, &pl);
+  if (!rc) {
+    RowArgs base;
+    fill_row_args(base, fm, &ix->view);
+    FmDetTargets o;
+    o.gP = fm->grad;
+    o.gw = fm->grad + fm->nP();
+    o.red4 = ctx->scalars + 8;
+    o.yhat = ix->yhat;
+    rc = nimfm_fm_det_pass(ctx, fm, &ix->tw, pl, loss, thr, 0, nRows, mb, nullptr, base, o);
+  }
+  nimfm_trace_end(ctx);
+  return rc;
+}
+
 
 int32_t nimfm_fm_loss_grad(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, int32_t loss,
                            double huberThreshold, int64_t rowBegin, int64_t nRows, const int64_t *rowIdx,
@@ -565,10 +598,10 @@ static int apply_prox(nimfm_ctx *ctx, nimfm_fm *fm, int reg, double lam) {
 
 // entry points for psgd.cu (the SquaredL12 route of PSGD reuses the row kernel and the prox kernels)
 int nimfm_fm_apply_prox(nimfm_ctx *ctx, nimfm_fm *fm, int reg, double lam) { return apply_prox(ctx, fm, reg, lam); }
-// the row kernel over rows of a resident dataset into fm->grad (+ red4 at ctx->scalars+8), for sgd_mb.cu
+// the gradient of rows of a resident dataset into fm->grad (+ red4 at ctx->scalars+8), for sgd_mb.cu
 int nimfm_fm_launch_grad_rows(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, int loss, double thr,
                               int64_t rowBegin, int64_t nRows, const int32_t *rowIdxDev, double mb) {
-  return launch_loss_grad(ctx, fm, X, loss, thr, rowBegin, nRows, rowIdxDev, mb, nullptr);
+  return minibatch_loss_grad(ctx, fm, X, loss, thr, rowBegin, nRows, rowIdxDev, mb);
 }
 double nimfm_get_eta(int sched, double eta0, double power, double reg, int64_t it) { return get_eta(sched, eta0, power, reg, it); }
 int nimfm_fm_loss_grad_one_row(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, int loss, double thr,
@@ -715,8 +748,8 @@ int32_t nimfm_fm_mbpsgd_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset 
   if (sliceC) CK(cudaMemsetAsync(fm->b + 1, 0, 8, ctx->stream));   // epoch loss slot of the parameter pool
   for (int64_t inner = 0; inner < cfg->maxIterInner; inner++) {
     nimfm_trace_begin(ctx, "K2");
-    if ((rc = launch_loss_grad(ctx, fm, X, cfg->loss, cfg->huberThreshold, cur, localBatch,
-                               idxDev ? idxDev + inner * localBatch : nullptr, (double)cfg->miniBatchSize, nullptr)))
+    if ((rc = minibatch_loss_grad(ctx, fm, X, cfg->loss, cfg->huberThreshold, cur, localBatch,
+                                  idxDev ? idxDev + inner * localBatch : nullptr, (double)cfg->miniBatchSize)))
       return rc;
     add_tail_kernel<<<1, 1, 0, ctx->stream>>>(fm->grad + nG - 2, ctx->scalars + 8);
     LAUNCHED(ctx);
@@ -831,6 +864,7 @@ int nimfm_fm_sgd_mb_lazy_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset
   // measured on the C4 shape: 4 096-row minibatches 11.6 -> 26.4 M samples/s, 65 536-row 73.7 (dense) vs 61.7 (lazy)
   bool lazy = ctx->nranks == 1 && T >= 2 && T < (1 << 30) && touchedUpper <= 2.0 * (double)fm->dd();
   if (env) lazy = env[0] == '1' && ctx->nranks == 1 && T < (1 << 30);
+  if (const char *det = getenv("NIMFM_DETERMINISTIC"); det && det[0] == '1') lazy = false;   // the lazy step folds factors into x: RED route only
   const int SB8 = fm->nOrders * fm->k;
   if (SB8 < 1 || (SB8 & (SB8 - 1))) lazy = false;
   RowPlan plq;

@@ -151,6 +151,7 @@ int sgd_mb_epoch(nimfm_ctx *ctx, const MbModel &M, const nimfm_dataset *X, const
   if ((rc = nimfm_mb_schedule(ctx, nRows, localBatch, *it, &sch))) return rc;
   PeerScope peers(ctx, {M.grad, cnt});
   if (peers.rc) return peers.rc;
+  TraceReport traceReport{ctx, "minibatch sgd epoch", true};   // NIMFM_TRACE=1: the deterministic index / passes spans
   for (int64_t t = 0; t < sch.T; t++) {
     const int64_t q0 = std::min(t * localBatch, nRows);
     const int64_t Bl = sch.local(t), Bm = sch.global(t);   // rows of this rank / of the whole minibatch
