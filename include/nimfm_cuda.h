@@ -318,6 +318,13 @@ int32_t nimfm_ffm_adagrad_epoch(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_datase
                                 const nimfm_adagrad_cfg *cfg, int64_t *it, const int64_t *perm,
                                 int64_t nRows, double *viol, double *lossSum);
 int32_t nimfm_ffm_adagrad_finalize(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_adagrad_cfg *cfg, int64_t it);
+/* optimizer state for warm starts (AdaGrad.g_sum / g_norm, adagrad.nim:15-16, kept by init when warmStart and the
+ * shapes match, :47-62), gsP / gnP in the REFERENCE layout [field][j][s] of ffm.P.  Both need nimfm_ffm_adagrad_init
+ * first (else NIMFM_ERR_STATE); set_state takes no NULL array. */
+int32_t nimfm_ffm_adagrad_get_state(nimfm_ctx *ctx, nimfm_ffm *m, double *gsP, double *gnP, double *gsw,
+                                    double *gnw, double *gsb, double *gnb);
+int32_t nimfm_ffm_adagrad_set_state(nimfm_ctx *ctx, nimfm_ffm *m, const double *gsP, const double *gnP,
+                                    const double *gsw, const double *gnw, double gsb, double gnb);
 /* Synchronous-minibatch SGD: the deterministic device analogue of the Hogwild variants fit(..., maxThreads)
  * (optimizer/sgd_multi.nim:40-120, sgd_ffm_multi.nim:31-103).  The miniBatchSize samples of a minibatch are
  * evaluated at the same parameters and their updates applied at once with the step sizes of the minibatch's

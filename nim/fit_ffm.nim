@@ -67,8 +67,16 @@ proc runAdaGradFFM[L](self: AdaGrad[L], X: RowFieldDataset, y: seq[float64], ffm
                        alpha0: self.alpha0, alpha: self.alpha, beta: self.beta, eps: self.eps,
                        miniBatchSize: miniBatch)
   try:
+    # init (adagrad.nim:47-62): g_sum <- 0, g_norm <- eps unless warm-started with a state of the right shape
     if not ffm.warmStart: self.it = 1
-    check nimfm_ffm_adagrad_init(ctx(), h, self.eps, 1)          # init (adagrad.nim:47-62)
+    check nimfm_ffm_adagrad_init(ctx(), h, self.eps, 1)
+    if self.it != 1:
+      var
+        gsP = flat(self.g_sum.P)
+        gnP = flat(self.g_norm.P)
+      check nimfm_ffm_adagrad_set_state(ctx(), h, cast[ptr cdouble](p(gsP)), cast[ptr cdouble](p(gnP)),
+                                        cast[ptr cdouble](p(self.g_sum.w)), cast[ptr cdouble](p(self.g_norm.w)),
+                                        self.g_sum.intercept, self.g_norm.intercept)
     for epoch in 0..<self.maxIter:
       var viol, lossSum: cdouble
       if X.nCached == X.nSamples and self.shuffle: shuffle(indices)
@@ -89,7 +97,25 @@ proc runAdaGradFFM[L](self: AdaGrad[L], X: RowFieldDataset, y: seq[float64], ffm
       if not isContinue: break
     if not isConverged and self.verbose > 0:
       echo("Objective did not converge. Increase maxIter.")
-    check nimfm_ffm_adagrad_finalize(ctx(), h, addr cfg, self.it)  # finalize (adagrad.nim:65-84)
+    # keep g_sum / g_norm for warm starts (adagrad.nim:15-16), shaped like ffm.P, then finalize (adagrad.nim:65-84)
+    block:
+      var
+        gsP = newSeq[float64](ffm.P.shape[0] * ffm.P.shape[1] * ffm.P.shape[2])
+        gnP = newSeq[float64](gsP.len)
+        gsb, gnb: cdouble
+      if self.g_sum.isNil:
+        self.g_sum = newParams([ffm.P.shape[0], ffm.P.shape[1], ffm.P.shape[2]], ffm.w.len, ffm.fitLinear,
+                               ffm.fitIntercept)
+        self.g_norm = newParams([ffm.P.shape[0], ffm.P.shape[1], ffm.P.shape[2]], ffm.w.len, ffm.fitLinear,
+                                ffm.fitIntercept)
+      check nimfm_ffm_adagrad_get_state(ctx(), h, cast[ptr cdouble](p(gsP)), cast[ptr cdouble](p(gnP)),
+                                        cast[ptr cdouble](p(self.g_sum.w)), cast[ptr cdouble](p(self.g_norm.w)),
+                                        addr gsb, addr gnb)
+      unflat(self.g_sum.P, gsP)
+      unflat(self.g_norm.P, gnP)
+      self.g_sum.intercept = gsb
+      self.g_norm.intercept = gnb
+    check nimfm_ffm_adagrad_finalize(ctx(), h, addr cfg, self.it)
     fromDevice(ffm, h)
   finally:
     discard nimfm_ffm_free(ctx(), h)

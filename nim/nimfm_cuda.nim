@@ -130,6 +130,8 @@ proc nimfm_ffm_adagrad_init*(ctx: Ctx, m: DeviceFFM, eps: cdouble, reset: int32)
 proc nimfm_ffm_adagrad_epoch*(ctx: Ctx, m: DeviceFFM, X: DeviceDataset, cfg: ptr AdagradCfg, it: ptr int64,
                              perm: ptr int64, nRows: int64, viol, lossSum: ptr cdouble): int32
 proc nimfm_ffm_adagrad_finalize*(ctx: Ctx, m: DeviceFFM, cfg: ptr AdagradCfg, it: int64): int32
+proc nimfm_ffm_adagrad_get_state*(ctx: Ctx, m: DeviceFFM, gsP, gnP, gsw, gnw, gsb, gnb: ptr cdouble): int32
+proc nimfm_ffm_adagrad_set_state*(ctx: Ctx, m: DeviceFFM, gsP, gnP, gsw, gnw: ptr cdouble, gsb, gnb: cdouble): int32
 proc nimfm_ffm_sgd_begin*(ctx: Ctx, m: DeviceFFM): int32
 proc nimfm_fm_sgd_minibatch_epoch*(ctx: Ctx, fm: DeviceFM, X: DeviceDataset, cfg: ptr SgdCfg, miniBatchSize, localBatch: int64,
                                   it: ptr int64, perm: ptr int64, nRows: int64, viol, lossSum: ptr cdouble): int32

@@ -131,6 +131,8 @@ SYMBOLS = {
     "nimfm_ffm_adagrad_init": (c_i32, [VP, VP, c_dbl, c_i32]),
     "nimfm_ffm_adagrad_epoch": (c_i32, [VP, VP, VP, C.POINTER(AdagradCfg), PI64, VP, c_i64, PD, PD]),
     "nimfm_ffm_adagrad_finalize": (c_i32, [VP, VP, C.POINTER(AdagradCfg), c_i64]),
+    "nimfm_ffm_adagrad_get_state": (c_i32, [VP, VP, VP, VP, VP, VP, PD, PD]),
+    "nimfm_ffm_adagrad_set_state": (c_i32, [VP, VP, VP, VP, VP, VP, c_dbl, c_dbl]),
     "nimfm_ffm_sgd_begin": (c_i32, [VP, VP]),
     "nimfm_ffm_sgd_epoch": (c_i32, [VP, VP, VP, C.POINTER(SgdCfg), PI64, VP, c_i64, PD, PD]),
     "nimfm_fm_sgd_minibatch_epoch": (c_i32, [VP, VP, VP, C.POINTER(SgdCfg), c_i64, c_i64, PI64, VP, c_i64, PD, PD]),

@@ -1071,4 +1071,41 @@ int32_t nimfm_ffm_adagrad_finalize(nimfm_ctx *ctx, nimfm_ffm *m, const nimfm_ada
   return NIMFM_OK;
 }
 
+// g_sum / g_norm for warm starts (adagrad.nim:15-16, kept by init :47-62).  gsP / gnP cross in the reference layout
+// P[field][j][s] and go through the same permutation as the parameters; the intercept's pair is adaScal[0..1].
+int32_t nimfm_ffm_adagrad_get_state(nimfm_ctx *ctx, nimfm_ffm *m, double *gsP, double *gnP, double *gsw, double *gnw,
+                                    double *gsb, double *gnb) {
+  if (!ctx || !m) return NIMFM_ERR_INVALID;
+  if (!m->adaReady) return nimfm_fail(ctx, NIMFM_ERR_STATE, "nimfm_ffm_adagrad_init was not called");
+  CK(cudaSetDevice(ctx->device));
+  int rc;
+  if (gsP && (rc = ffm_permute(ctx, m, gsP, m->gsP, 0))) return rc;
+  if (gnP && (rc = ffm_permute(ctx, m, gnP, m->gnP, 0))) return rc;
+  if (gsw) CK(cudaMemcpyAsync(gsw, m->gsw, (size_t)m->d * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  if (gnw) CK(cudaMemcpyAsync(gnw, m->gnw, (size_t)m->d * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  double sc[2];
+  CK(cudaMemcpyAsync(sc, m->adaScal, 16, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (gsb) *gsb = sc[0];
+  if (gnb) *gnb = sc[1];
+  return NIMFM_OK;
+}
+
+int32_t nimfm_ffm_adagrad_set_state(nimfm_ctx *ctx, nimfm_ffm *m, const double *gsP, const double *gnP,
+                                    const double *gsw, const double *gnw, double gsb, double gnb) {
+  if (!ctx || !m) return NIMFM_ERR_INVALID;
+  if (!m->adaReady) return nimfm_fail(ctx, NIMFM_ERR_STATE, "nimfm_ffm_adagrad_init was not called");
+  REQUIRE(gsP && gnP && gsw && gnw, "NULL state array");
+  CK(cudaSetDevice(ctx->device));
+  int rc;
+  if ((rc = ffm_permute(ctx, m, const_cast<double *>(gsP), m->gsP, 1))) return rc;
+  if ((rc = ffm_permute(ctx, m, const_cast<double *>(gnP), m->gnP, 1))) return rc;
+  const double sc[2] = {gsb, gnb};
+  CK(cudaMemcpyAsync(m->gsw, gsw, (size_t)m->d * 8, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(m->gnw, gnw, (size_t)m->d * 8, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaMemcpyAsync(m->adaScal, sc, 16, cudaMemcpyHostToDevice, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return NIMFM_OK;
+}
+
 }  // extern "C"

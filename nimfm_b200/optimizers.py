@@ -343,10 +343,14 @@ class AdaGrad(_Base):
         X.set_targets(y)
         n = X.nSamples
         h = fm._to_device(X) if is_ffm else fm._to_device(X.nFeatures)
-        init, epoch, fin, free = ((lib.nimfm_ffm_adagrad_init, lib.nimfm_ffm_adagrad_epoch,
-                                   lib.nimfm_ffm_adagrad_finalize, lib.nimfm_ffm_free) if is_ffm else
-                                  (lib.nimfm_fm_adagrad_init, lib.nimfm_fm_adagrad_epoch,
-                                   lib.nimfm_fm_adagrad_finalize, lib.nimfm_fm_free))
+        init, epoch, fin, free, get_state, set_state = (
+            (lib.nimfm_ffm_adagrad_init, lib.nimfm_ffm_adagrad_epoch, lib.nimfm_ffm_adagrad_finalize, lib.nimfm_ffm_free,
+             lib.nimfm_ffm_adagrad_get_state, lib.nimfm_ffm_adagrad_set_state) if is_ffm else
+            (lib.nimfm_fm_adagrad_init, lib.nimfm_fm_adagrad_epoch, lib.nimfm_fm_adagrad_finalize, lib.nimfm_fm_free,
+             lib.nimfm_fm_adagrad_get_state, lib.nimfm_fm_adagrad_set_state))
+        # g_sum.P / g_norm.P: the FM solver layout [nOrders, d+nAug, k], the FFM reference layout of ffm.P [nFields, d, k]
+        state_shape = ((X.nFields, X.nFeatures, fm.nComponents) if is_ffm else
+                       (fm.nOrders, X.nFeatures + fm.nAugments, fm.nComponents))
         # data parallel (distributed.init_comm): X is this rank's shard and miniBatchSize the GLOBAL
         # synchronous minibatch; the library all-reduces the per-minibatch deltas
         world = _dist.world()
@@ -379,12 +383,12 @@ class AdaGrad(_Base):
         self.epoch_seconds = []     # host wall time of each epoch's single library call (blocking)
         try:
             _lib.check(init(ctx, h, self.eps, 1))
-            if self.it != 1 and not is_ffm:
+            if self.it != 1:
                 if self.g_sum is None:
                     raise ValueError("warmStart=true but the optimizer has no g_sum / g_norm state.")
-                if self.g_sum["P"].shape != (fm.nOrders, X.nFeatures + fm.nAugments, fm.nComponents):
+                if self.g_sum["P"].shape != state_shape:
                     raise ValueError("warmStart=true but P.shape != g_sum.P.shape.")   # adagrad.nim:57-59
-                _lib.check(lib.nimfm_fm_adagrad_set_state(
+                _lib.check(set_state(
                     ctx, h, _lib.ptr(_lib.f64(self.g_sum["P"])), _lib.ptr(_lib.f64(self.g_norm["P"])),
                     _lib.ptr(_lib.f64(self.g_sum["w"])), _lib.ptr(_lib.f64(self.g_norm["w"])),
                     float(self.g_sum["intercept"]), float(self.g_norm["intercept"])))
@@ -417,15 +421,13 @@ class AdaGrad(_Base):
                     break
             if not self._converged and self.verbose > 0:
                 print("Objective did not converge. Increase maxIter.")
-            if not is_ffm:
-                d, dd = X.nFeatures, X.nFeatures + fm.nAugments
-                gsP, gnP = np.zeros((fm.nOrders, dd, fm.nComponents)), np.zeros((fm.nOrders, dd, fm.nComponents))
-                gsw, gnw = np.zeros(d), np.zeros(d)
-                gsb, gnb = C.c_double(), C.c_double()
-                _lib.check(lib.nimfm_fm_adagrad_get_state(ctx, h, _lib.ptr(gsP), _lib.ptr(gnP), _lib.ptr(gsw),
-                                                          _lib.ptr(gnw), C.byref(gsb), C.byref(gnb)))
-                self.g_sum = dict(P=gsP, w=gsw, intercept=gsb.value)
-                self.g_norm = dict(P=gnP, w=gnw, intercept=gnb.value)
+            gsP, gnP = np.zeros(state_shape), np.zeros(state_shape)
+            gsw, gnw = np.zeros(X.nFeatures), np.zeros(X.nFeatures)
+            gsb, gnb = C.c_double(), C.c_double()
+            _lib.check(get_state(ctx, h, _lib.ptr(gsP), _lib.ptr(gnP), _lib.ptr(gsw), _lib.ptr(gnw), C.byref(gsb),
+                                 C.byref(gnb)))
+            self.g_sum = dict(P=gsP, w=gsw, intercept=gsb.value)
+            self.g_norm = dict(P=gnP, w=gnw, intercept=gnb.value)
             _lib.check(fin(ctx, h, C.byref(cfg), self.it))     # finalize, adagrad.nim:65-84
             fm._from_device(h)
         finally:
