@@ -147,7 +147,10 @@ int32_t nimfm_stream_close(nimfm_stream *sh);
 int32_t nimfm_dataset_get_targets(nimfm_ctx *ctx, const nimfm_dataset *ds, double *y);
 
 /* ---------------------------------------------------------------- FM model state
- * FactorizationMachine (model/factorization_machine.nim:11-139).  nOrders / nAug follow :81-97. */
+ * FactorizationMachine (model/factorization_machine.nim:11-139).  nOrders / nAug follow :81-97.
+ * 1 <= degree <= 6.  nOrders = 0 if and only if degree = 1: the linear model b + <w, x>, which has no P (nAugments
+ * must be 0 as well).  Every array argument shaped like P (P, gP, the AdaGrad gsP / gnP) may be NULL when the
+ * model has no P, and nothing is copied for it. */
 int32_t nimfm_fm_create(nimfm_ctx *ctx, int32_t degree, int32_t nComponents, int32_t nOrders,
                         int32_t nAugments, int64_t nFeatures, int32_t fitLinear,
                         int32_t fitIntercept, nimfm_fm **out);

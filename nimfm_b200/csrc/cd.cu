@@ -492,8 +492,10 @@ int32_t nimfm_fm_cd_begin(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X, 
     st->updCap = nUpd;
   }
   fm->cdN = n;
-  cd_permute_kernel<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(fm->P, fm->Pcm, fm->nOrders, fm->k, dd, 1);
-  LAUNCHED(ctx);
+  if (nP > 0) {   // degree 1: no P
+    cd_permute_kernel<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(fm->P, fm->Pcm, fm->nOrders, fm->k, dd, 1);
+    LAUNCHED(ctx);
+  }
   if (fm->fitLinear) {
     cd_colnorm_kernel<<<(int)((d * 32 + 127) / 128), 128, 0, ctx->stream>>>(X->data, X->indptr, d, fm->colNormSq);
     LAUNCHED(ctx);
@@ -656,6 +658,10 @@ static int cd_enqueue_epoch(nimfm_ctx *ctx, CdState *st, nimfm_fm *fm, const nim
   (void)grid;
   if ((rc = cd_reduce(ctx, 1, X->y, fm->yPred, n, cfg->loss, cfg->huberThreshold, fm->cdScal, 1))) return rc;
   if ((rc = cd_reduce(ctx, 2, fm->w, nullptr, d, 0, 0, fm->cdScal, 4))) return rc;
+  if (fm->nP() == 0) {   // degree 1: no P, ||P||^2 = 0
+    CK(cudaMemsetAsync(fm->cdScal + 5, 0, 8, ctx->stream));
+    return NIMFM_OK;
+  }
   if ((rc = cd_reduce(ctx, 2, fm->Pcm, nullptr, fm->nP(), 0, 0, fm->cdScal, 5))) return rc;
   // keep the feature-major copy current so get_params / callbacks see this epoch's parameters
   cd_permute_kernel<<<ew_grid(ctx, fm->nP()), 256, 0, ctx->stream>>>(fm->P, fm->Pcm, fm->nOrders, fm->k, dd, 0);
@@ -677,8 +683,10 @@ int32_t nimfm_fm_cd_end(nimfm_ctx *ctx, nimfm_fm *fm) {
   if (!ctx || !fm) return NIMFM_ERR_INVALID;
   if (!fm->cdReady) return nimfm_fail(ctx, NIMFM_ERR_STATE, "nimfm_fm_cd_begin was not called");
   CK(cudaSetDevice(ctx->device));
-  cd_permute_kernel<<<ew_grid(ctx, fm->nP()), 256, 0, ctx->stream>>>(fm->P, fm->Pcm, fm->nOrders, fm->k, fm->dd(), 0);
-  LAUNCHED(ctx);
+  if (fm->nP() > 0) {
+    cd_permute_kernel<<<ew_grid(ctx, fm->nP()), 256, 0, ctx->stream>>>(fm->P, fm->Pcm, fm->nOrders, fm->k, fm->dd(), 0);
+    LAUNCHED(ctx);
+  }
   CK(cudaStreamSynchronize(ctx->stream));
   CK(cudaGetLastError());
   CdState *st = cd_state(fm, false);

@@ -59,12 +59,20 @@ int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, co
 
 static bool is_explicit(const nimfm_fm *fm) { return fm->degree > 2 && fm->nOrders == fm->degree - 1; }
 
+// the multiple a rank's flat slice of [P | w | b] is rounded up to: whole (feature, order-block) vectors, an even
+// number of doubles; 2 for the linear model (no P)
+static int64_t slice_align(const nimfm_fm *fm) {
+  const int64_t SB8 = (int64_t)fm->nOrders * fm->k;
+  return SB8 == 0 ? 2 : ((SB8 & 1) ? 2 * SB8 : SB8);
+}
+
 // Chooses the kernel (the streaming instance when one exists for the shape and no row, dummy features
 // included, holds more than 512 nonzeros, else the generic one), the staging capacity CH, the block size
 // that maximises resident warps under the shared-memory budget, and a persistent grid of occupancy x
 // numSMs blocks.
 static int plan_rows(nimfm_ctx *ctx, const nimfm_fm *fm, const nimfm_dataset *X, int64_t nRows, int mode,
                      RowPlan *pl) {
+  if (fm->nOrders == 0) return nimfm_fm_linear_plan(ctx, X, nRows, mode, pl);   // degree 1 (fm_linear.cu)
   const int nAcc = (mode == MODE_PREDICT || mode == MODE_STASH) ? 0 : (mode == MODE_GRAD ? 1 : 2);
   const int nHotTot = nAcc ? (X->hotSlot ? X->nHot : 0) + fm->nAug : 0;
   const int k = fm->k;
@@ -173,12 +181,18 @@ int32_t nimfm_fm_create(nimfm_ctx *ctx, int32_t degree, int32_t nComponents, int
                         nimfm_fm **out) {
   if (!ctx) return NIMFM_ERR_INVALID;
   REQUIRE(out != nullptr, "out is NULL");
-  REQUIRE(degree >= 2, "degree < 2 has no ANOVA term; not supported on the device path");
+  REQUIRE(degree >= 1, "degree < 1.");
   if (degree > NIMFM_MAX_DEGREE)
     return nimfm_fail(ctx, NIMFM_ERR_UNSUPPORTED, "degree %d > %d not instantiated", degree, NIMFM_MAX_DEGREE);
   REQUIRE(nComponents >= 1, "nComponents < 1.");
-  REQUIRE(nOrders == 1 || nOrders == degree - 1, "nOrders must be 1 or degree-1 (factorization_machine.nim:89-97)");
-  REQUIRE(nAugments >= 0 && nAugments < degree, "bad nAugments");
+  if (degree == 1) {   // the linear model: no ANOVA term, no P (factorization_machine.nim:89-97)
+    REQUIRE(nOrders == 0, "degree 1 has nOrders = 0 (got %d)", nOrders);
+    REQUIRE(nAugments == 0, "degree 1 has no dummy features: nAugments = %d (fitLower = augment with fitLinear gives "
+            "degree - 2 = -1 at degree 1)", nAugments);
+  } else {
+    REQUIRE(nOrders == 1 || nOrders == degree - 1, "nOrders must be 1 or degree-1 (factorization_machine.nim:89-97)");
+    REQUIRE(nAugments >= 0 && nAugments < degree, "bad nAugments");
+  }
   REQUIRE(nFeatures >= 1, "nFeatures < 1");
   CK(cudaSetDevice(ctx->device));
   nimfm_fm *fm = new nimfm_fm();
@@ -191,8 +205,7 @@ int32_t nimfm_fm_create(nimfm_ctx *ctx, int32_t degree, int32_t nComponents, int
   fm->fitIntercept = fitIntercept != 0;
   const int64_t nP = fm->nP(), d = fm->d;
   // slack: room to round a rank's flat slice up to whole (feature, order-block) vectors for up to 64 ranks
-  const int64_t SB8 = (int64_t)fm->nOrders * fm->k;
-  fm->poolCap = nP + d + 8 + 64 * ((SB8 & 1) ? 2 * SB8 : SB8);
+  fm->poolCap = nP + d + 8 + 64 * slice_align(fm);
   int rc;
   if ((rc = nimfm_comm_alloc(ctx, &fm->pool, (size_t)fm->poolCap)) || (rc = nimfm_comm_alloc(ctx, &fm->grad, (size_t)fm->poolCap))) {
     nimfm_fm_free(ctx, fm);
@@ -233,14 +246,16 @@ int32_t nimfm_fm_free(nimfm_ctx *ctx, nimfm_fm *fm) {
 int32_t nimfm_fm_set_params(nimfm_ctx *ctx, nimfm_fm *fm, const double *P, const double *w, double intercept,
                             const double *lams) {
   if (!ctx || !fm) return NIMFM_ERR_INVALID;
-  REQUIRE(P != nullptr && w != nullptr, "P / w are NULL");
-  CK(cudaSetDevice(ctx->device));
   const int64_t nP = fm->nP();
+  REQUIRE((P != nullptr || nP == 0) && w != nullptr, "P / w are NULL");
+  CK(cudaSetDevice(ctx->device));
   double *tmp = nullptr;
-  CK(cudaMalloc(&tmp, (size_t)nP * 8));
-  { int rcs = nimfm_staged_h2d(ctx, tmp, P, (size_t)nP * 8); if (rcs) { cudaFree(tmp); return rcs; } }
-  permute_model_to_dev<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(tmp, fm->P, fm->nOrders, fm->k, fm->dd());
-  LAUNCHED(ctx);
+  if (nP > 0) {
+    CK(cudaMalloc(&tmp, (size_t)nP * 8));
+    { int rcs = nimfm_staged_h2d(ctx, tmp, P, (size_t)nP * 8); if (rcs) { cudaFree(tmp); return rcs; } }
+    permute_model_to_dev<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(tmp, fm->P, fm->nOrders, fm->k, fm->dd());
+    LAUNCHED(ctx);
+  }
   CK(cudaMemcpyAsync(fm->w, w, (size_t)fm->d * 8, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(fm->b, &intercept, 8, cudaMemcpyHostToDevice, ctx->stream));
   fm->lamsAreOnes = true;
@@ -257,6 +272,7 @@ int32_t nimfm_fm_set_params(nimfm_ctx *ctx, nimfm_fm *fm, const double *P, const
 
 static int get_permuted(nimfm_ctx *ctx, nimfm_fm *fm, const double *dev, double *host) {
   const int64_t nP = fm->nP();
+  if (nP == 0) return NIMFM_OK;   // degree 1: no P
   double *tmp = nullptr;
   CK(cudaMalloc(&tmp, (size_t)nP * 8));
   permute_dev_to_model<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(dev, tmp, fm->nOrders, fm->k, fm->dd());
@@ -559,7 +575,7 @@ static double get_eta(int sched, double eta0, double power, double reg, int64_t 
 // regularisers the dense step kernel does not fuse (L1 is fused there).  Enqueued on ctx->stream; the
 // column-wise SquaredL12 iterates to its fixed point with a host check every few sweeps.
 static int apply_prox(nimfm_ctx *ctx, nimfm_fm *fm, int reg, double lam) {
-  if (reg == NIMFM_REG_IDENTITY || reg == NIMFM_REG_L1 || lam == 0.0) return NIMFM_OK;
+  if (reg == NIMFM_REG_IDENTITY || reg == NIMFM_REG_L1 || lam == 0.0 || fm->nOrders == 0) return NIMFM_OK;   // degree 1: no P to prox
   const int64_t dd = fm->dd();
   const int SB8 = fm->nOrders * fm->k;
   if (reg == NIMFM_REG_L21 || reg == NIMFM_REG_SQUAREDL12_ROWS) {
@@ -739,7 +755,7 @@ int32_t nimfm_fm_mbpsgd_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset 
   bool viaPeer = false;
   {
     const char *envS = getenv("NIMFM_MBPSGD_SHARDED");
-    const int64_t SB8 = (int64_t)fm->nOrders * fm->k, align = (SB8 & 1) ? 2 * SB8 : SB8;
+    const int64_t align = slice_align(fm);
     const int64_t c = ((nG + ctx->nranks - 1) / ctx->nranks + align - 1) / align * align;
     const bool fits = ctx->nranks > 1 && cfg->reg != NIMFM_REG_SQUAREDL12 && c * ctx->nranks <= fm->poolCap;
     viaPeer = fits && ctx->peerOK && !(envS && envS[0] == '0');
@@ -829,7 +845,7 @@ int32_t nimfm_fm_mbpsgd_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset 
     const double rP = 1.0 / (1.0 + etaP * cfg->beta), rW = 1.0 / (1.0 + etaW * cfg->alpha),
                  rB = 1.0 / (1.0 + etaB * cfg->alpha0);
     const double lam = cfg->gamma * etaP / (1.0 + etaP * cfg->beta);                         // :119-121
-    mbpsgd_step_kernel<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(
+    mbpsgd_step_kernel<<<ew_grid(ctx, std::max(nP, d)), 256, 0, ctx->stream>>>(
         fm->P, fm->grad, nP, -etaP, rP, cfg->reg, lam, fm->w, fm->grad + nP, d, -etaW, rW, fm->fitLinear, fm->b,
         fm->grad + nG - 2, -etaB, rB, fm->fitIntercept, ctx->scalars);
     LAUNCHED(ctx);
@@ -942,21 +958,26 @@ int32_t nimfm_fm_adagrad_init(nimfm_ctx *ctx, nimfm_fm *fm, double eps, int32_t 
   if (!ctx || !fm) return NIMFM_ERR_INVALID;
   CK(cudaSetDevice(ctx->device));
   const int64_t nP = fm->nP(), d = fm->d, dd = fm->dd();
-  const bool fresh = !fm->gsP;
+  const bool fresh = !fm->gsw;   // (not gsP: degree 1 has no P state)
   if (fresh) {
-    CK(cudaMalloc(&fm->gsP, (size_t)nP * 8));
-    CK(cudaMalloc(&fm->gnP, (size_t)nP * 8));
+    if (nP > 0) {
+      CK(cudaMalloc(&fm->gsP, (size_t)nP * 8));
+      CK(cudaMalloc(&fm->gnP, (size_t)nP * 8));
+    }
     CK(cudaMalloc(&fm->gsw, (size_t)d * 8));
     CK(cudaMalloc(&fm->gnw, (size_t)d * 8));
     { int rca = nimfm_comm_alloc(ctx, &fm->dG, (size_t)(2 * nP + 2 * d + dd + 8)); if (rca) return rca; }
     CK(cudaMalloc(&fm->adaScal, 8 * 8));
   }
   if (fresh || reset) {   // AdaGrad.init, :47-55
-    CK(cudaMemsetAsync(fm->gsP, 0, (size_t)nP * 8, ctx->stream));
+    if (nP > 0) {
+      CK(cudaMemsetAsync(fm->gsP, 0, (size_t)nP * 8, ctx->stream));
+      fill_kernel<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(fm->gnP, nP, eps);
+      LAUNCHED(ctx);
+    }
     CK(cudaMemsetAsync(fm->gsw, 0, (size_t)d * 8, ctx->stream));
-    fill_kernel<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(fm->gnP, nP, eps);
     fill_kernel<<<ew_grid(ctx, d), 256, 0, ctx->stream>>>(fm->gnw, d, eps);
-    ctx->launches += 2;
+    LAUNCHED(ctx);
     const double sc[2] = {0.0, eps};
     CK(cudaMemcpyAsync(fm->adaScal, sc, 16, cudaMemcpyHostToDevice, ctx->stream));
   }
@@ -1000,6 +1021,8 @@ int32_t nimfm_fm_adagrad_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset
     const char *env = getenv("NIMFM_ADAGRAD_SEQ");
     if (mb == 1 && ctx->nranks == 1 && nRows > 0 && SB8 <= ADASEQ_THREADS && smem + 2048 <= (size_t)ctx->smemOptin &&
         !(env && env[0] == '0')) {
+      // degree 1 (SB8 = 0) takes the staged kernel: its P passes are empty loops, while the pipelined kernel
+      // divides by SB8
       AdaSeqArgs q;
       memset(&q, 0, sizeof(q));
       q.data = X->data; q.indices = X->indices; q.indptr = X->indptr; q.y = X->y; q.perm = idxDev;
@@ -1013,7 +1036,7 @@ int32_t nimfm_fm_adagrad_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset
       q.it0 = *it; q.zmax = zmax;
       const size_t smemPipe = (3 * (size_t)zmax * SB8 + (size_t)SB8 * (NIMFM_MAX_DEGREE + 1) + 3 * (size_t)zmax) * 8 +
                               2 * (size_t)zmax * 4 + (size_t)SB8 + 16;
-      if (zmax <= 64 && smemPipe + 4096 <= (size_t)ctx->smemOptin && !(env && env[0] == 's')) {   // NIMFM_ADAGRAD_SEQ=staged
+      if (SB8 > 0 && zmax <= 64 && smemPipe + 4096 <= (size_t)ctx->smemOptin && !(env && env[0] == 's')) {   // NIMFM_ADAGRAD_SEQ=staged
         CK(cudaFuncSetAttribute(adagrad_fm_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemPipe));
         adagrad_fm_pipe_kernel<<<1, ADAPIPE_THREADS, smemPipe, ctx->stream>>>(q);
       } else {
@@ -1058,7 +1081,7 @@ int32_t nimfm_fm_adagrad_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset
     }
     if (!first) {
       // update() (adagrad.nim:87-110), once per touched feature
-      const int rgrid = ew_grid(ctx, nP);
+      const int rgrid = ew_grid(ctx, std::max(nP, dd));
       if ((rc = nimfm_ensure_partials(ctx, (size_t)rgrid * 4))) return rc;
       adagrad_refresh_kernel<<<rgrid, 256, 0, ctx->stream>>>(fm->P, fm->gsP, fm->gnP, dd, SB8, cntF, fm->w, fm->gsw,
                                                              fm->gnw, d, fm->fitLinear, cfg->eta0, tIt, cfg->alpha,
@@ -1131,7 +1154,7 @@ int32_t nimfm_fm_adagrad_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset
     if (direct) {
       CK(cudaMemsetAsync(cntF, 0, (size_t)dd * 8, ctx->stream));
     } else {
-      adagrad_apply_kernel<<<ew_grid(ctx, nP), 256, 0, ctx->stream>>>(fm->gsP, fm->gnP, dGsP, dGnP, nP, fm->gsw, fm->gnw,
+      adagrad_apply_kernel<<<ew_grid(ctx, std::max(nP, dd)), 256, 0, ctx->stream>>>(fm->gsP, fm->gnP, dGsP, dGnP, nP, fm->gsw, fm->gnw,
                                                                      dGsw, dGnw, d, fm->fitLinear, cntF, dd);
       LAUNCHED(ctx);
     }
@@ -1149,7 +1172,7 @@ int32_t nimfm_fm_adagrad_finalize(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_adag
   if (!ctx || !fm || !cfg) return NIMFM_ERR_INVALID;
   if (!fm->adaReady) return nimfm_fail(ctx, NIMFM_ERR_STATE, "nimfm_fm_adagrad_init was not called");
   CK(cudaSetDevice(ctx->device));
-  adagrad_finalize_kernel<<<ew_grid(ctx, fm->nP()), 256, 0, ctx->stream>>>(
+  adagrad_finalize_kernel<<<ew_grid(ctx, std::max(fm->nP(), fm->d)), 256, 0, ctx->stream>>>(
       fm->P, fm->gsP, fm->gnP, fm->nP(), fm->w, fm->gsw, fm->gnw, fm->d, fm->fitLinear, fm->b, fm->adaScal,
       fm->fitIntercept, cfg->eta0, (double)(it - 1), cfg->alpha0, cfg->alpha, cfg->beta);
   LAUNCHED(ctx);
@@ -1160,6 +1183,7 @@ int32_t nimfm_fm_adagrad_finalize(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_adag
 
 static int permute_solver(nimfm_ctx *ctx, nimfm_fm *fm, double *hostSolver, double *dev, int toDev) {
   const int64_t nP = fm->nP();
+  if (nP == 0) return NIMFM_OK;   // degree 1: no P
   double *tmp = nullptr;
   CK(cudaMalloc(&tmp, (size_t)nP * 8));
   if (toDev) CK(cudaMemcpyAsync(tmp, hostSolver, (size_t)nP * 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -1193,7 +1217,7 @@ int32_t nimfm_fm_adagrad_set_state(nimfm_ctx *ctx, nimfm_fm *fm, const double *g
                                    const double *gsw, const double *gnw, double gsb, double gnb) {
   if (!ctx || !fm) return NIMFM_ERR_INVALID;
   if (!fm->adaReady) return nimfm_fail(ctx, NIMFM_ERR_STATE, "nimfm_fm_adagrad_init was not called");
-  REQUIRE(gsP && gnP && gsw && gnw, "NULL state array");
+  REQUIRE(((gsP && gnP) || fm->nP() == 0) && gsw && gnw, "NULL state array");
   CK(cudaSetDevice(ctx->device));
   int rc;
   if ((rc = permute_solver(ctx, fm, const_cast<double *>(gsP), fm->gsP, 1))) return rc;

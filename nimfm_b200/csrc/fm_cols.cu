@@ -323,6 +323,43 @@ __global__ void __launch_bounds__(256, ADA ? 1 : 2) fm_cols_grad_generic_kernel(
   }
 }
 
+// The column pass of the degree-1 model (nOrders = 0, no P, no dummy features; the stash forward is fm_linear.cu's
+// MODE_STASH): one thread per segment walks its entries in ascending row order and adds coef * x into one register,
+// written with one plain store per column (or into the segment's partial slot, [w] / [w | w^2], for the combine
+// kernels at SB8 = 0).  ADA: g = coef * x is rounded on its own and g * g is summed into gnw, as in the other forms.
+template <bool ADA>
+__global__ void __launch_bounds__(256) fm_cols_linear_kernel(const ColArgs a) {
+  const int64_t nth = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < a.nTasks; t += nth) {
+    const int64_t j = a.taskCol[t];
+    int64_t eb = a.taskBeg[t], ee = eb + a.taskLen[t];
+    if ((int64_t)a.crow[eb] < a.rowBegin) eb = lower_bound_row(a.crow, eb, ee, a.rowBegin);
+    if (eb < ee && (int64_t)a.crow[ee - 1] >= a.rowEnd) ee = lower_bound_row(a.crow, eb, ee, a.rowEnd);
+    double accW = 0.0, accWN = 0.0;
+    for (int64_t e = eb; e < ee; ++e) {
+      const double coef = a.stash[(size_t)((int64_t)a.crow[e] - a.rowBegin) * a.stashStride];
+      if (ADA) {
+        const double gx = __dmul_rn(coef, a.cdata[e]);
+        accW += gx;
+        accWN += __dmul_rn(gx, gx);
+      } else {
+        accW += coef * a.cdata[e];
+      }
+    }
+    const int slot = a.taskSlot[t];
+    if (slot < 0) {
+      if (a.fitLinear) {
+        a.gw[j] += accW;
+        if (ADA) a.gnw[j] += accWN;
+      }
+    } else {
+      double *ps = a.partial + (size_t)slot * (ADA ? 2 : 1);
+      ps[0] = accW;
+      if (ADA) ps[1] = accWN;
+    }
+  }
+}
+
 // columns cut into several segments: their partial sums are added in segment order
 __global__ void fm_cols_combine_kernel(const int32_t *multiCol, const int32_t *multiFirst, const int32_t *multiCount,
                                        int64_t nMulti, const double *partial, int SB8, int64_t d, double *gP, double *gw,
@@ -471,10 +508,13 @@ int nimfm_fm_det_pass(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_det_twin *tw, co
                       int64_t rowBegin, int64_t nRows, double mb, double *yOutDev, const RowArgs &base,
                       const FmDetTargets &o) {
   const bool expl = fm->degree > 2 && fm->nOrders == fm->degree - 1;
-  const bool ada = o.gnP != nullptr;
+  const bool ada = o.gnP != nullptr || o.gnw != nullptr;   // (degree 1 has no P: gnP stays NULL)
   ColKernel ck = nullptr;
   int colKT = fm->k;
-  if (pl.stream)
+  if (fm->nOrders == 0) {   // degree 1: the w-only column pass, one thread per segment
+    ck = ada ? fm_cols_linear_kernel<true> : fm_cols_linear_kernel<false>;
+    colKT = 1;
+  } else if (pl.stream)
     ck = ada ? (fm->degree == 2 ? pick_cols<2, false, true>(fm->k)
                 : fm->degree == 3 ? (expl ? pick_cols<3, true, true>(fm->k) : pick_cols<3, false, true>(fm->k)) : nullptr)
              : (fm->degree == 2 ? pick_cols<2, false, false>(fm->k)

@@ -82,6 +82,9 @@ struct RowPlan {
   int64_t nWarps;
 };
 
+// fm_linear.cu: the plan of the degree-1 (nOrders = 0) row kernel, which plan_rows returns for a model without P
+int nimfm_fm_linear_plan(nimfm_ctx *ctx, const nimfm_dataset *X, int64_t nRows, int mode, RowPlan *pl);
+
 // where the deterministic route's outputs go (nimfm_fm_det_pass)
 struct FmDetTargets {
   double *gP = nullptr, *gw = nullptr;     // gradient sums (the model's gradient, g_sum or its delta block)

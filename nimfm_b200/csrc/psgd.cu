@@ -778,7 +778,8 @@ int32_t nimfm_fm_psgd_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X
     const size_t smemPipe = ((size_t)zmax * SB8 + (size_t)SB8 * (NIMFM_MAX_DEGREE + 1) + 5 * (size_t)zmax) * 8 +
                             2 * (size_t)zmax * 4 + (size_t)SB8 + 16;
     const char *env = getenv("NIMFM_PSGD_KERNEL");   // "staged": the unpipelined kernel
-    if (zmax <= 64 && (size_t)zmax * SB8 <= (size_t)PSGD_PIPE_R * PSGD_PIPE_THREADS &&
+    // degree 1 (SB8 = 0, no P) takes the staged kernel, whose P passes are empty loops; the pipelined one divides by SB8
+    if (SB8 > 0 && zmax <= 64 && (size_t)zmax * SB8 <= (size_t)PSGD_PIPE_R * PSGD_PIPE_THREADS &&
         smemPipe + 4096 <= (size_t)ctx->smemOptin && !(env && env[0] == 's')) {
       a.profile = getenv("NIMFM_PSGD_PROFILE") != nullptr;
       CK(cudaFuncSetAttribute(psgd_lazy_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemPipe));

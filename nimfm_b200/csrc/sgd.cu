@@ -728,7 +728,10 @@ int32_t nimfm_fm_sgd_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_dataset *X,
   const size_t smem = ((size_t)zmax * SB8 + 3 * (size_t)zmax) * 8 + (size_t)zmax * 8;
   const char *env = getenv("NIMFM_SGD_KERNEL");
   const size_t smemPipe = ((size_t)zmax * SB8 + (size_t)SB8 * (NIMFM_MAX_DEGREE + 1) + 4 * (size_t)zmax) * 8 + 2 * (size_t)zmax * 4 + (size_t)SB8 + 16;
-  if (SB8 <= SGDP_THREADS - 64 && zmax <= 64 && (size_t)zmax * SB8 <= (size_t)SGDP_R * SGDP_THREADS && smemPipe <= (size_t)ctx->smemOptin - 4096 && !env) {
+  // degree 1 (SB8 = 0, no P) runs the unstaged loop: its P passes are empty, the staged and pipelined forms divide by SB8
+  if (SB8 == 0) {
+    sgd_epoch_kernel<false><<<1, SGD_THREADS, 0, ctx->stream>>>(a);
+  } else if (SB8 <= SGDP_THREADS - 64 && zmax <= 64 && (size_t)zmax * SB8 <= (size_t)SGDP_R * SGDP_THREADS && smemPipe <= (size_t)ctx->smemOptin - 4096 && !env) {
     if (getenv("NIMFM_SGD_PROFILE")) a.nFields = -7;
     CK(cudaFuncSetAttribute(sgd_fm_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemPipe));
     sgd_fm_pipe_kernel<<<1, SGDP_THREADS, smemPipe, ctx->stream>>>(a, zmax);

@@ -145,7 +145,7 @@ int sgd_mb_epoch(nimfm_ctx *ctx, const MbModel &M, const nimfm_dataset *X, const
   CK(cudaMemsetAsync(M.grad, 0, (size_t)nG * 8, ctx->stream));
   CK(cudaMemsetAsync(ctx->scalars, 0, 8, ctx->stream));          // [0]: loss sum of the epoch
   CK(cudaMemsetAsync(ctx->scalars + 20, 0, 4 * 8, ctx->stream)); // [20]: viol of the epoch
-  const int gridP = ew_grid(ctx, M.nP), gridF = ew_grid(ctx, M.dd);
+  const int gridP = M.nP > 0 ? ew_grid(ctx, M.nP) : 0, gridF = ew_grid(ctx, M.dd);   // degree 1: no P pass
   // shards and shares may be uneven: all ranks run the same number of minibatches and use the GLOBAL row count
   MbSchedule sch;
   if ((rc = nimfm_mb_schedule(ctx, nRows, localBatch, *it, &sch))) return rc;
@@ -176,8 +176,10 @@ int sgd_mb_epoch(nimfm_ctx *ctx, const MbModel &M, const nimfm_dataset *X, const
     const double sP = shrink_pow(1.0 - etaP * cfg->beta, Bm), sW = shrink_pow(1.0 - etaW * cfg->alpha, Bm),
                  sB = shrink_pow(1.0 - etaB * cfg->alpha0, Bm);
     if ((rc = nimfm_ensure_partials(ctx, (size_t)(gridP + gridF) * 4))) return rc;
-    sgd_mb_P_kernel<<<gridP, 256, 0, ctx->stream>>>(M.P, M.grad, M.SB8, M.nP, cnt, sP, -etaP, ctx->partials);
-    LAUNCHED(ctx);
+    if (gridP) {
+      sgd_mb_P_kernel<<<gridP, 256, 0, ctx->stream>>>(M.P, M.grad, M.SB8, M.nP, cnt, sP, -etaP, ctx->partials);
+      LAUNCHED(ctx);
+    }
     sgd_mb_feat_kernel<<<gridF, 256, 0, ctx->stream>>>(M.w, M.grad + M.nP, M.d, cnt, M.dd, sW, -etaW, M.fitLinear, M.b,
                                                       ctx->scalars + 8, R > 1 ? M.grad + nG - 2 : nullptr, sB, -etaB,
                                                       M.fitIntercept, ctx->scalars, ctx->partials + (size_t)gridP * 4);
@@ -224,7 +226,6 @@ int32_t nimfm_fm_sgd_minibatch_epoch(nimfm_ctx *ctx, nimfm_fm *fm, const nimfm_d
   }
   MbModel M{fm->P, fm->grad, fm->w, fm->b, fm->nP(), (int64_t)fm->nOrders * fm->k, fm->d, fm->dd(), fm->nAug,
             fm->fitLinear, fm->fitIntercept, &fm->sgdCnt};
-  if (fm->nOrders == 0) M.SB8 = 1;
   return sgd_mb_epoch(ctx, M, X, cfg, miniBatchSize, localBatch, it, perm, nRows, viol, lossSum,
                       [&](int64_t q0, int64_t Bm, const int32_t *idx) {
                         return nimfm_fm_launch_grad_rows(ctx, fm, X, cfg->loss, cfg->huberThreshold, q0, Bm, idx, 1.0);

@@ -71,7 +71,15 @@ class FactorizationMachine(_FMBase):
             return 0
         return self.degree - 1 if self.fitLower == explicit else 1
 
+    def _check_augments(self):
+        # degree 1 with fitLower=augment and fitLinear=true: the reference's formula gives degree - 2 = -1 dummy
+        # features, and what it does with them is not pinned down -- refused rather than guessed
+        if self.nAugments < 0:
+            raise ValueError(f"nAugments = {self.nAugments} < 0: fitLower=augment with fitLinear=true adds degree - 2 "
+                             f"dummy features, which is negative at degree {self.degree}.")
+
     def init(self, X, force=False):            # factorization_machine.nim:125-139
+        self._check_augments()
         if force or not (self.warmStart and self.isInitialized):
             rng = np.random.default_rng(self.randomState)   # Nim's RNG stream is unpinned (SURVEY App. B)
             d = X.nFeatures
@@ -82,6 +90,7 @@ class FactorizationMachine(_FMBase):
 
     # ---- device twin
     def _to_device(self, nFeatures):
+        self._check_augments()
         P = _lib.f64(self.P)
         if P.ndim != 3 or P.shape[0] != self.nOrders or P.shape[1] != self.nComponents:
             raise ValueError("fm.P has the wrong shape")
