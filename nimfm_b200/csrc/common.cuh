@@ -212,7 +212,7 @@ struct nimfm_fm {
   bool lamsAreOnes = true;
   // gradient buffer: [gP (nP) | gw (d) | gb, lossSum | slack] contiguous for a single collective
   double *grad = nullptr;
-  double *proxState = nullptr;   // SquaredL12 column prox: [tau | prevCnt | done] (prox_kernels.cuh)
+  double *proxState = nullptr;   // SquaredL12 column prox: [tau | prevCnt | settled | done] (prox_kernels.cuh)
   // lazy MBPSGD epoch: per-feature {1/cumP, 1/cumW} at the feature's last update, touched flags
   double2 *lazyInv = nullptr;
   uint8_t *lazyFlag = nullptr;

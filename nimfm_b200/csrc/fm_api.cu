@@ -592,7 +592,7 @@ static int apply_prox(nimfm_ctx *ctx, nimfm_fm *fm, int reg, double lam) {
   const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((dd + R - 1) / R, (int64_t)ctx->numSMs * 8));
   int rc = nimfm_ensure_partials(ctx, (size_t)grid * SB8 * 2);
   if (rc) return rc;
-  if (!fm->proxState) CK(cudaMalloc(&fm->proxState, (size_t)(2 * SB8 + 8) * 8));
+  if (!fm->proxState) CK(cudaMalloc(&fm->proxState, (size_t)(3 * SB8 + 8) * 8));
   sql12_init_kernel<<<1, 256, 0, ctx->stream>>>(fm->proxState, SB8);
   LAUNCHED(ctx);
   bool done = false;
@@ -601,7 +601,7 @@ static int apply_prox(nimfm_ctx *ctx, nimfm_fm *fm, int reg, double lam) {
     sql12_update_kernel<<<1, 256, 0, ctx->stream>>>(ctx->partials, grid, SB8, lam, fm->proxState);
     ctx->launches += 2;
     if ((iter & 3) == 3) {
-      CK(cudaMemcpyAsync(ctx->hostScalars + 8, fm->proxState + 2 * SB8, 8, cudaMemcpyDeviceToHost, ctx->stream));
+      CK(cudaMemcpyAsync(ctx->hostScalars + 8, fm->proxState + 3 * SB8, 8, cudaMemcpyDeviceToHost, ctx->stream));
       CK(cudaStreamSynchronize(ctx->stream));
       done = ctx->hostScalars[8] != 0.0;
     }

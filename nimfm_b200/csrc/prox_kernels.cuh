@@ -13,6 +13,10 @@
 // the device computes it with Michelot's iteration: start from all elements, recompute tau from the
 // active set {|p| > tau}, repeat until the set stops shrinking (tau only grows, each pass is one
 // coalesced sweep with fixed-order reductions).  S is then formed exactly as the reference forms it.
+// The iteration stops at the first pass whose count does not decrease and keeps the tau that pass took
+// as input.  Stopping only on an equal count cycles in floating point when an element sits at the
+// threshold of the others: the set with it rounds tau up to it (it drops out), the set without it rounds
+// tau one ulp below it (it comes back), and the counts alternate n+1, n, n+1, ... for ever.
 #pragma once
 #include "common.cuh"
 
@@ -38,8 +42,8 @@ static __global__ void prox_rows_kernel(double *P, int64_t nRows, int k, double 
       for (int i = 0; i < NIMFM_PROX_MAXE; ++i)
         if (lane + 32 * i < k) row[lane + 32 * i] = nrm > lam ? p[i] * f : 0.0;
     } else {
-      double tau = -1.0, prevCnt = -1.0;
-      for (int iter = 0; iter < 4096; ++iter) {
+      double tau = -1.0, prevCnt = INFINITY;
+      for (int iter = 0; iter < 4096; ++iter) {   // at most k + 2 passes: the count decreases until the last
         double cnt = 0.0, sum = 0.0;
 #pragma unroll
         for (int i = 0; i < NIMFM_PROX_MAXE; ++i) {
@@ -48,10 +52,10 @@ static __global__ void prox_rows_kernel(double *P, int64_t nRows, int k, double 
         }
         cnt = warp_sum(cnt);
         sum = warp_sum(sum);
+        if (cnt >= prevCnt) break;                                 // keep the tau of the smaller set
+        prevCnt = cnt;
         const double S = sum / (1.0 + 2.0 * lam * cnt);           // squaredl12.nim:67
         tau = 2 * lam * S;
-        if (cnt == prevCnt) break;
-        prevCnt = cnt;
       }
 #pragma unroll
       for (int i = 0; i < NIMFM_PROX_MAXE; ++i)
@@ -64,14 +68,15 @@ static __global__ void prox_rows_kernel(double *P, int64_t nRows, int k, double 
 }
 
 // ------------------------------------------------------------------ column-wise: SquaredL12(transpose=true)
-// state: [tau (SB8) | prevCnt (SB8) | done flag]
+// state: [tau (SB8) | prevCnt (SB8) | settled (SB8) | done flag].  A column is settled by the first pass whose
+// count does not decrease; from then on its tau stays put while the other columns iterate.
 // One sweep: per column c, count and sum of |P[j][c]| > tau[c] over this block's features, written as
 // partials[block][c][2].  blockDim.x = R * SB8: thread -> (feature-in-block r, column c).
 static __global__ void sql12_pass_kernel(const double *P, int64_t dd, int SB8, int R, const double *state,
                                          double *partials) {
   extern __shared__ double sh[];   // [blockDim.x][2]
   const double *tau = state;
-  if (state[2 * SB8] != 0.0) return;   // converged: nothing left to do
+  if (state[3 * SB8] != 0.0) return;   // converged: nothing left to do
   const int c = threadIdx.x % SB8, rr = threadIdx.x / SB8;
   const double t = tau[c];
   double cnt = 0.0, sum = 0.0;
@@ -92,21 +97,26 @@ static __global__ void sql12_pass_kernel(const double *P, int64_t dd, int SB8, i
   }
 }
 
-// one block: fixed-order sum of the partials, new tau per column, convergence flag
+// one block: fixed-order sum of the partials, new tau per unsettled column, convergence flag
 static __global__ void sql12_update_kernel(const double *partials, int nBlocks, int SB8, double lam, double *state) {
-  double *tau = state, *prevCnt = state + SB8, *done = state + 2 * SB8;
+  double *tau = state, *prevCnt = state + SB8, *settled = state + 2 * SB8, *done = state + 3 * SB8;
   if (*done != 0.0) return;
   int conv = 1;
   for (int c = threadIdx.x; c < SB8; c += blockDim.x) {
+    if (settled[c] != 0.0) continue;
     double cnt = 0.0, sum = 0.0;
     for (int b = 0; b < nBlocks; ++b) {
       cnt += partials[((int64_t)b * SB8 + c) * 2];
       sum += partials[((int64_t)b * SB8 + c) * 2 + 1];
     }
+    if (cnt >= prevCnt[c]) {                                      // keep the tau of the smaller set
+      settled[c] = 1.0;
+      continue;
+    }
+    conv = 0;
+    prevCnt[c] = cnt;
     const double S = sum / (1.0 + 2.0 * lam * cnt);               // squaredl12.nim:67
     tau[c] = 2 * lam * S;                                         // the threshold of :69
-    conv = conv && (cnt == prevCnt[c]);
-    prevCnt[c] = cnt;
   }
   const int all = __syncthreads_and(conv);
   if (threadIdx.x == 0 && all) *done = 1.0;
@@ -123,6 +133,10 @@ static __global__ void sql12_apply_kernel(double *P, int64_t dd, int SB8, int R,
 }
 
 static __global__ void sql12_init_kernel(double *state, int SB8) {
-  for (int c = threadIdx.x; c < 2 * SB8; c += blockDim.x) state[c] = -1.0;
-  if (threadIdx.x == 0) state[2 * SB8] = 0.0;
+  for (int c = threadIdx.x; c < SB8; c += blockDim.x) {
+    state[c] = -1.0;             // tau: every element is active in the first pass
+    state[SB8 + c] = INFINITY;   // prevCnt: the first pass never stops
+    state[2 * SB8 + c] = 0.0;
+  }
+  if (threadIdx.x == 0) state[3 * SB8] = 0.0;
 }
